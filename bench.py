@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: GEdges/s for A_hat X aggregation + homophily metrics (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[4]): synthetic CSBM-H graph with power-law row lengths,
@@ -62,7 +62,43 @@ def parse():
                          "through the whole large-dataset flow of homophily_tests.py:88-137 (seconds per flow)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy: the counters, node_sum, and Y = "
+                         "A_hat X on a fixed, seeded sample of rows (at most 32 MB of Y)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "csbm"):
+        ap.error("--dump-outputs writes the outputs of --impl ours --workload csbm")
+    return args
+
+
+DUMP_Y_BYTES = 32 << 20
+
+
+def dump_rows(n, d):
+    """Sorted global row ids of the Y sample --dump-outputs writes: the same for every run and every partition."""
+    k = min(n, max(1, DUMP_Y_BYTES // (4 * d)))
+    return np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, rows, y_local, r0, r1, counters, node_sum, world):
+    """Gather the sampled rows of Y from the ranks that own them (all ranks call this); rank 0 writes the .npy files."""
+    import torch.distributed as dist
+    device = y_local.device
+    rows_t = torch.from_numpy(rows).to(device)
+    mine = (rows_t >= r0) & (rows_t < r1)
+    y_s = torch.zeros((rows.shape[0], y_local.shape[1]), dtype=torch.float32, device=device)
+    y_s[mine] = y_local.index_select(0, rows_t[mine] - r0)
+    if world > 1:
+        dist.all_reduce(y_s)
+    if int(os.environ.get("RANK", "0")) != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"y_sample": y_s.cpu().numpy(), "y_sample_rows": rows.astype(np.float64),
+              "counters": counters.cpu().numpy().astype(np.float64), "node_sum": node_sum.cpu().numpy().astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------
@@ -594,6 +630,8 @@ def main():
     if world > 1:
         dist.all_reduce(y_chk)
     y_chk = [float(v) for v in y_chk.tolist()]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump_rows(n, d), y_last, r0, r1, counters, node_sum, world)
 
     # ---- N > 1: EVERY element of Y against an independent path -- plain NCCL all-gather of the features into a
     # fresh buffer, then the N = 1 kernel in one launch on this rank's rows.  A wrong Y fails the run (exit 3).

@@ -30,7 +30,7 @@ def _free_port():
 def test_partitions_agree_on_real_gpus(world):
     n_gpus = torch.cuda.device_count()
     if n_gpus < world:
-        pytest.skip(f"needs {world} GPUs (gpurun --gpus {world})")
+        pytest.skip(f"needs {world} GPUs, {n_gpus} visible")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
            "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),
            os.path.join(ROOT, "tools", "check_partitions.py"), "--nodes", "1000003", "2000000"]

@@ -123,22 +123,40 @@ def test_kr_svm_classifiers(W):
         close(p, s[f"out_kr_p_{clf}"], rtol=1e-6, atol=1e-12)
 
 
+def golden_synthesis_archive(path):
+    """The data_synthesis graphs stored in the golden fixtures (syn_* and plot_syn_*), packed like
+    oracle/build_ref.py packs the reference's 580: {"<size>/<h>/<s>/edges": int16 [2, nnz], ".../labels": int8 [n]}."""
+    out = {}
+    for name in G.names("syn_") + G.names("plot_syn_"):
+        z = G.load(name)
+        key = "/".join(name.split("_")[-3:])
+        out[key + "/edges"] = z["in_edge_index"].astype(np.int16)
+        out[key + "/labels"] = z["in_labels"].astype(np.int8)
+    np.savez(path, **out)
+    return len(out) // 2
+
+
 @pytest.mark.timeout(3000)
-def test_data_synthesis_sweep(W):
+def test_data_synthesis_sweep(W, tmp_path):
     """synthetic_plot.py:60-110 over the data_synthesis graphs the reference ships (tools/sweep_synthesis.py): every
     metric against the oracle on a subset spread over both sizes and the whole h range; WDGH_FULL_SWEEP=1 replays all
-    580 graphs (slow: the CPU oracle needs minutes).  Skipped when oracle/_ref/data_synthesis.npz did not travel."""
+    580 graphs (slow: the CPU oracle needs minutes).  Without the packed archive (oracle/build_ref.py, made from the
+    reference) the sweep replays the six data_synthesis graphs of the golden fixtures."""
     import json
     import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    if not os.path.exists(os.path.join(root, "oracle", "_ref", "data_synthesis.npz")):
-        pytest.skip("oracle/_ref/data_synthesis.npz is not present (built by oracle/build_ref.py in the build container)")
-    limit = "0" if os.environ.get("WDGH_FULL_SWEEP") == "1" else "12"
-    out = subprocess.run([sys.executable, os.path.join(root, "tools", "sweep_synthesis.py"), "--limit", limit],
-                         capture_output=True, text=True, timeout=2900, cwd=root)
+    archive = os.path.join(root, "oracle", "_ref", "data_synthesis.npz")
+    if os.path.exists(archive):
+        limit = "0" if os.environ.get("WDGH_FULL_SWEEP") == "1" else "12"
+        expect = 580 if limit == "0" else 12
+    else:
+        archive = str(tmp_path / "data_synthesis.npz")
+        limit, expect = "0", golden_synthesis_archive(archive)
+    out = subprocess.run([sys.executable, os.path.join(root, "tools", "sweep_synthesis.py"), "--limit", limit,
+                          "--archive", archive], capture_output=True, text=True, timeout=2900, cwd=root)
     lines = [ln for ln in out.stdout.splitlines() if ln.startswith('{"sweep"')]
     assert out.returncode == 0 and lines, out.stdout[-1500:] + out.stderr[-1500:]
     rep = json.loads(lines[-1])
-    assert rep["ok"] and rep["graphs"] == (580 if limit == "0" else 12) and rep["kr"]["flips_outside_unstable"] == 0
+    assert rep["ok"] and rep["graphs"] == expect and rep["kr"]["flips_outside_unstable"] == 0

@@ -163,7 +163,9 @@ def compare(O, key, n, got, traces, ref, ref_traces, near, worst, kr, bad):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--limit", type=int, default=0, help="number of graphs (0 = all 580)")
+    ap.add_argument("--limit", type=int, default=0, help="number of graphs (0 = all of the archive)")
+    ap.add_argument("--archive", default=os.path.join("oracle", "_ref", "data_synthesis.npz"),
+                    help="graphs to replay, packed as oracle/build_ref.py packs them (relative paths: from the repo root)")
     ap.add_argument("--kr-epochs", type=int, default=2)
     ap.add_argument("--kr-sample-max", type=int, default=500)
     ap.add_argument("--out", default="")
@@ -181,10 +183,10 @@ def main():
     W = None
     if not args.compare:
         import wdgh_b200 as W
-    path = os.path.join(ROOT, "oracle", "_ref", "data_synthesis.npz")
+    path = os.path.join(ROOT, args.archive)
     if not os.path.exists(path):
-        print(json.dumps({"sweep": "data_synthesis", "unavailable": "oracle/_ref/data_synthesis.npz is missing "
-                          "(python oracle/build_ref.py in the build container)"}))
+        print(json.dumps({"sweep": "data_synthesis", "unavailable": f"{args.archive} is missing "
+                          "(python oracle/build_ref.py packs it from the reference)"}))
         return 0
     archive = np.load(path)
     worst = {k: 0.0 for k in TOL}
