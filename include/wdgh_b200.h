@@ -127,6 +127,20 @@ int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, i
                   int64_t *plan_i64, const int64_t *plan_host, float *partial,
                   int64_t row_offset, void *stream);
 
+/* Element types of wdgh_spmm_csr_bf16's output */
+#define WDGH_DTYPE_F32  0
+#define WDGH_DTYPE_BF16 1
+/* wdgh_spmm_csr with a bfloat16 feature matrix (raw bf16 bits), fp32 accumulation, y float32 or bf16 (y_dtype).
+ * ldx / ldy in elements; plan, dinv, deg_code, partial (float32) exactly as for wdgh_spmm_csr.
+ * Every row is summed in the order of wdgh_spmm_csr, and bf16 -> fp32 is exact: fp32 output is bit-identical to
+ * wdgh_spmm_csr on the upcast matrix, bf16 output is that result rounded to nearest even.  Rows of x starting on an
+ * 8-byte boundary with d and ldx multiples of 4 take the vectorised kernels; any other width or alignment works. */
+int wdgh_spmm_csr_bf16(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                       const uint16_t *x, int64_t d, int64_t ldx, void *y, int64_t ldy, int y_dtype,
+                       int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                       int64_t *plan_i64, const int64_t *plan_host, float *partial,
+                       int64_t row_offset, void *stream);
+
 /* ---- phased aggregation (overlap of the feature all-gather with compute, N > 1) ---- */
 /* seg[b][r] (int64[num_bounds][n]) = first stored entry of row r whose column id is >= bounds_dev[b]; with
  * bounds = the partition's node-id boundaries, [seg[b][r], seg[b+1][r]) are the entries of row r whose source

@@ -18,12 +18,37 @@
 //   * degree-binned load balance: rows longer than the plan's threshold are skipped
 //     here and split into fixed-size chunks, one warp per chunk, summed in a fixed
 //     order by a second small kernel (deterministic, no float atomics).
+//
+// bfloat16 features (wdgh_spmm_csr_bf16): the same kernels with the element type of x (Tin) and of y (Tout) as
+// template parameters.  Loads widen bf16 -> fp32 exactly (a 16-bit shift), the accumulators are fp32 and every row is
+// summed in the order of the fp32 instances -- stored entries in CSR order as fmaf(w, x_j, acc) per column, then the
+// self loop, then the row scale; split rows through the same chunks and the same fixed-order finish -- so a bf16 launch
+// with fp32 output is bit-identical to the fp32 launch on x.float(), and with bf16 output (round to nearest even) to
+// that result .to(bfloat16).  The fp32 instances are unchanged.
+#include <cuda_bf16.h>
 #include <limits.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "internal.cuh"
 
 namespace wdgh {
+
+using bf16 = __nv_bfloat16;
+
+// bf16 -> fp32 is exact: the bf16 bits are the upper half of the float
+__device__ __forceinline__ float bf16_lo(unsigned u) { return __uint_as_float(u << 16); }
+__device__ __forceinline__ float bf16_hi(unsigned u) { return __uint_as_float(u & 0xffff0000u); }
+__device__ __forceinline__ unsigned bf16x2_rn(float a, float b) {  // round to nearest even, a in the low half
+  const __nv_bfloat162 h = __float22bfloat162_rn(make_float2(a, b));
+  return *reinterpret_cast<const unsigned *>(&h);
+}
+// scalar element access of the split-row finish
+__device__ __forceinline__ float load1(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float load1(const bf16 *p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ void store1(float *p, float v) { *p = v; }
+__device__ __forceinline__ void store1(bf16 *p, float v) { *p = __float2bfloat16_rn(v); }
 
 template <int VEC>
 struct Vec;
@@ -45,6 +70,15 @@ struct Vec<4> {
   __device__ __forceinline__ void scale(float s) { v.x *= s; v.y *= s; v.z *= s; v.w *= s; }
   __device__ __forceinline__ void store_stream(float *p) const { st_cs(reinterpret_cast<float4 *>(p), v); }
   __device__ __forceinline__ void store(float *p) const { *reinterpret_cast<float4 *>(p) = v; }
+  __device__ __forceinline__ void load(const bf16 *p) {  // 8 bytes
+    unsigned a, b;
+    asm("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "l"(p));
+    v = make_float4(bf16_lo(a), bf16_hi(a), bf16_lo(b), bf16_hi(b));
+  }
+  __device__ __forceinline__ void store_stream(bf16 *p) const {
+    asm volatile("st.global.cs.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(bf16x2_rn(v.x, v.y)), "r"(bf16x2_rn(v.z, v.w))
+                 : "memory");
+  }
 };
 template <>
 struct Vec<2> {
@@ -64,6 +98,14 @@ struct Vec<2> {
     asm volatile("st.global.cs.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
   }
   __device__ __forceinline__ void store(float *p) const { *reinterpret_cast<float2 *>(p) = v; }
+  __device__ __forceinline__ void load(const bf16 *p) {  // 4 bytes
+    unsigned a;
+    asm("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(a) : "l"(p));
+    v = make_float2(bf16_lo(a), bf16_hi(a));
+  }
+  __device__ __forceinline__ void store_stream(bf16 *p) const {
+    asm volatile("st.global.cs.u32 [%0], %1;" ::"l"(p), "r"(bf16x2_rn(v.x, v.y)) : "memory");
+  }
 };
 template <>
 struct Vec<1> {
@@ -76,14 +118,20 @@ struct Vec<1> {
   __device__ __forceinline__ void scale(float s) { v *= s; }
   __device__ __forceinline__ void store_stream(float *p) const { __stcs(p, v); }
   __device__ __forceinline__ void store(float *p) const { *p = v; }
+  __device__ __forceinline__ void load(const bf16 *p) {  // 2 bytes
+    unsigned short a;
+    asm("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(a) : "l"(p));
+    v = bf16_lo(a);
+  }
+  __device__ __forceinline__ void store_stream(bf16 *p) const { __stcs(p, __float2bfloat16_rn(v)); }
 };
 
 // Accumulate entries [s, e) of one row into acc[NCH].  All G lanes of the group call this together.
-template <int G, int VEC, int NCH, bool HAS_VAL>
+template <int G, int VEC, int NCH, bool HAS_VAL, typename Tin>
 __device__ __forceinline__ void accumulate_range(Vec<VEC> (&acc)[NCH], int64_t s, int64_t e,
                                                  const int32_t *__restrict__ col, const float *__restrict__ val,
                                                  const float *__restrict__ tscale,  // t_j or nullptr
-                                                 const float *__restrict__ x, int64_t ldx, int cbase, int d,
+                                                 const Tin *__restrict__ x, int64_t ldx, int cbase, int d,
                                                  int gl, unsigned gmask) {
   constexpr int U0 = (NCH >= 4) ? 2 : (NCH == 2 ? 4 : 8);  // independent gathers in flight per lane
   constexpr int U = U0 < G ? U0 : G;
@@ -111,7 +159,7 @@ __device__ __forceinline__ void accumulate_range(Vec<VEC> (&acc)[NCH], int64_t s
         const int src = on ? k + u : 0;
         const int jj = __shfl_sync(gmask, j, src, G);
         ww[u] = __shfl_sync(gmask, w, src, G);
-        const float *xr = x + (int64_t)jj * ldx + cbase;
+        const Tin *xr = x + (int64_t)jj * ldx + cbase;
 #pragma unroll
         for (int t = 0; t < NCH; ++t) {
           if (on && live[t]) v[u][t].load(xr + (t * G + gl) * VEC);
@@ -128,11 +176,11 @@ __device__ __forceinline__ void accumulate_range(Vec<VEC> (&acc)[NCH], int64_t s
 }
 
 // One group of G lanes per row; rows longer than `threshold` are left to the chunk kernels.
-template <int G, int VEC, int NCH, bool HAS_VAL>
+template <int G, int VEC, int NCH, bool HAS_VAL, typename Tin = float, typename Tout = float>
 __global__ void __launch_bounds__(256)
 spmm_rows_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
-                 const float *__restrict__ val, int64_t n, const float *__restrict__ x, int d, int64_t ldx,
-                 float *__restrict__ y, int64_t ldy, int norm, int self_loop, const float *__restrict__ dinv,
+                 const float *__restrict__ val, int64_t n, const Tin *__restrict__ x, int d, int64_t ldx,
+                 Tout *__restrict__ y, int64_t ldy, int norm, int self_loop, const float *__restrict__ dinv,
                  int64_t threshold, int64_t row_offset) {
   constexpr int RPW = 32 / G;
   const int lane = threadIdx.x & 31;
@@ -170,10 +218,10 @@ spmm_rows_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__
 }
 
 // One warp per chunk of a split row: partial[chunk][:] = sum over the chunk's entries (unscaled by s_i).
-template <int VEC, int NCH, bool HAS_VAL>
+template <int VEC, int NCH, bool HAS_VAL, typename Tin = float>
 __global__ void __launch_bounds__(256)
 spmm_chunks_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
-                   const float *__restrict__ val, const float *__restrict__ x, int d, int64_t ldx, int norm,
+                   const float *__restrict__ val, const Tin *__restrict__ x, int d, int64_t ldx, int norm,
                    const float *__restrict__ dinv, const int64_t *__restrict__ plan, int64_t n_chunks,
                    float *__restrict__ partial, int64_t ldp) {
   const int lane = threadIdx.x & 31;
@@ -226,9 +274,10 @@ struct RangeArgs {
 };
 
 // One CTA per split row: fixed-order sum of its chunk partials, self loop, s_i scaling.
+template <typename Tin = float, typename Tout = float>
 __global__ void __launch_bounds__(128)
-spmm_heavy_finish_kernel(const int64_t *__restrict__ rowptr, const float *__restrict__ x, int d, int64_t ldx,
-                         float *__restrict__ y, int64_t ldy, int norm, int self_loop,
+spmm_heavy_finish_kernel(const int64_t *__restrict__ rowptr, const Tin *__restrict__ x, int d, int64_t ldx,
+                         Tout *__restrict__ y, int64_t ldy, int norm, int self_loop,
                          const float *__restrict__ dinv, const int64_t *__restrict__ plan,
                          const float *__restrict__ partial, int64_t ldp, int64_t row_offset, int finalize,
                          ExtraParts ex) {
@@ -245,8 +294,8 @@ spmm_heavy_finish_kernel(const int64_t *__restrict__ rowptr, const float *__rest
     float acc = 0.f;
     for (int64_t p = 0; p < nch; ++p) acc += partial[(c0 + p) * ldp + c];
     for (int q = 0; q < ex.n; ++q) acc += ex.base[(q * ex.part_rows + row) * ex.ld + c];
-    if (self_loop && finalize) acc = fmaf(self_w, __ldg(x + grow * ldx + c), acc);
-    y[row * ldy + c] = acc * si;  // finalize == 0: the raw partial sum (2-D partition: reduced across ranks later)
+    if (self_loop && finalize) acc = fmaf(self_w, load1(x + grow * ldx + c), acc);
+    store1(y + row * ldy + c, acc * si);  // finalize == 0: the raw partial sum (2-D partition: reduced across ranks later)
   }
 }
 
@@ -265,11 +314,12 @@ spmm_heavy_finish_kernel(const int64_t *__restrict__ rowptr, const float *__rest
 //     entries in CSR order, then the self loop -- is the one of the row kernels, so results are bit-identical.
 // Split ("heavy") rows contribute no entries and are not stored; the chunk kernels own them.
 // ---------------------------------------------------------------------------
-template <int VEC, int NCH, bool HAS_VAL, bool FULL, int MINB, bool EXTRA>
+template <int VEC, int NCH, bool HAS_VAL, bool FULL, int MINB, bool EXTRA, typename Tin = float,
+          typename Tout = float>
 __global__ void __launch_bounds__(32, MINB)
 spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
-                     const float *__restrict__ val, int64_t n, const float *__restrict__ x, int d, int64_t ldx,
-                     float *__restrict__ y, int64_t ldy, int norm, int self_loop,
+                     const float *__restrict__ val, int64_t n, const Tin *__restrict__ x, int d, int64_t ldx,
+                     Tout *__restrict__ y, int64_t ldy, int norm, int self_loop,
                      const float *__restrict__ dinv, const uint8_t *__restrict__ deg_code, int64_t threshold,
                      int64_t row_offset, RangeArgs ra, unsigned long long *__restrict__ sched) {
   constexpr int TILE = 32 * VEC * NCH;
@@ -279,6 +329,9 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
   // 20-21 ms (tools/phase_probe.py, profiles/phase_probe_r02.txt)
   constexpr int U = U0 > 8 ? 8 : (U0 < 2 ? 2 : U0);
   constexpr unsigned kFull = 0xffffffffu;
+  // the phased forms (y +=, raw partial sums, extra partial sums) exist for fp32 features and output only
+  constexpr bool PHASED = std::is_same<Tin, float>::value && std::is_same<Tout, float>::value;
+  static_assert(PHASED || !EXTRA, "extra partial sums are fp32");
   __shared__ float table[256];
   __shared__ int s_off[2][33];      // stream offset of every row slot of the group (exclusive scan), [32] = total
   __shared__ int64_t s_beg[2][32];  // first stored entry of every row slot
@@ -302,7 +355,7 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
   const int64_t W = gridDim.x;
   const int64_t n_groups = (n + 31) >> 5;
   const int ld32 = (int)ldx;
-  const float *xl = x + cbase + lane * VEC;
+  const Tin *xl = x + cbase + lane * VEC;
 
   auto load_bounds = [&](int64_t g, int64_t &b, int64_t &e, int &flag) {
     b = 0;
@@ -332,11 +385,11 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
     nostore = __ballot_sync(kFull, !inr || hv);
     total = __shfl_sync(kFull, inc, 31);
     si = (norm != WDGH_NORM_NONE && ra.finalize && inr) ? __ldg(dinv + r + row_offset) : 1.f;
-    if (FULL && ra.accumulate && inr && !hv && (e > b || ra.finalize)) {
+    if (PHASED && FULL && ra.accumulate && inr && !hv && (e > b || ra.finalize)) {
       // `y +=` phase: flush_row reads the row's earlier partial sum right before it stores -- a dependent HBM round
       // trip per row, 32 in a row per group.  Ask for the lines one group ahead so that the read is an L2 hit
       // (measured on the 16-phase e2e schedule at 64 columns: 59 -> 56 ms per phase).
-      const float *yp = y + r * ldy;
+      const Tout *yp = y + r * ldy;
 #pragma unroll
       for (int c0 = 0; c0 < TILE; c0 += 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(yp + c0));
     }
@@ -383,8 +436,10 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
   // address of the feature (or extra partial) row a stream entry gathers
   const float *el = EXTRA ? ra.ex.base + cbase + lane * VEC : nullptr;
   const int lde32 = EXTRA ? (int)ra.ex.ld : 0;
-  auto row_ptr = [&](int ju) -> const float * {
-    if (EXTRA && ju < 0) return el + (int64_t)(ju & 0x7fffffff) * lde32;
+  auto row_ptr = [&](int ju) -> const Tin * {
+    if constexpr (EXTRA) {
+      if (ju < 0) return el + (int64_t)(ju & 0x7fffffff) * lde32;
+    }
     return xl + (int64_t)ju * ld32;
   };
 
@@ -426,16 +481,21 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
         for (int t = 0; t < NCH; ++t) {
           if (live[t]) {
             const int c = cbase + (t * 32 + lane) * VEC;
-            if (ra.accumulate) {
-              Vec<VEC> prev;
-              prev.load_plain(y + row * ldy + c);
-              acc[t].add(prev);
-            }
-            if (ra.finalize) {
+            if constexpr (PHASED) {
+              if (ra.accumulate) {
+                Vec<VEC> prev;
+                prev.load_plain(y + row * ldy + c);
+                acc[t].add(prev);
+              }
+              if (ra.finalize) {
+                acc[t].scale(si);
+                acc[t].store_stream(y + row * ldy + c);
+              } else {
+                acc[t].store(y + row * ldy + c);
+              }
+            } else {
               acc[t].scale(si);
               acc[t].store_stream(y + row * ldy + c);
-            } else {
-              acc[t].store(y + row * ldy + c);
             }
           }
         }
@@ -474,7 +534,7 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
         if (k + U <= cnt) {
 #pragma unroll
           for (int u = 0; u < U; ++u) {
-            const float *xr = row_ptr(__shfl_sync(kFull, j, k + u));
+            const Tin *xr = row_ptr(__shfl_sync(kFull, j, k + u));
 #pragma unroll
             for (int t = 0; t < NCH; ++t) {
               if (live[t]) v[u][t].load(xr + t * (32 * VEC));
@@ -485,7 +545,7 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
 #pragma unroll
           for (int u = 0; u < U; ++u) {
             const bool on = k + u < cnt;
-            const float *xr = row_ptr(__shfl_sync(kFull, j, on ? k + u : 0));
+            const Tin *xr = row_ptr(__shfl_sync(kFull, j, on ? k + u : 0));
 #pragma unroll
             for (int t = 0; t < NCH; ++t) {
               if (on && live[t]) v[u][t].load(xr + t * (32 * VEC));
@@ -525,10 +585,10 @@ struct SpmmArgs {
   const int32_t *col;
   const float *val;
   int64_t n;
-  const float *x;
+  const void *x;  // float or bf16 (the Tin of the launch)
   int d;
   int64_t ldx;
-  float *y;
+  void *y;        // float or bf16 (Tout)
   int64_t ldy;
   int norm, self_loop;
   const float *dinv;
@@ -546,37 +606,38 @@ struct SpmmArgs {
 // Plain row kernel (any width / alignment): one-warp CTAs keep warp slots busy when row lengths are skewed (a CTA's
 // slots are only recycled when its longest row finishes; measured on the 1B-entry graph: 256 threads 123.8 ms,
 // 128 -> 114.7, 64 -> 112.4, 32 -> 111.3).
-template <int G, int VEC, int NCH, bool HAS_VAL>
+template <int G, int VEC, int NCH, bool HAS_VAL, typename Tin, typename Tout>
 static int launch_rows(const SpmmArgs &a) {
   constexpr int RPW = 32 / G;
   const int tile = G * VEC * NCH;
   dim3 grid((unsigned)ceil_div(a.n, RPW), (unsigned)ceil_div(a.d, tile));
-  spmm_rows_kernel<G, VEC, NCH, HAS_VAL><<<grid, 32, 0, a.st>>>(a.rowptr, a.col, a.val, a.n, a.x, a.d, a.ldx, a.y,
-                                                             a.ldy, a.norm, a.self_loop, a.dinv, a.threshold,
-                                                             a.row_offset);
+  spmm_rows_kernel<G, VEC, NCH, HAS_VAL, Tin, Tout><<<grid, 32, 0, a.st>>>(
+      a.rowptr, a.col, a.val, a.n, static_cast<const Tin *>(a.x), a.d, a.ldx, static_cast<Tout *>(a.y), a.ldy, a.norm,
+      a.self_loop, a.dinv, a.threshold, a.row_offset);
   WDGH_LAUNCHED("spmm_rows_kernel");
   return 0;
 }
 
 // split rows: one warp per chunk, then one CTA per row (fixed-order sum, extras, self loop, scale)
-template <int VEC, int NCH, bool HAS_VAL>
+template <int VEC, int NCH, bool HAS_VAL, typename Tin = float, typename Tout = float>
 static int launch_heavy(const SpmmArgs &a, const ExtraParts &ex) {
   if (a.n_chunks == 0) return 0;
   const int tile = 32 * VEC * NCH;
+  const Tin *x = static_cast<const Tin *>(a.x);
   dim3 grid((unsigned)ceil_div(a.n_chunks, 8), (unsigned)ceil_div(a.d, tile));
-  spmm_chunks_kernel<VEC, NCH, HAS_VAL><<<grid, 256, 0, a.st>>>(a.rowptr, a.col, a.val, a.x, a.d, a.ldx, a.norm,
-                                                               a.dinv, a.plan, a.n_chunks, a.partial, a.ldp);
+  spmm_chunks_kernel<VEC, NCH, HAS_VAL, Tin><<<grid, 256, 0, a.st>>>(a.rowptr, a.col, a.val, x, a.d, a.ldx, a.norm,
+                                                                    a.dinv, a.plan, a.n_chunks, a.partial, a.ldp);
   WDGH_LAUNCHED("spmm_chunks_kernel");
-  spmm_heavy_finish_kernel<<<(unsigned)a.n_heavy, 128, 0, a.st>>>(a.rowptr, a.x, a.d, a.ldx, a.y, a.ldy, a.norm,
-                                                                  a.self_loop, a.dinv, a.plan, a.partial, a.ldp,
-                                                                  a.row_offset, a.ra.finalize, ex);
+  spmm_heavy_finish_kernel<Tin, Tout><<<(unsigned)a.n_heavy, 128, 0, a.st>>>(
+      a.rowptr, x, a.d, a.ldx, static_cast<Tout *>(a.y), a.ldy, a.norm, a.self_loop, a.dinv, a.plan, a.partial, a.ldp,
+      a.row_offset, a.ra.finalize, ex);
   WDGH_LAUNCHED("spmm_heavy_finish_kernel");
   return 0;
 }
 
 // Row-group kernel: persistent grid of one-warp CTAs, 32 per SM for a single 128-column tile (measured on the
 // 1B-entry graph, d = 128: 16 CTAs/SM 118.1 ms, 24 -> 100.4, 32 -> 95.6), 16 per SM for the wider tiles.
-template <int VEC, int NCH, bool HAS_VAL>
+template <int VEC, int NCH, bool HAS_VAL, typename Tin, typename Tout>
 static int launch_rowgroup(const SpmmArgs &a) {
   constexpr int TILE = 32 * VEC * NCH;
   constexpr int MINB = (NCH == 1) ? 32 : 16;
@@ -588,13 +649,14 @@ static int launch_rowgroup(const SpmmArgs &a) {
   const bool full = (a.d == TILE);
   unsigned long long *sched = plan_sched(a.plan, kPlanSpmmTicket);
 #define WDGH_RG_LAUNCH(FULLV, MINBV, EXTRAV)                                                                        \
-  spmm_rowgroup_kernel<VEC, NCH, HAS_VAL, FULLV, MINBV, EXTRAV><<<grid, 32, 0, a.st>>>(                               \
-      a.rowptr, a.col, a.val, a.n, a.x, a.d, a.ldx, a.y, a.ldy, a.norm, a.self_loop, a.dinv, a.deg_code, a.threshold, \
-      a.row_offset, a.ra, sched)
-  if (a.ra.ex.n > 0) {
+  spmm_rowgroup_kernel<VEC, NCH, HAS_VAL, FULLV, MINBV, EXTRAV, Tin, Tout><<<grid, 32, 0, a.st>>>(                    \
+      a.rowptr, a.col, a.val, a.n, static_cast<const Tin *>(a.x), a.d, a.ldx, static_cast<Tout *>(a.y), a.ldy, a.norm, \
+      a.self_loop, a.dinv, a.deg_code, a.threshold, a.row_offset, a.ra, sched)
+  constexpr bool F32 = std::is_same<Tin, float>::value && std::is_same<Tout, float>::value;
+  if (F32 && a.ra.ex.n > 0) {  // (the bf16 entry has no extra partial sums)
     if (VEC != 4) return fail(WDGH_EINVAL, "wdgh_spmm_csr_ranged: extra partial sums need d >= 128");
-    if (full) WDGH_RG_LAUNCH(true, MINB, (VEC == 4));
-    else WDGH_RG_LAUNCH(false, 16, (VEC == 4));
+    if (full) WDGH_RG_LAUNCH(true, MINB, (F32 && VEC == 4));
+    else WDGH_RG_LAUNCH(false, 16, (F32 && VEC == 4));
   } else if (full) {
     WDGH_RG_LAUNCH(true, MINB, false);
   } else {
@@ -607,49 +669,51 @@ static int launch_rowgroup(const SpmmArgs &a) {
 
 static bool rowgroup_width(int64_t d) { return d >= 128 || d == 64 || d == 32; }
 
-template <bool HAS_VAL>
+template <bool HAS_VAL, typename Tin = float, typename Tout = float>
 static int dispatch(const SpmmArgs &a, bool vec4) {
   int rc;
   const int d = a.d;
   const ExtraParts none = {0, 0, 0, nullptr};
   if (vec4 && rowgroup_width(d)) {
-    if (d == 32) rc = launch_rowgroup<1, 1, HAS_VAL>(a);
-    else if (d == 64) rc = launch_rowgroup<2, 1, HAS_VAL>(a);
-    else if (d <= 128) rc = launch_rowgroup<4, 1, HAS_VAL>(a);
-    else if (d <= 256) rc = launch_rowgroup<4, 2, HAS_VAL>(a);
-    else rc = launch_rowgroup<4, 4, HAS_VAL>(a);
+    if (d == 32) rc = launch_rowgroup<1, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d == 64) rc = launch_rowgroup<2, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 128) rc = launch_rowgroup<4, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 256) rc = launch_rowgroup<4, 2, HAS_VAL, Tin, Tout>(a);
+    else rc = launch_rowgroup<4, 4, HAS_VAL, Tin, Tout>(a);
     if (rc || !a.heavy_pass) return rc;
-    if (d <= 128) return launch_heavy<4, 1, HAS_VAL>(a, none);
-    if (d <= 256) return launch_heavy<4, 2, HAS_VAL>(a, none);
-    return launch_heavy<4, 4, HAS_VAL>(a, none);
+    if (d <= 128) return launch_heavy<4, 1, HAS_VAL, Tin, Tout>(a, none);
+    if (d <= 256) return launch_heavy<4, 2, HAS_VAL, Tin, Tout>(a, none);
+    return launch_heavy<4, 4, HAS_VAL, Tin, Tout>(a, none);
   }
   if (vec4) {
-    if (d <= 4) rc = launch_rows<1, 4, 1, HAS_VAL>(a);
-    else if (d <= 8) rc = launch_rows<2, 4, 1, HAS_VAL>(a);
-    else if (d <= 16) rc = launch_rows<4, 4, 1, HAS_VAL>(a);
-    else if (d <= 32) rc = launch_rows<8, 4, 1, HAS_VAL>(a);
-    else if (d <= 64) rc = launch_rows<16, 4, 1, HAS_VAL>(a);
-    else rc = launch_rows<32, 4, 1, HAS_VAL>(a);
+    if (d <= 4) rc = launch_rows<1, 4, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 8) rc = launch_rows<2, 4, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 16) rc = launch_rows<4, 4, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 32) rc = launch_rows<8, 4, 1, HAS_VAL, Tin, Tout>(a);
+    else if (d <= 64) rc = launch_rows<16, 4, 1, HAS_VAL, Tin, Tout>(a);
+    else rc = launch_rows<32, 4, 1, HAS_VAL, Tin, Tout>(a);
     if (rc) return rc;
-    return launch_heavy<4, 1, HAS_VAL>(a, none);
+    return launch_heavy<4, 1, HAS_VAL, Tin, Tout>(a, none);
   }
-  if (d <= 1) rc = launch_rows<1, 1, 1, HAS_VAL>(a);
-  else if (d <= 2) rc = launch_rows<2, 1, 1, HAS_VAL>(a);
-  else if (d <= 4) rc = launch_rows<4, 1, 1, HAS_VAL>(a);
-  else if (d <= 8) rc = launch_rows<8, 1, 1, HAS_VAL>(a);
-  else if (d <= 16) rc = launch_rows<16, 1, 1, HAS_VAL>(a);
-  else if (d <= 32) rc = launch_rows<32, 1, 1, HAS_VAL>(a);
-  else if (d <= 64) rc = launch_rows<32, 1, 2, HAS_VAL>(a);
-  else rc = launch_rows<32, 1, 4, HAS_VAL>(a);
+  if (d <= 1) rc = launch_rows<1, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 2) rc = launch_rows<2, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 4) rc = launch_rows<4, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 8) rc = launch_rows<8, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 16) rc = launch_rows<16, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 32) rc = launch_rows<32, 1, 1, HAS_VAL, Tin, Tout>(a);
+  else if (d <= 64) rc = launch_rows<32, 1, 2, HAS_VAL, Tin, Tout>(a);
+  else rc = launch_rows<32, 1, 4, HAS_VAL, Tin, Tout>(a);
   if (rc) return rc;
-  if (d <= 32) return launch_heavy<1, 1, HAS_VAL>(a, none);
-  if (d <= 64) return launch_heavy<1, 2, HAS_VAL>(a, none);
-  return launch_heavy<1, 4, HAS_VAL>(a, none);
+  if (d <= 32) return launch_heavy<1, 1, HAS_VAL, Tin, Tout>(a, none);
+  if (d <= 64) return launch_heavy<1, 2, HAS_VAL, Tin, Tout>(a, none);
+  return launch_heavy<1, 4, HAS_VAL, Tin, Tout>(a, none);
 }
 
-static bool rows_vec4(const float *x, int64_t d, int64_t ldx, const float *y, int64_t ldy, const float *partial) {
-  return (d % 4 == 0) && (ldx % 4 == 0) && (ldy % 4 == 0) && (reinterpret_cast<uintptr_t>(x) % 16 == 0) &&
-         (reinterpret_cast<uintptr_t>(y) % 16 == 0) &&
+// every row of x / y starts on a 4-element boundary (16 bytes for fp32, 8 for bf16)
+template <typename Tin, typename Tout>
+static bool rows_vec4(const Tin *x, int64_t d, int64_t ldx, const Tout *y, int64_t ldy, const float *partial) {
+  return (d % 4 == 0) && (ldx % 4 == 0) && (ldy % 4 == 0) && (reinterpret_cast<uintptr_t>(x) % (4 * sizeof(Tin)) == 0) &&
+         (reinterpret_cast<uintptr_t>(y) % (4 * sizeof(Tout)) == 0) &&
          (partial == nullptr || reinterpret_cast<uintptr_t>(partial) % 16 == 0);
 }
 
@@ -657,16 +721,28 @@ static bool rows_vec4(const float *x, int64_t d, int64_t ldx, const float *y, in
 
 using namespace wdgh;
 
-extern "C" int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
-                             const float *x, int64_t d, int64_t ldx, float *y, int64_t ldy, int norm,
-                             int add_self_loop, const float *dinv, const uint8_t *deg_code, int64_t *plan_i64,
-                             const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
-  WDGH_REQUIRE(rowptr && x && y && plan_i64 && plan_host, "wdgh_spmm_csr: null pointer");  // col may be NULL iff nnz == 0
-  WDGH_REQUIRE(n >= 0 && d > 0 && d <= (1 << 24) && ldx >= d && ldy >= d, "wdgh_spmm_csr: bad shape");
-  WDGH_REQUIRE(norm == WDGH_NORM_NONE || norm == WDGH_NORM_RW || norm == WDGH_NORM_SYM, "wdgh_spmm_csr: bad norm");
-  WDGH_REQUIRE(norm == WDGH_NORM_NONE || dinv != nullptr, "wdgh_spmm_csr: norm requires dinv");
-  WDGH_REQUIRE(x != y, "wdgh_spmm_csr: in-place aggregation is not supported");
-  WDGH_REQUIRE(row_offset >= 0, "wdgh_spmm_csr: negative row_offset");
+namespace wdgh {
+// argument checks and dispatch shared by wdgh_spmm_csr (Tin = float) and wdgh_spmm_csr_bf16; `fn` names the entry in
+// the error messages
+#define WDGH_REQUIRE_AT(cond, what)                                      \
+  do {                                                                   \
+    if (!(cond)) {                                                       \
+      snprintf(g_err, sizeof(g_err), "%s: %s", fn, what);                \
+      return WDGH_EINVAL;                                                \
+    }                                                                    \
+  } while (0)
+template <typename Tin>
+static int spmm_csr(const char *fn, const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                    const Tin *x, int64_t d, int64_t ldx, void *y, int64_t ldy, int y_dtype, int norm,
+                    int add_self_loop, const float *dinv, const uint8_t *deg_code, int64_t *plan_i64,
+                    const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  WDGH_REQUIRE_AT(rowptr && x && y && plan_i64 && plan_host, "null pointer");  // col may be NULL iff nnz == 0
+  WDGH_REQUIRE_AT(n >= 0 && d > 0 && d <= (1 << 24) && ldx >= d && ldy >= d, "bad shape");
+  WDGH_REQUIRE_AT(norm == WDGH_NORM_NONE || norm == WDGH_NORM_RW || norm == WDGH_NORM_SYM, "bad norm");
+  WDGH_REQUIRE_AT(norm == WDGH_NORM_NONE || dinv != nullptr, "norm requires dinv");
+  WDGH_REQUIRE_AT(static_cast<const void *>(x) != y, "in-place aggregation is not supported");
+  WDGH_REQUIRE_AT(row_offset >= 0, "negative row_offset");
+  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == WDGH_DTYPE_BF16, "bad y_dtype");
   if (n == 0) return 0;
   SpmmArgs a;
   a.rowptr = rowptr; a.col = col; a.val = val; a.n = n; a.x = x; a.d = (int)d; a.ldx = ldx; a.y = y; a.ldy = ldy;
@@ -675,9 +751,34 @@ extern "C" int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const fl
   a.partial = partial; a.ldp = (d + 3) & ~int64_t(3);
   a.row_offset = row_offset;
   a.st = as_stream(stream);
-  WDGH_REQUIRE(a.n_chunks == 0 || partial != nullptr, "wdgh_spmm_csr: split rows need the partial buffer");
-  const bool vec4 = rows_vec4(x, d, ldx, y, ldy, partial);
-  return val ? dispatch<true>(a, vec4) : dispatch<false>(a, vec4);
+  WDGH_REQUIRE_AT(a.n_chunks == 0 || partial != nullptr, "split rows need the partial buffer");
+  if constexpr (!std::is_same<Tin, float>::value) {  // (fp32 features have fp32 output only)
+    if (y_dtype == WDGH_DTYPE_BF16) {
+      const bool vec4 = rows_vec4(x, d, ldx, static_cast<const bf16 *>(y), ldy, partial);
+      return val ? dispatch<true, Tin, bf16>(a, vec4) : dispatch<false, Tin, bf16>(a, vec4);
+    }
+  }
+  const bool vec4 = rows_vec4(x, d, ldx, static_cast<const float *>(y), ldy, partial);
+  return val ? dispatch<true, Tin, float>(a, vec4) : dispatch<false, Tin, float>(a, vec4);
+}
+#undef WDGH_REQUIRE_AT
+}  // namespace wdgh
+
+extern "C" int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                             const float *x, int64_t d, int64_t ldx, float *y, int64_t ldy, int norm,
+                             int add_self_loop, const float *dinv, const uint8_t *deg_code, int64_t *plan_i64,
+                             const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  return spmm_csr("wdgh_spmm_csr", rowptr, col, val, n, x, d, ldx, y, ldy, WDGH_DTYPE_F32, norm, add_self_loop, dinv,
+                  deg_code, plan_i64, plan_host, partial, row_offset, stream);
+}
+
+extern "C" int wdgh_spmm_csr_bf16(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                                  const uint16_t *x, int64_t d, int64_t ldx, void *y, int64_t ldy, int y_dtype,
+                                  int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                                  int64_t *plan_i64, const int64_t *plan_host, float *partial, int64_t row_offset,
+                                  void *stream) {
+  return spmm_csr("wdgh_spmm_csr_bf16", rowptr, col, val, n, reinterpret_cast<const bf16 *>(x), d, ldx, y, ldy, y_dtype,
+                  norm, add_self_loop, dinv, deg_code, plan_i64, plan_host, partial, row_offset, stream);
 }
 
 extern "C" int wdgh_structure_counts(const int64_t *, const int32_t *, int64_t, int64_t, const int32_t *, int32_t,

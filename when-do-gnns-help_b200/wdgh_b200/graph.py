@@ -194,15 +194,34 @@ class CSRGraph:
 # ---------------------------------------------------------------------------
 # A_hat X aggregation
 # ---------------------------------------------------------------------------
-def spmm(g: CSRGraph, x, norm=NORM_NONE, add_self_loop=False, out=None, dinv=None, deg_code=None):
-    """y = norm(A [+I]) x in float32 on the GPU (hm.py:192,199,234; util_funcs.py:383-390,418-426).
+def spmm(g: CSRGraph, x, norm=NORM_NONE, add_self_loop=False, out=None, dinv=None, deg_code=None, out_dtype=None):
+    """y = norm(A [+I]) x on the GPU with fp32 accumulation (hm.py:192,199,234; util_funcs.py:383-390,418-426).
 
+    A bfloat16 `x` is read as it is (no fp32 copy); its result is bit-identical to the one of `x.float()`.  The result
+    has the dtype of `out` if given, else `out_dtype`, else float32; bfloat16 output (round to nearest even) needs
+    bfloat16 features.  Any other `x` dtype is converted to float32 first.
     For a row shard `x` (and `dinv`, the all-gathered degree scale) are global, the result is local."""
-    x = _cuda(x, torch.float32)
+    bf16 = isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16
+    if out is not None:
+        if out_dtype is not None and out_dtype != out.dtype:
+            raise ValueError(f"out has dtype {out.dtype}, out_dtype asks for {out_dtype}")
+        out_dtype = out.dtype
+    out_dtype = torch.float32 if out_dtype is None else out_dtype
+    if out_dtype not in ((torch.float32, torch.bfloat16) if bf16 else (torch.float32,)):
+        raise ValueError(f"cannot write a {out_dtype} result from {x.dtype if bf16 else 'float32'} features "
+                         "(float32 output; bfloat16 output needs bfloat16 features)")
+    if bf16:
+        # views with a unit column stride and whole rows apart (a column slab of a wider matrix) are read in place;
+        # any other layout (transposed, broadcast rows) is copied like the float32 path does
+        x = x.to(_dev(), non_blocking=True) if x.device.type != "cuda" else x
+        if x.dim() == 2 and (x.stride(1) != 1 or x.stride(0) < x.shape[1]):
+            x = x.new_empty(x.shape).copy_(x)   # (not .contiguous(): a [1, d] view with row stride 1 counts as such)
+    else:
+        x = _cuda(x, torch.float32)
     if x.dim() != 2 or x.shape[0] < g.n_global or (x.shape[0] != g.n_global and g.n_global == g.n):
         raise ValueError(f"features must be [n={g.n_global}, d], got {tuple(x.shape)}")
     d = int(x.shape[1])
-    y = out if out is not None else torch.empty((g.n, d), dtype=torch.float32, device=g.device)
+    y = out if out is not None else torch.empty((g.n, d), dtype=out_dtype, device=g.device)
     if y.shape != (g.n, d) or y.stride(1) != 1:
         raise ValueError("out must be [n, d] with unit column stride (a column slab of a wider matrix is fine)")
     plan, plan_host = g.plan
@@ -211,6 +230,13 @@ def spmm(g: CSRGraph, x, norm=NORM_NONE, add_self_loop=False, out=None, dinv=Non
         if g.n_global != g.n:
             raise ValueError("a row shard needs the all-gathered degree scale (dinv=...)")
         dinv, _, deg_code = g.degree_scale(norm, add_self_loop)
+    if bf16:
+        y_dtype = _lib.DTYPE_BF16 if out_dtype == torch.bfloat16 else _lib.DTYPE_F32
+        check(lib.wdgh_spmm_csr_bf16(ptr(g.rowptr), ptr(g.col), ptr(g.val), g.n, ptr(x), d, x.stride(0), ptr(y),
+                                     y.stride(0), y_dtype, norm, int(bool(add_self_loop)), ptr(dinv), ptr(deg_code),
+                                     ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()),
+              "wdgh_spmm_csr_bf16")
+        return y
     check(lib.wdgh_spmm_csr(ptr(g.rowptr), ptr(g.col), ptr(g.val), g.n, ptr(x), d, x.stride(0), ptr(y), y.stride(0),
                             norm, int(bool(add_self_loop)), ptr(dinv), ptr(deg_code), ptr(plan), plan_host,
                             ptr(partial), g.row_offset, stream_ptr()), "wdgh_spmm_csr")
