@@ -127,7 +127,7 @@ int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, i
                   int64_t *plan_i64, const int64_t *plan_host, float *partial,
                   int64_t row_offset, void *stream);
 
-/* Element types of wdgh_spmm_csr_bf16's output */
+/* Element types of wdgh_spmm_csr_bf16's and wdgh_pipeline_host_bf16's output */
 #define WDGH_DTYPE_F32  0
 #define WDGH_DTYPE_BF16 1
 /* wdgh_spmm_csr with a bfloat16 feature matrix (raw bf16 bits), fp32 accumulation, y float32 or bf16 (y_dtype).
@@ -173,6 +173,18 @@ int wdgh_spmm_csr_ranged(const int64_t *rowptr, const int64_t *range_begin, cons
                          int64_t extra_part_rows, int64_t ld_extra, int32_t ctas_per_sm,
                          int64_t *plan_i64, const int64_t *plan_host, float *partial,
                          int64_t row_offset, void *stream);
+/* wdgh_spmm_csr_ranged with a bfloat16 feature matrix (raw bf16 bits, ldx in elements) and float32 y: every phase
+ * accumulates in fp32 and stores fp32 (raw partial sums are never rounded), so each call is bit-identical to
+ * wdgh_spmm_csr_ranged on the upcast matrix with the same arguments.  No extra partial sums and no ctas_per_sm (the
+ * 2-D multi-GPU partition is fp32).  Needs rows on 8-byte boundaries (d and ldx multiples of 4) and d in {32, 64} or
+ * d >= 128. */
+int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                              const int32_t *col, const float *val, int64_t n,
+                              const uint16_t *x, int64_t d, int64_t ldx, float *y, int64_t ldy,
+                              int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                              const uint8_t *skip_rows, int accumulate, int finalize, int run_split_rows,
+                              int64_t *plan_i64, const int64_t *plan_host, float *partial,
+                              int64_t row_offset, void *stream);
 
 /* ---- label metrics: one pass over the edges ------------------------------ */
 /* Integer statistics every label metric of homophily_metrics.py is a ratio of
@@ -293,7 +305,16 @@ int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col_host, int6
                        const float *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
                        int norm, int add_self_loop,
                        float *y_host, int64_t *counters_host, double *node_sum_host);
-/* free the buffers cached by wdgh_pipeline_host */
+/* wdgh_pipeline_host with a bfloat16 feature matrix (raw bf16 bits, [n][d] contiguous): half the bytes of X on the
+ * link.  y_host (NULL = counters only) is [n][d] of y_dtype: WDGH_DTYPE_F32, or WDGH_DTYPE_BF16 (half the bytes back).
+ * Aggregation is fp32; a bf16 Y is the fp32 Y of the same call rounded to nearest even.  The copy / compute schedule
+ * depends on (n, nnz, d, feature type, y_host != NULL), not on y_dtype.  Shares the cached pipeline (and
+ * wdgh_pipeline_host_release) with wdgh_pipeline_host.  SYNCHRONOUS. */
+int wdgh_pipeline_host_bf16(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                            const uint16_t *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
+                            int norm, int add_self_loop,
+                            void *y_host, int y_dtype, int64_t *counters_host, double *node_sum_host);
+/* free the buffers cached by wdgh_pipeline_host / wdgh_pipeline_host_bf16 */
 int wdgh_pipeline_host_release(void);
 
 #ifdef __cplusplus

@@ -1,0 +1,166 @@
+#!/usr/bin/env python
+"""Host-buffer pipeline (the e2e path) with bf16 features against fp32 features on the headline graph (BASELINE.json
+configs[4], bench.gen_rows): 50M nodes, ~976M stored entries, d = 128, 10 classes, Y = D^-1/2 (A+I) D^-1/2 X.
+
+    python tools/e2e_bf16_bench.py [--reps 5] [--warmup 1] [--out profiles/e2e_bf16_r04.json]
+
+X is drawn in fp32 by the generator and cast to bf16 once; the fp32 arms read Xb.float(), so every arm moves the same
+values.  All inputs and outputs live in pinned host memory (about 80 GB at full size).  Timed in one process with a host
+clock around the synchronous call, the arms alternating within every repetition:
+    e2e_f32          wdgh_pipeline_host, fp32 X, fp32 Y back          (what bench.py's e2e times)
+    e2e_bf16_f32y    wdgh_pipeline_host_bf16, bf16 X, fp32 Y back
+    e2e_bf16_bf16y   wdgh_pipeline_host_bf16, bf16 X, bf16 Y back
+    counters_f32     wdgh_pipeline_host, fp32 X, counters only (y_host = NULL)
+    counters_bf16    wdgh_pipeline_host_bf16, bf16 X, counters only
+Per arm: median ms and spread, GEdges/s, H2D / D2H bytes and the effective link rate ((H2D + D2H) / time).
+Checks in the same run: the counters of every arm are identical; on a seeded sample of rows, the fp32 Y of the bf16
+features equals the fp32 Y of e2e_f32 exactly (both feature types take the same copy / compute form, whose phases are
+bit-identical), and the bf16 Y equals the fp32 Y of the bf16 features rounded to nearest even.  Prints one JSON line,
+writes it to --out and exits non-zero when a check fails.  WDGH_E2E_COLW (0 = row blocks, 64 = column blocks) selects
+the form of the Y-returning arms for both feature types.
+"""
+import argparse
+import json
+import os
+import statistics
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+for _p in (ROOT, os.path.join(ROOT, "when-do-gnns-help_b200"), os.path.join(ROOT, "tools")):
+    if _p not in sys.path:
+        sys.path.insert(0, _p)
+
+import torch  # noqa: E402
+
+import bench  # noqa: E402
+from bf16_bench import card  # noqa: E402
+
+HEADLINE_NODES = 50_000_000
+
+
+def column_blocks(d):
+    """True when the Y-returning form of the pipeline uses column blocks (csrc/pipeline_host.cu, e2e_col_width)"""
+    env = os.environ.get("WDGH_E2E_COLW")
+    w = int(env) if env in ("0", "32", "64") else 64
+    return w > 0 and d % w == 0 and 2 <= d // w <= 64
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--nodes", type=int, default=HEADLINE_NODES)
+    ap.add_argument("--avg-degree", type=float, default=20.0)
+    ap.add_argument("--dim", type=int, default=128)
+    ap.add_argument("--classes", type=int, default=10)
+    ap.add_argument("--homophily", type=float, default=0.3)
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--warmup", type=int, default=1)
+    ap.add_argument("--sample-rows", type=int, default=1 << 20)
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "e2e_bf16_r04.json"))
+    args = ap.parse_args()
+
+    import wdgh_b200 as W
+    from wdgh_b200 import graph as G
+
+    W._lib.require_device()
+    device = torch.device("cuda", torch.cuda.current_device())
+    n, d, C = args.nodes, args.dim, args.classes
+    rowptr, col, x, labels = bench.gen_rows(0, n, n, args.avg_degree, C, args.homophily, d, device)
+    nnz = int(col.shape[0])
+    xb = x.to(torch.bfloat16)
+    del x
+
+    def pinned(t, dtype=None):
+        h = torch.empty(t.shape, dtype=dtype or t.dtype, pin_memory=True)
+        for r in range(0, t.shape[0], 1 << 22):   # row blocks: no full-size device temporary for the fp32 copy
+            h[r:r + (1 << 22)].copy_(t[r:r + (1 << 22)])
+        return h
+
+    try:
+        rowptr_h, col_h = pinned(rowptr), pinned(col)
+        lab_h = pinned(labels, torch.int32)
+        xb_h, x32_h = pinned(xb), pinned(xb, torch.float32)
+        y32_h = torch.empty((n, d), dtype=torch.float32, pin_memory=True)
+        ybf_h = torch.empty((n, d), dtype=torch.bfloat16, pin_memory=True)
+    except RuntimeError as e:
+        print(json.dumps({"tool": "tools/e2e_bf16_bench.py", "nodes": n,
+                          "error": f"pinning the host buffers failed ({str(e)[:120]}); run again with a smaller --nodes"}),
+              flush=True)
+        sys.exit(2)
+    del rowptr, col, labels, xb
+    torch.cuda.empty_cache()
+
+    n_cnt = W._lib.sc_words(C)
+    small_d2h = n_cnt * 8 + 16
+    graph_h2d = (n + 1) * 8 + nnz * 4 + n * 4
+    counters = {}
+
+    def run(k, x_h, y_h):
+        counters[k] = G.pipeline_host(rowptr_h, col_h, x_h, lab_h, C, W.NORM_SYM, True, y=y_h)
+
+    arms = {
+        "e2e_f32": (x32_h, y32_h),
+        "e2e_bf16_f32y": (xb_h, y32_h),
+        "e2e_bf16_bf16y": (xb_h, ybf_h),
+        "counters_f32": (x32_h, None),
+        "counters_bf16": (xb_h, None),
+    }
+    for _ in range(args.warmup):
+        for k, (xh, yh) in arms.items():
+            run(k, xh, yh)
+    times = {k: [] for k in arms}
+    for _ in range(args.reps):
+        for k, (xh, yh) in arms.items():
+            t0 = time.perf_counter()
+            run(k, xh, yh)
+            times[k].append(time.perf_counter() - t0)
+
+    # checks: counters of the last timed call of every arm; Y on a seeded row sample of one more call per Y arm
+    ref_c, ref_s = counters["e2e_f32"]
+    counters_equal = all((c == ref_c).all() and (s == ref_s).all() for c, s in counters.values())
+    gen = torch.Generator().manual_seed(7)
+    rows = torch.randint(0, n, (min(args.sample_rows, n),), generator=gen)
+    run("e2e_f32", x32_h, y32_h)
+    y_f32 = y32_h[rows].clone()
+    run("e2e_bf16_f32y", xb_h, y32_h)
+    y_bf = y32_h[rows].clone()
+    run("e2e_bf16_bf16y", xb_h, ybf_h)
+    y_bfbf = ybf_h[rows].clone()
+    scale = y_f32.abs().max().item()
+    err = (y_bf - y_f32).abs().max().item()
+    y_ok = torch.equal(y_bf, y_f32)
+    bf16_ok = torch.equal(y_bfbf, y_bf.to(torch.bfloat16))
+    W._lib.lib.wdgh_pipeline_host_release()
+
+    x_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 2, "e2e_bf16_bf16y": 2, "counters_f32": 4, "counters_bf16": 2}
+    y_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 4, "e2e_bf16_bf16y": 2, "counters_f32": 0, "counters_bf16": 0}
+    res = {}
+    for k, ts in times.items():
+        ms = statistics.median(ts) * 1e3
+        h2d = graph_h2d + n * d * x_bytes[k]
+        d2h = small_d2h + n * d * y_bytes[k]
+        form = "column blocks" if y_bytes[k] and column_blocks(d) else "row blocks"
+        res[k] = {"ms": ms, "ms_min": min(ts) * 1e3, "ms_max": max(ts) * 1e3, "gedges_s": nnz / (ms * 1e-3) / 1e9,
+                  "h2d_bytes": h2d, "d2h_bytes": d2h, "link_gbs": (h2d + d2h) / (ms * 1e-3) / 1e9, "form": form}
+    line = {"tool": "tools/e2e_bf16_bench.py", "nodes": n, "headline_graph": n == HEADLINE_NODES,
+            "stored_entries": nnz, "dim": d, "classes": C, "norm": "sym D^-1/2 (A+I) D^-1/2 on the fly",
+            "reps": args.reps, "warmup": args.warmup, "timer": "host clock around the synchronous call",
+            "host_memory": "pinned", "e2e_colw_env": os.environ.get("WDGH_E2E_COLW"), "arms": res,
+            "speedup_e2e_bf16_f32y": res["e2e_f32"]["ms"] / res["e2e_bf16_f32y"]["ms"],
+            "speedup_e2e_bf16_bf16y": res["e2e_f32"]["ms"] / res["e2e_bf16_bf16y"]["ms"],
+            "speedup_counters_bf16": res["counters_f32"]["ms"] / res["counters_bf16"]["ms"],
+            "check_counters_identical": bool(counters_equal), "check_sample_rows": int(rows.shape[0]),
+            "check_y_f32_max_abs_err": err, "check_y_max_abs": scale,
+            "check_y_f32": bool(y_ok), "check_y_bf16_is_rounded_f32": bool(bf16_ok), "card": card(device)}
+    text = json.dumps(line)
+    print(text, flush=True)
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write(text + "\n")
+    if not (counters_equal and y_ok and bf16_ok):
+        sys.exit(3)
+
+
+if __name__ == "__main__":
+    main()

@@ -19,20 +19,32 @@
 // tools/colblock_probe.py) phased by arriving row chunk exactly like the counters-only form, so that only the last
 // chunk's phase separates the end of a block's H2D copy from the start of its D2H copy, and the D2H copy of block k
 // runs under the H2D copy of block k + 1.
+//
+// bfloat16 features (wdgh_pipeline_host_bf16) take the same body with the bf16 aggregation entries: half the bytes of
+// X on the link, fp32 phases (a phase is bit-identical to the fp32 phase on the upcast matrix).  Y is always
+// aggregated in fp32 into the device Y buffer; for a bf16 Y the last phase of a block is followed by a rounding pass
+// into a bf16 staging buffer, which the D2H copy reads -- so a bf16 Y is exactly the rounding of the fp32 Y of the
+// same schedule, and the schedule does not depend on the type of Y.
 #include <stdlib.h>
 
 #include <mutex>
+#include <type_traits>
 
-#include "common.cuh"
+#include "internal.cuh"
 
 namespace wdgh {
 
 struct HostPipelineCache {
   int64_t n = -1, nnz = -1, d = -1, cap = -1, partial_elems = 0;
   int C = -1, device = -1;
+  // The feature buffer is sized in bytes and grows when a call needs more (an fp32 call after a bf16 one); a bf16 call
+  // after an fp32 one reuses it, so a caller alternating feature types does not reallocate the largest buffer.
+  size_t x_bytes = 0, ystage_bytes = 0;
   int64_t *rowptr = nullptr;
   int32_t *col = nullptr;
-  float *x = nullptr, *y = nullptr, *dinv = nullptr, *partial = nullptr;
+  void *x = nullptr;
+  float *y = nullptr, *dinv = nullptr, *partial = nullptr;
+  void *ystage = nullptr;  // bf16 Y rounded for the D2H copy (allocated by the first bf16-Y call)
   int32_t *labels = nullptr, *deg = nullptr, *match = nullptr;
   uint8_t *labels8 = nullptr, *deg_code = nullptr;
   int64_t *plan = nullptr, *counters = nullptr;
@@ -48,7 +60,7 @@ struct HostPipelineCache {
     if (ev_csr) cudaEventDestroy(ev_csr);
     for (auto &e : ev_x) if (e) cudaEventDestroy(e);
     for (auto &e : ev_y) if (e) cudaEventDestroy(e);
-    cudaFree(rowptr); cudaFree(col); cudaFree(x); cudaFree(y); cudaFree(dinv); cudaFree(partial);
+    cudaFree(rowptr); cudaFree(col); cudaFree(x); cudaFree(y); cudaFree(ystage); cudaFree(dinv); cudaFree(partial);
     cudaFree(labels); cudaFree(labels8); cudaFree(deg_code); cudaFree(deg); cudaFree(match); cudaFree(plan); cudaFree(counters); cudaFree(node_sum);
     if (st) cudaStreamDestroy(st);
     *this = HostPipelineCache();
@@ -69,9 +81,13 @@ static int e2e_chunks() {
   return cached;
 }
 
-// Width (floats) of the column blocks of the Y-returning form, 0 = row-block form.  64 floats = 256-byte rows: the
+// Width (elements) of the column blocks of the Y-returning form, 0 = row-block form.  64 floats = 256-byte rows: the
 // narrowest pitched copy that still runs at the full PCIe rate in both directions (128-byte rows: 34 + 40 GB/s), and a
 // width the row-group aggregation kernel runs natively.  WDGH_E2E_COLW overrides (0, 32 or 64).
+// bf16 features take the same 64 columns, i.e. 128-byte rows (the slower pitched copy): measured on the 50M-node /
+// 976M-entry graph at d = 128 (tools/e2e_bf16_bench.py, NVIDIA B200, 1000 W power limit, each form in its own process),
+// column blocks 735.7 ms with fp32 Y back and 536.8 ms with bf16 Y back, against 795.1 / 578.3 ms for row blocks (full-rate
+// contiguous H2D, Y copied after the last phase).
 static int64_t e2e_col_width(int64_t d) {
   static int cached = -1;
   if (cached < 0) {
@@ -98,22 +114,23 @@ static int e2e_col_rows() {
   return cached;
 }
 
-}  // namespace wdgh
+#define WDGH_REQUIRE_AT(cond, what)                                      \
+  do {                                                                   \
+    if (!(cond)) {                                                       \
+      snprintf(g_err, sizeof(g_err), "%s: %s", fn, what);                \
+      return WDGH_EINVAL;                                                \
+    }                                                                    \
+  } while (0)
 
-using namespace wdgh;
-
-extern "C" int wdgh_pipeline_host_release(void) {
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  g_cache.release();
-  return 0;
-}
-
-extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
-                                  const float *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
-                                  int norm, int add_self_loop, float *y_host, int64_t *counters_host,
-                                  double *node_sum_host) {
-  WDGH_REQUIRE(rowptr_host && x_host && labels_host && counters_host && node_sum_host, "wdgh_pipeline_host: null pointer");
-  WDGH_REQUIRE(n > 0 && nnz >= 0 && d > 0 && num_classes >= 1 && (col_host || nnz == 0), "wdgh_pipeline_host: bad shape");
+// The body of wdgh_pipeline_host (Tin = float) and wdgh_pipeline_host_bf16 (Tin = uint16_t, raw bf16 bits).
+template <typename Tin>
+static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                         const Tin *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes, int norm,
+                         int add_self_loop, void *y_host, int y_dtype, int64_t *counters_host, double *node_sum_host) {
+  constexpr bool F32 = std::is_same<Tin, float>::value;
+  WDGH_REQUIRE_AT(rowptr_host && x_host && labels_host && counters_host && node_sum_host, "null pointer");
+  WDGH_REQUIRE_AT(n > 0 && nnz >= 0 && d > 0 && num_classes >= 1 && (col_host || nnz == 0), "bad shape");
+  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == WDGH_DTYPE_BF16, "bad y_dtype");
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached buffers and streams serve one call at a time
   HostPipelineCache &c = g_cache;
   const int C = num_classes;
@@ -126,7 +143,6 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
     WDGH_CUDA(cudaStreamCreateWithFlags(&c.st, cudaStreamNonBlocking));
     WDGH_CUDA(cudaMalloc(&c.rowptr, (n + 1) * sizeof(int64_t)));
     WDGH_CUDA(cudaMalloc(&c.col, (nnz > 0 ? nnz : 1) * sizeof(int32_t)));
-    WDGH_CUDA(cudaMalloc(&c.x, n * d * sizeof(float)));
     WDGH_CUDA(cudaMalloc(&c.y, n * d * sizeof(float)));
     WDGH_CUDA(cudaMalloc(&c.dinv, n * sizeof(float)));
     WDGH_CUDA(cudaMalloc(&c.labels, n * sizeof(int32_t)));
@@ -147,6 +163,23 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
     WDGH_CUDA(cudaMalloc(&c.skip, (size_t)n));
     c.n = n; c.nnz = nnz; c.d = d; c.C = C; c.cap = cap; c.device = device;
   }
+  if (c.x_bytes < (size_t)(n * d) * sizeof(Tin)) {
+    cudaFree(c.x);
+    c.x = nullptr;
+    c.x_bytes = 0;
+    WDGH_CUDA(cudaMalloc(&c.x, (size_t)(n * d) * sizeof(Tin)));
+    c.x_bytes = (size_t)(n * d) * sizeof(Tin);
+  }
+  const bool y16 = y_host && y_dtype == WDGH_DTYPE_BF16;
+  if (y16 && c.ystage_bytes < (size_t)(n * d) * 2) {
+    cudaFree(c.ystage);
+    c.ystage = nullptr;
+    c.ystage_bytes = 0;
+    WDGH_CUDA(cudaMalloc(&c.ystage, (size_t)(n * d) * 2));
+    c.ystage_bytes = (size_t)(n * d) * 2;
+  }
+  const size_t ysz = y16 ? 2 : sizeof(float);  // bytes of one element of Y on the host
+  Tin *x = static_cast<Tin *>(c.x);
   cudaStream_t st = c.st, sc = c.st_copy, sb = c.st_back;
   const bool ranged_ok = (d % 4 == 0) && (d >= 128 || d == 64 || d == 32);
   const int64_t colw = y_host ? e2e_col_width(d) : 0;   // > 0: column-block form (Y travels back under the X copies)
@@ -168,15 +201,15 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
     for (int r = 0; r < R; ++r) {
       const int64_t r0 = bounds_h[r], r1 = (r0 + blk < n) ? r0 + blk : n;
       if (r1 > r0)
-        WDGH_CUDA(cudaMemcpy2DAsync(c.x + r0 * d + kc * colw, d * sizeof(float), x_host + r0 * d + kc * colw,
-                                    d * sizeof(float), colw * sizeof(float), r1 - r0, cudaMemcpyHostToDevice, sc));
+        WDGH_CUDA(cudaMemcpy2DAsync(x + r0 * d + kc * colw, d * sizeof(Tin), x_host + r0 * d + kc * colw,
+                                    d * sizeof(Tin), colw * sizeof(Tin), r1 - r0, cudaMemcpyHostToDevice, sc));
       WDGH_CUDA(cudaEventRecord(c.ev_x[kc * R + r], sc));
     }
   }
   for (int k = 0; k < K && !colw; ++k) {
     const int64_t r0 = bounds_h[k], r1 = (r0 + blk < n) ? r0 + blk : n;
     if (r1 > r0)
-      WDGH_CUDA(cudaMemcpyAsync(c.x + r0 * d, x_host + r0 * d, (size_t)(r1 - r0) * d * sizeof(float),
+      WDGH_CUDA(cudaMemcpyAsync(x + r0 * d, x_host + r0 * d, (size_t)(r1 - r0) * d * sizeof(Tin),
                                 cudaMemcpyHostToDevice, sc));
     WDGH_CUDA(cudaEventRecord(c.ev_x[k], sc));
   }
@@ -199,13 +232,33 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
   }
   const float *dinv = norm != WDGH_NORM_NONE ? c.dinv : nullptr;
   const uint8_t *code = norm != WDGH_NORM_NONE ? c.deg_code : nullptr;
+  // one launch over every row of a column slab of width w (fp32 Y)
+  auto full = [&](const Tin *xb, int64_t w, float *yb) -> int {
+    if constexpr (F32)
+      return wdgh_spmm_csr(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv, code, c.plan,
+                           plan_host, c.partial, 0, st);
+    else
+      return wdgh_spmm_csr_bf16(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, WDGH_DTYPE_F32, norm, add_self_loop, dinv,
+                                code, c.plan, plan_host, c.partial, 0, st);
+  };
+  // the phase of row block k: y (+)= the entries whose column lies in block k; the last phase finalizes
+  auto phase = [&](int k, const Tin *xb, int64_t w, float *yb, int accumulate, int last) -> int {
+    const int64_t *b = c.seg + (size_t)k * n, *e = c.seg + (size_t)(k + 1) * n;
+    if constexpr (F32)
+      return wdgh_spmm_csr_ranged(c.rowptr, b, e, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv, code,
+                                  c.skip, accumulate, last, last, nullptr, 0, 0, 0, 0, 0, c.plan, plan_host, c.partial,
+                                  0, st);
+    else
+      return wdgh_spmm_csr_ranged_bf16(c.rowptr, b, e, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv,
+                                       code, c.skip, accumulate, last, last, c.plan, plan_host, c.partial, 0, st);
+  };
   // 3. label pass: needs only the graph and the labels, runs under the feature copy
   rc = wdgh_structure_counts(c.rowptr, c.col, n, nnz, c.labels, C, c.plan, plan_host, c.counters, c.node_sum, c.deg,
                              c.match, c.labels8, n, 0, st);
   if (rc) return rc;
   if (colw) {
     // 4'. per column block: one aggregation phase per arriving row chunk (R = 1: one full-graph launch); the Y block
-    //     leaves on the third stream as soon as its last phase is done
+    //     leaves on the third stream as soon as its last phase (and, for a bf16 Y, its rounding) is done
     if (R > 1) {
       WDGH_CUDA(cudaMemcpyAsync(c.bounds, bounds_h, (R + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
       rc = wdgh_column_segments(c.rowptr, c.col, n, c.bounds, R + 1, c.seg, st);
@@ -214,30 +267,27 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
       if (rc) return rc;
     }
     for (int kc = 0; kc < KC; ++kc) {
-      const float *xb = c.x + kc * colw;
+      const Tin *xb = x + kc * colw;
       float *yb = c.y + kc * colw;
       for (int r = 0; r < R; ++r) {
         WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[kc * R + r], 0));
-        if (R == 1) {
-          rc = wdgh_spmm_csr(c.rowptr, c.col, nullptr, n, xb, colw, d, yb, d, norm, add_self_loop, dinv, code, c.plan,
-                             plan_host, c.partial, 0, st);
-        } else {
-          const int last = (r == R - 1);
-          rc = wdgh_spmm_csr_ranged(c.rowptr, c.seg + (size_t)r * n, c.seg + (size_t)(r + 1) * n, c.col, nullptr, n, xb,
-                                    colw, d, yb, d, norm, add_self_loop, dinv, code, c.skip, r > 0, last, last, nullptr,
-                                    0, 0, 0, 0, 0, c.plan, plan_host, c.partial, 0, st);
-        }
+        rc = (R == 1) ? full(xb, colw, yb) : phase(r, xb, colw, yb, r > 0, r == R - 1);
         if (rc) return rc;
       }
+      uint16_t *yb16 = y16 ? static_cast<uint16_t *>(c.ystage) + kc * colw : nullptr;
+      if (y16) {
+        rc = round_to_bf16(yb, n, colw, d, yb16, d, st);
+        if (rc) return rc;
+      }
+      const void *src = y16 ? static_cast<const void *>(yb16) : yb;
       WDGH_CUDA(cudaEventRecord(c.ev_y[kc], st));
       WDGH_CUDA(cudaStreamWaitEvent(sb, c.ev_y[kc], 0));
-      WDGH_CUDA(cudaMemcpy2DAsync(y_host + kc * colw, d * sizeof(float), yb, d * sizeof(float), colw * sizeof(float), n,
+      WDGH_CUDA(cudaMemcpy2DAsync(static_cast<char *>(y_host) + kc * colw * ysz, d * ysz, src, d * ysz, colw * ysz, n,
                                   cudaMemcpyDeviceToHost, sb));
     }
   } else if (K == 1) {
     WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[0], 0));
-    rc = wdgh_spmm_csr(c.rowptr, c.col, nullptr, n, c.x, d, d, c.y, d, norm, add_self_loop, dinv, code, c.plan,
-                       plan_host, c.partial, 0, st);
+    rc = full(x, d, c.y);
     if (rc) return rc;
   } else {
     // 4. one aggregation phase per arriving feature block
@@ -248,18 +298,20 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
     if (rc) return rc;
     for (int k = 0; k < K; ++k) {
       WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[k], 0));
-      const int last = (k == K - 1);
-      rc = wdgh_spmm_csr_ranged(c.rowptr, c.seg + (size_t)k * n, c.seg + (size_t)(k + 1) * n, c.col, nullptr, n, c.x, d,
-                                d, c.y, d, norm, add_self_loop, dinv, code, c.skip, k > 0, last, last, nullptr, 0, 0, 0, 0, 0,
-                                c.plan, plan_host, c.partial, 0, st);
+      rc = phase(k, x, d, c.y, k > 0, k == K - 1);
       if (rc) return rc;
     }
   }
   // Y leaves on the copy stream as soon as the last phase is done; the counters follow on the compute stream
   if (y_host && !colw) {
+    if (y16) {
+      rc = round_to_bf16(c.y, n, d, d, c.ystage, d, st);
+      if (rc) return rc;
+    }
     WDGH_CUDA(cudaEventRecord(c.ev_csr, st));
     WDGH_CUDA(cudaStreamWaitEvent(sc, c.ev_csr, 0));
-    WDGH_CUDA(cudaMemcpyAsync(y_host, c.y, n * d * sizeof(float), cudaMemcpyDeviceToHost, sc));
+    WDGH_CUDA(cudaMemcpyAsync(y_host, y16 ? c.ystage : static_cast<void *>(c.y), n * d * ysz, cudaMemcpyDeviceToHost,
+                              sc));
   }
   WDGH_CUDA(cudaMemcpyAsync(counters_host, c.counters, n_counters * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
   WDGH_CUDA(cudaMemcpyAsync(node_sum_host, c.node_sum, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -276,4 +328,31 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
   }
   if (y_host) WDGH_CUDA(cudaStreamSynchronize(colw ? sb : sc));
   return 0;
+}
+#undef WDGH_REQUIRE_AT
+
+}  // namespace wdgh
+
+using namespace wdgh;
+
+extern "C" int wdgh_pipeline_host_release(void) {
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  g_cache.release();
+  return 0;
+}
+
+extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                                  const float *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
+                                  int norm, int add_self_loop, float *y_host, int64_t *counters_host,
+                                  double *node_sum_host) {
+  return pipeline_host("wdgh_pipeline_host", rowptr_host, col_host, n, nnz, x_host, d, labels_host, num_classes, norm,
+                       add_self_loop, y_host, WDGH_DTYPE_F32, counters_host, node_sum_host);
+}
+
+extern "C" int wdgh_pipeline_host_bf16(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                                       const uint16_t *x_host, int64_t d, const int32_t *labels_host,
+                                       int32_t num_classes, int norm, int add_self_loop, void *y_host, int y_dtype,
+                                       int64_t *counters_host, double *node_sum_host) {
+  return pipeline_host("wdgh_pipeline_host_bf16", rowptr_host, col_host, n, nnz, x_host, d, labels_host, num_classes,
+                       norm, add_self_loop, y_host, y_dtype, counters_host, node_sum_host);
 }

@@ -24,7 +24,8 @@
 // summed in the order of the fp32 instances -- stored entries in CSR order as fmaf(w, x_j, acc) per column, then the
 // self loop, then the row scale; split rows through the same chunks and the same fixed-order finish -- so a bf16 launch
 // with fp32 output is bit-identical to the fp32 launch on x.float(), and with bf16 output (round to nearest even) to
-// that result .to(bfloat16).  The fp32 instances are unchanged.
+// that result .to(bfloat16).  The fp32 instances are unchanged.  The phased form (wdgh_spmm_csr_ranged_bf16) takes bf16
+// features with fp32 output only: its partial sums stay fp32, so a phase is bit-identical to the fp32 phase on x.float().
 #include <cuda_bf16.h>
 #include <limits.h>
 #include <stdlib.h>
@@ -315,7 +316,7 @@ spmm_heavy_finish_kernel(const int64_t *__restrict__ rowptr, const Tin *__restri
 // Split ("heavy") rows contribute no entries and are not stored; the chunk kernels own them.
 // ---------------------------------------------------------------------------
 template <int VEC, int NCH, bool HAS_VAL, bool FULL, int MINB, bool EXTRA, typename Tin = float,
-          typename Tout = float>
+          typename Tout = float, bool PHASED = true>
 __global__ void __launch_bounds__(32, MINB)
 spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col,
                      const float *__restrict__ val, int64_t n, const Tin *__restrict__ x, int d, int64_t ldx,
@@ -329,9 +330,13 @@ spmm_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restri
   // 20-21 ms (tools/phase_probe.py, profiles/phase_probe_r02.txt)
   constexpr int U = U0 > 8 ? 8 : (U0 < 2 ? 2 : U0);
   constexpr unsigned kFull = 0xffffffffu;
-  // the phased forms (y +=, raw partial sums, extra partial sums) exist for fp32 features and output only
-  constexpr bool PHASED = std::is_same<Tin, float>::value && std::is_same<Tout, float>::value;
-  static_assert(PHASED || !EXTRA, "extra partial sums are fp32");
+  // PHASED: the phased forms (y +=, raw partial sums) are compiled in; they need fp32 output, a phase never rounds its
+  // partial sum.  bf16 features get them only in the instances of wdgh_spmm_csr_ranged_bf16: compiled into the
+  // instances of wdgh_spmm_csr_bf16 as well, they made its d = 128 launch slower (64.87 against 64.52 ms on the full
+  // graph, same call, non-overlapping spreads).  The extra partial sums ride in the gather batches as rows of x, so they
+  // exist for fp32 features only.
+  static_assert(!PHASED || std::is_same<Tout, float>::value, "phases store fp32 partial sums");
+  static_assert(std::is_same<Tin, float>::value || !EXTRA, "extra partial sums are fp32");
   __shared__ float table[256];
   __shared__ int s_off[2][33];      // stream offset of every row slot of the group (exclusive scan), [32] = total
   __shared__ int64_t s_beg[2][32];  // first stored entry of every row slot
@@ -637,7 +642,7 @@ static int launch_heavy(const SpmmArgs &a, const ExtraParts &ex) {
 
 // Row-group kernel: persistent grid of one-warp CTAs, 32 per SM for a single 128-column tile (measured on the
 // 1B-entry graph, d = 128: 16 CTAs/SM 118.1 ms, 24 -> 100.4, 32 -> 95.6), 16 per SM for the wider tiles.
-template <int VEC, int NCH, bool HAS_VAL, typename Tin, typename Tout>
+template <int VEC, int NCH, bool HAS_VAL, typename Tin, typename Tout, bool PHASED>
 static int launch_rowgroup(const SpmmArgs &a) {
   constexpr int TILE = 32 * VEC * NCH;
   constexpr int MINB = (NCH == 1) ? 32 : 16;
@@ -649,7 +654,7 @@ static int launch_rowgroup(const SpmmArgs &a) {
   const bool full = (a.d == TILE);
   unsigned long long *sched = plan_sched(a.plan, kPlanSpmmTicket);
 #define WDGH_RG_LAUNCH(FULLV, MINBV, EXTRAV)                                                                        \
-  spmm_rowgroup_kernel<VEC, NCH, HAS_VAL, FULLV, MINBV, EXTRAV, Tin, Tout><<<grid, 32, 0, a.st>>>(                    \
+  spmm_rowgroup_kernel<VEC, NCH, HAS_VAL, FULLV, MINBV, EXTRAV, Tin, Tout, PHASED><<<grid, 32, 0, a.st>>>(            \
       a.rowptr, a.col, a.val, a.n, static_cast<const Tin *>(a.x), a.d, a.ldx, static_cast<Tout *>(a.y), a.ldy, a.norm, \
       a.self_loop, a.dinv, a.deg_code, a.threshold, a.row_offset, a.ra, sched)
   constexpr bool F32 = std::is_same<Tin, float>::value && std::is_same<Tout, float>::value;
@@ -669,17 +674,18 @@ static int launch_rowgroup(const SpmmArgs &a) {
 
 static bool rowgroup_width(int64_t d) { return d >= 128 || d == 64 || d == 32; }
 
-template <bool HAS_VAL, typename Tin = float, typename Tout = float>
+// PHASED: the row-group instances carry the phased forms (the ranged entries, and every fp32 launch)
+template <bool HAS_VAL, typename Tin, typename Tout, bool PHASED>
 static int dispatch(const SpmmArgs &a, bool vec4) {
   int rc;
   const int d = a.d;
   const ExtraParts none = {0, 0, 0, nullptr};
   if (vec4 && rowgroup_width(d)) {
-    if (d == 32) rc = launch_rowgroup<1, 1, HAS_VAL, Tin, Tout>(a);
-    else if (d == 64) rc = launch_rowgroup<2, 1, HAS_VAL, Tin, Tout>(a);
-    else if (d <= 128) rc = launch_rowgroup<4, 1, HAS_VAL, Tin, Tout>(a);
-    else if (d <= 256) rc = launch_rowgroup<4, 2, HAS_VAL, Tin, Tout>(a);
-    else rc = launch_rowgroup<4, 4, HAS_VAL, Tin, Tout>(a);
+    if (d == 32) rc = launch_rowgroup<1, 1, HAS_VAL, Tin, Tout, PHASED>(a);
+    else if (d == 64) rc = launch_rowgroup<2, 1, HAS_VAL, Tin, Tout, PHASED>(a);
+    else if (d <= 128) rc = launch_rowgroup<4, 1, HAS_VAL, Tin, Tout, PHASED>(a);
+    else if (d <= 256) rc = launch_rowgroup<4, 2, HAS_VAL, Tin, Tout, PHASED>(a);
+    else rc = launch_rowgroup<4, 4, HAS_VAL, Tin, Tout, PHASED>(a);
     if (rc || !a.heavy_pass) return rc;
     if (d <= 128) return launch_heavy<4, 1, HAS_VAL, Tin, Tout>(a, none);
     if (d <= 256) return launch_heavy<4, 2, HAS_VAL, Tin, Tout>(a, none);
@@ -755,13 +761,13 @@ static int spmm_csr(const char *fn, const int64_t *rowptr, const int32_t *col, c
   if constexpr (!std::is_same<Tin, float>::value) {  // (fp32 features have fp32 output only)
     if (y_dtype == WDGH_DTYPE_BF16) {
       const bool vec4 = rows_vec4(x, d, ldx, static_cast<const bf16 *>(y), ldy, partial);
-      return val ? dispatch<true, Tin, bf16>(a, vec4) : dispatch<false, Tin, bf16>(a, vec4);
+      return val ? dispatch<true, Tin, bf16, false>(a, vec4) : dispatch<false, Tin, bf16, false>(a, vec4);
     }
   }
   const bool vec4 = rows_vec4(x, d, ldx, static_cast<const float *>(y), ldy, partial);
-  return val ? dispatch<true, Tin, float>(a, vec4) : dispatch<false, Tin, float>(a, vec4);
+  constexpr bool F32 = std::is_same<Tin, float>::value;
+  return val ? dispatch<true, Tin, float, F32>(a, vec4) : dispatch<false, Tin, float, F32>(a, vec4);
 }
-#undef WDGH_REQUIRE_AT
 }  // namespace wdgh
 
 extern "C" int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
@@ -857,26 +863,59 @@ extern "C" int wdgh_plan_heavy_flags(const int64_t *plan_i64, const int64_t *pla
   return 0;
 }
 
-extern "C" int wdgh_spmm_csr_ranged(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
-                                    const int32_t *col, const float *val, int64_t n, const float *x, int64_t d,
-                                    int64_t ldx, float *y, int64_t ldy, int norm, int add_self_loop,
-                                    const float *dinv, const uint8_t *deg_code, const uint8_t *skip_rows,
-                                    int accumulate, int finalize, int run_split_rows,
-                                    const float *extra_parts, int32_t n_extra, int32_t n_extra_split,
-                                    int64_t extra_part_rows, int64_t ld_extra, int32_t ctas_per_sm, int64_t *plan_i64,
-                                    const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
-  WDGH_REQUIRE(rowptr && range_begin && range_end && x && y && plan_i64 && plan_host, "wdgh_spmm_csr_ranged: null pointer");
-  WDGH_REQUIRE(n >= 0 && d > 0 && ldx >= d && ldy >= d, "wdgh_spmm_csr_ranged: bad shape");
-  WDGH_REQUIRE(norm == WDGH_NORM_NONE || dinv != nullptr, "wdgh_spmm_csr_ranged: norm requires dinv");
-  WDGH_REQUIRE(rows_vec4(x, d, ldx, y, ldy, partial) && rowgroup_width(d),
-               "wdgh_spmm_csr_ranged: needs 16-byte aligned rows and d in {32, 64} or d >= 128");
-  WDGH_REQUIRE(plan_host[1] == 0 || skip_rows != nullptr, "wdgh_spmm_csr_ranged: split rows need skip_rows (wdgh_plan_heavy_flags)");
-  WDGH_REQUIRE(n_extra >= 0 && n_extra <= kMaxExtra && n_extra_split >= 0 && n_extra_split <= n_extra &&
-                   (n_extra == 0 || (extra_parts != nullptr && ld_extra >= d && ld_extra % 4 == 0 && d >= 128 &&
-                                     extra_part_rows >= n && reinterpret_cast<uintptr_t>(extra_parts) % 16 == 0 &&
-                                     (int64_t)n_extra * extra_part_rows < ((int64_t)1 << 31))),
-               "wdgh_spmm_csr_ranged: bad extra partial sums");
-  WDGH_REQUIRE(ctas_per_sm >= 0, "wdgh_spmm_csr_ranged: bad ctas_per_sm");
+namespace wdgh {
+// fp32 -> bf16 of a strided block, round to nearest even (the rounding of __float22bfloat162_rn): one warp per row
+__global__ void round_bf16_kernel(const float *__restrict__ x, int64_t rows, int64_t cols, int64_t ldx,
+                                  bf16 *__restrict__ y, int64_t ldy, int pairs) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < rows; r += warps) {
+    const float *xr = x + r * ldx;
+    bf16 *yr = y + r * ldy;
+    if (pairs) {
+      for (int64_t c = 2 * lane; c < cols; c += 64) {
+        const float2 v = *reinterpret_cast<const float2 *>(xr + c);
+        *reinterpret_cast<unsigned *>(yr + c) = bf16x2_rn(v.x, v.y);
+      }
+    } else {
+      for (int64_t c = lane; c < cols; c += 32) yr[c] = __float2bfloat16_rn(xr[c]);
+    }
+  }
+}
+
+int round_to_bf16(const float *x, int64_t rows, int64_t cols, int64_t ldx, void *y, int64_t ldy, cudaStream_t st) {
+  if (rows == 0) return 0;
+  const int pairs = (cols % 2 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (reinterpret_cast<uintptr_t>(x) % 8 == 0) &&
+                    (reinterpret_cast<uintptr_t>(y) % 4 == 0);
+  round_bf16_kernel<<<persistent_grid(ceil_div(rows, 8), 8), 256, 0, st>>>(x, rows, cols, ldx, static_cast<bf16 *>(y),
+                                                                          ldy, pairs);
+  WDGH_LAUNCHED("round_bf16_kernel");
+  return 0;
+}
+
+// argument checks and dispatch shared by wdgh_spmm_csr_ranged (Tin = float) and wdgh_spmm_csr_ranged_bf16 (no extra
+// partial sums, n_extra = 0)
+template <typename Tin>
+static int spmm_ranged(const char *fn, const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                       const int32_t *col, const float *val, int64_t n, const Tin *x, int64_t d, int64_t ldx, float *y,
+                       int64_t ldy, int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                       const uint8_t *skip_rows, int accumulate, int finalize, int run_split_rows,
+                       const float *extra_parts, int32_t n_extra, int32_t n_extra_split, int64_t extra_part_rows,
+                       int64_t ld_extra, int32_t ctas_per_sm, int64_t *plan_i64, const int64_t *plan_host,
+                       float *partial, int64_t row_offset, void *stream) {
+  WDGH_REQUIRE_AT(rowptr && range_begin && range_end && x && y && plan_i64 && plan_host, "null pointer");
+  WDGH_REQUIRE_AT(n >= 0 && d > 0 && ldx >= d && ldy >= d, "bad shape");
+  WDGH_REQUIRE_AT(norm == WDGH_NORM_NONE || dinv != nullptr, "norm requires dinv");
+  WDGH_REQUIRE_AT(rows_vec4(x, d, ldx, y, ldy, partial) && rowgroup_width(d),
+                  sizeof(Tin) == 4 ? "needs 16-byte aligned rows and d in {32, 64} or d >= 128"
+                                   : "needs 8-byte aligned rows (d, ldx multiples of 4) and d in {32, 64} or d >= 128");
+  WDGH_REQUIRE_AT(plan_host[1] == 0 || skip_rows != nullptr, "split rows need skip_rows (wdgh_plan_heavy_flags)");
+  WDGH_REQUIRE_AT(n_extra >= 0 && n_extra <= kMaxExtra && n_extra_split >= 0 && n_extra_split <= n_extra &&
+                      (n_extra == 0 || (extra_parts != nullptr && ld_extra >= d && ld_extra % 4 == 0 && d >= 128 &&
+                                        extra_part_rows >= n && reinterpret_cast<uintptr_t>(extra_parts) % 16 == 0 &&
+                                        (int64_t)n_extra * extra_part_rows < ((int64_t)1 << 31))),
+                  "bad extra partial sums");
+  WDGH_REQUIRE_AT(ctas_per_sm >= 0, "bad ctas_per_sm");
   if (n == 0) return 0;
   SpmmArgs a;
   a.rowptr = range_begin; a.col = col; a.val = val; a.n = n; a.x = x; a.d = (int)d; a.ldx = ldx; a.y = y; a.ldy = ldy;
@@ -890,21 +929,49 @@ extern "C" int wdgh_spmm_csr_ranged(const int64_t *rowptr, const int64_t *range_
   a.ra.ex = ExtraParts{n_extra, ld_extra, extra_part_rows, extra_parts};
   a.cta_limit = ctas_per_sm;
   a.heavy_pass = false;
-  int rc = val ? dispatch<true>(a, true) : dispatch<false>(a, true);
+  int rc = val ? dispatch<true, Tin, float, true>(a, true) : dispatch<false, Tin, float, true>(a, true);
   if (rc || !run_split_rows || a.n_chunks == 0) return rc;
   // split rows: always over their full column range, after the last phase (they overwrite their Y rows); of the
   // extra partial sums only the LAST n_extra_split apply (an earlier phase of this rank never stored split rows)
-  WDGH_REQUIRE(partial != nullptr, "wdgh_spmm_csr_ranged: split rows need the partial buffer");
+  WDGH_REQUIRE_AT(partial != nullptr, "split rows need the partial buffer");
   ExtraParts ex = {n_extra_split, ld_extra, extra_part_rows,
                    n_extra ? extra_parts + (int64_t)(n_extra - n_extra_split) * extra_part_rows * ld_extra : nullptr};
   a.rowptr = rowptr; a.threshold = plan_host[2];
   a.ra = RangeArgs{nullptr, nullptr, 0, finalize ? 1 : 0, {0, 0, 0, nullptr}};
   if (val) {
-    if (d <= 128) return launch_heavy<4, 1, true>(a, ex);
-    if (d <= 256) return launch_heavy<4, 2, true>(a, ex);
-    return launch_heavy<4, 4, true>(a, ex);
+    if (d <= 128) return launch_heavy<4, 1, true, Tin>(a, ex);
+    if (d <= 256) return launch_heavy<4, 2, true, Tin>(a, ex);
+    return launch_heavy<4, 4, true, Tin>(a, ex);
   }
-  if (d <= 128) return launch_heavy<4, 1, false>(a, ex);
-  if (d <= 256) return launch_heavy<4, 2, false>(a, ex);
-  return launch_heavy<4, 4, false>(a, ex);
+  if (d <= 128) return launch_heavy<4, 1, false, Tin>(a, ex);
+  if (d <= 256) return launch_heavy<4, 2, false, Tin>(a, ex);
+  return launch_heavy<4, 4, false, Tin>(a, ex);
+}
+#undef WDGH_REQUIRE_AT
+}  // namespace wdgh
+
+extern "C" int wdgh_spmm_csr_ranged(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                                    const int32_t *col, const float *val, int64_t n, const float *x, int64_t d,
+                                    int64_t ldx, float *y, int64_t ldy, int norm, int add_self_loop,
+                                    const float *dinv, const uint8_t *deg_code, const uint8_t *skip_rows,
+                                    int accumulate, int finalize, int run_split_rows,
+                                    const float *extra_parts, int32_t n_extra, int32_t n_extra_split,
+                                    int64_t extra_part_rows, int64_t ld_extra, int32_t ctas_per_sm, int64_t *plan_i64,
+                                    const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  return spmm_ranged("wdgh_spmm_csr_ranged", rowptr, range_begin, range_end, col, val, n, x, d, ldx, y, ldy, norm,
+                     add_self_loop, dinv, deg_code, skip_rows, accumulate, finalize, run_split_rows, extra_parts,
+                     n_extra, n_extra_split, extra_part_rows, ld_extra, ctas_per_sm, plan_i64, plan_host, partial,
+                     row_offset, stream);
+}
+
+extern "C" int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                                         const int32_t *col, const float *val, int64_t n, const uint16_t *x, int64_t d,
+                                         int64_t ldx, float *y, int64_t ldy, int norm, int add_self_loop,
+                                         const float *dinv, const uint8_t *deg_code, const uint8_t *skip_rows,
+                                         int accumulate, int finalize, int run_split_rows, int64_t *plan_i64,
+                                         const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  return spmm_ranged("wdgh_spmm_csr_ranged_bf16", rowptr, range_begin, range_end, col, val, n,
+                     reinterpret_cast<const bf16 *>(x), d, ldx, y, ldy, norm, add_self_loop, dinv, deg_code, skip_rows,
+                     accumulate, finalize, run_split_rows, nullptr, 0, 0, 0, 0, 0, plan_i64, plan_host, partial,
+                     row_offset, stream);
 }

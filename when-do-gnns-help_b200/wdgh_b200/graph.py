@@ -279,11 +279,25 @@ def spmm_ranged(g: CSRGraph, range_begin, range_end, x, y, norm, add_self_loop, 
     feature shard in place (the kernel is handed the address x[0] would have at global id 0).
     extra: [parts, rows >= n, d] tensor of raw partial sums of the same rows (possibly peer-mapped), added to every row
     as it is aggregated; the split-row pass adds only the last `extra_split` parts.  y may be peer memory.
-    ctas_per_sm: 0 = default grid, smaller = leave room for a kernel running concurrently on another stream."""
+    ctas_per_sm: 0 = default grid, smaller = leave room for a kernel running concurrently on another stream.
+    A bfloat16 `x` (float32 `y`, no `extra`, no `ctas_per_sm`) is read as it is; every phase sums in fp32 and is
+    bit-identical to the same call on `x.float()`."""
     d = int(x.shape[1])
-    x_ptr = x.data_ptr() - int(x_row0) * x.stride(0) * 4
+    x_ptr = x.data_ptr() - int(x_row0) * x.stride(0) * x.element_size()
     plan, plan_host = g.plan
     partial = _partial_scratch(g, d)
+    if x.dtype == torch.bfloat16:
+        if extra is not None or ctas_per_sm:
+            raise ValueError("extra partial sums and ctas_per_sm need float32 features")
+        if y.dtype != torch.float32:
+            raise ValueError(f"a phase writes float32 partial sums, got a {y.dtype} y")
+        check(lib.wdgh_spmm_csr_ranged_bf16(ptr(g.rowptr), ptr(range_begin), ptr(range_end), ptr(g.col), ptr(g.val),
+                                            g.n, x_ptr, d, x.stride(0), ptr(y), y.stride(0), norm,
+                                            int(bool(add_self_loop)), ptr(dinv), ptr(deg_code), ptr(skip_rows),
+                                            int(bool(accumulate)), int(bool(finalize)), int(bool(run_split_rows)),
+                                            ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()),
+              "wdgh_spmm_csr_ranged_bf16")
+        return y
     n_extra = part_rows = ld_extra = 0
     if extra is not None:
         if extra.dim() != 3 or extra.shape[1] < g.n or extra.shape[2] != d or extra.stride(2) != 1:
@@ -387,12 +401,19 @@ def structure_counts(g: CSRGraph, labels32, num_classes) -> StructureCounts:
 
 
 def spmm_structure_fused(g: CSRGraph, x, labels32, num_classes, norm=NORM_SYM, add_self_loop=True, out=None,
-                         dinv=None, deg_code=None, scratch=None):
+                         dinv=None, deg_code=None, scratch=None, out_dtype=None):
     """One call: y = norm(A [+I]) x and the label statistics (device tensors, no sync).
 
-    Returns (y, (counters, node_sum, deg, match, labels_u8)); binary adjacency only."""
+    Returns (y, (counters, node_sum, deg, match, labels_u8)); binary adjacency only.  A bfloat16 `x` is read as it is
+    (the bf16 aggregation, then the label pass on the same stream); `out_dtype` / `out` as in `spmm`."""
     if g.val is not None:
         raise ValueError("the fused pass needs a binary adjacency (values = None)")
+    if isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16:
+        y = spmm(g, x, norm, add_self_loop, out=out, dinv=dinv, deg_code=deg_code, out_dtype=out_dtype)
+        return y, structure_counts_raw(g, labels32, num_classes, scratch)
+    if out_dtype not in (None, torch.float32):
+        raise ValueError(f"cannot write a {out_dtype} result from float32 features (bfloat16 output needs bfloat16 "
+                         "features)")
     x = _cuda(x, torch.float32)
     d = int(x.shape[1])
     c = int(num_classes)
@@ -416,6 +437,52 @@ def spmm_structure_fused(g: CSRGraph, x, labels32, num_classes, norm=NORM_SYM, a
                                         ptr(node_sum), ptr(deg), ptr(match), ptr(lab8), n_labels, g.row_offset,
                                         stream_ptr()), "wdgh_spmm_structure_fused")
     return y, scratch
+
+
+def pipeline_host(rowptr, col, x, labels, num_classes, norm=NORM_SYM, add_self_loop=True, y=None):
+    """The whole pass from HOST memory (wdgh_pipeline_host / wdgh_pipeline_host_bf16): copies in, plan, degree scale,
+    y = norm(A [+I]) x, label statistics, copies back.  Synchronous; device buffers are cached between calls.
+
+    rowptr int64 [n+1], col int32 [nnz], labels int32 [n] and x [n, d] float32 or bfloat16 (bfloat16 halves the
+    feature bytes on the link) are contiguous CPU tensors -- pinned memory lets the copies run at the full link rate.
+    y: None (counters only) or a contiguous [n, d] CPU tensor, filled in place: float32, or bfloat16 with bfloat16
+    features (the float32 result rounded to nearest even).  Returns (counters int64[sc_words(C)], node_sum float64[2])
+    as numpy arrays."""
+    named = [("rowptr", rowptr, (torch.int64,)), ("col", col, (torch.int32,)), ("labels", labels, (torch.int32,)),
+             ("x", x, (torch.float32, torch.bfloat16))]
+    if y is not None:
+        named.append(("y", y, (torch.float32, torch.bfloat16)))
+    for name, t, dtypes in named:
+        if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
+            raise ValueError(f"{name} must be a CPU tensor")
+        if not t.is_contiguous():
+            raise ValueError(f"{name} must be contiguous")
+        if t.dtype not in dtypes:
+            raise ValueError(f"{name} must be {' or '.join(str(d) for d in dtypes)}, got {t.dtype}")
+    if x.dim() != 2:
+        raise ValueError(f"x must be [n, d], got {tuple(x.shape)}")
+    n, d = int(x.shape[0]), int(x.shape[1])
+    if rowptr.shape != (n + 1,) or col.dim() != 1 or labels.shape != (n,):
+        raise ValueError(f"rowptr must be [{n + 1}], col 1-D and labels [{n}]; got {tuple(rowptr.shape)}, "
+                         f"{tuple(col.shape)}, {tuple(labels.shape)}")
+    bf16 = x.dtype == torch.bfloat16
+    if y is not None:
+        if y.shape != (n, d):
+            raise ValueError(f"y must be [{n}, {d}], got {tuple(y.shape)}")
+        if y.dtype == torch.bfloat16 and not bf16:
+            raise ValueError("a bfloat16 y needs bfloat16 features")
+    c = int(num_classes)
+    counters = np.zeros(_lib.sc_words(c), np.int64)
+    node_sum = np.zeros(2, np.float64)
+    _lib.require_device()
+    args = (ptr(rowptr), ptr(col), n, int(col.shape[0]), ptr(x), d, ptr(labels), c, norm, int(bool(add_self_loop)))
+    if bf16:
+        y_dtype = _lib.DTYPE_BF16 if y is not None and y.dtype == torch.bfloat16 else _lib.DTYPE_F32
+        check(lib.wdgh_pipeline_host_bf16(*args, ptr(y), y_dtype, counters.ctypes.data, node_sum.ctypes.data),
+              "wdgh_pipeline_host_bf16")
+    else:
+        check(lib.wdgh_pipeline_host(*args, ptr(y), counters.ctypes.data, node_sum.ctypes.data), "wdgh_pipeline_host")
+    return counters, node_sum
 
 
 def structure_counts_coo(edge_index, n, labels32, num_classes, hist_includes_self_loops=False) -> StructureCounts:
