@@ -191,7 +191,7 @@ def test_bf16_pipeline_forms(W, host_graph, d, form):
     scale = y_res.abs().max().item()
     assert (y1 - y_res).abs().max().item() <= 1e-5 * scale
     assert (y32 - y_res).abs().max().item() <= 1e-5 * scale
-    assert torch.equal(y1, y32)          # both feature types take the same form (csrc/pipeline_host.cu, e2e_col_width)
+    assert torch.equal(y1, y32)          # both feature types take the same schedule (csrc/pipeline_host.cu)
     if d in (96, 70):
         assert torch.equal(y1, y_res)
     assert torch.equal(y2, y1.to(BF16))

@@ -16,8 +16,7 @@ Per arm: median ms and spread, GEdges/s, H2D / D2H bytes and the effective link 
 Checks in the same run: the counters of every arm are identical; on a seeded sample of rows, the fp32 Y of the bf16
 features equals the fp32 Y of e2e_f32 exactly (both feature types take the same copy / compute form, whose phases are
 bit-identical), and the bf16 Y equals the fp32 Y of the bf16 features rounded to nearest even.  Prints one JSON line,
-writes it to --out and exits non-zero when a check fails.  WDGH_E2E_COLW (0 = row blocks, 64 = column blocks) selects
-the form of the Y-returning arms for both feature types.
+writes it to --out and exits non-zero when a check fails.
 """
 import argparse
 import json
@@ -40,10 +39,8 @@ HEADLINE_NODES = 50_000_000
 
 
 def column_blocks(d):
-    """True when the Y-returning form of the pipeline uses column blocks (csrc/pipeline_host.cu, e2e_col_width)"""
-    env = os.environ.get("WDGH_E2E_COLW")
-    w = int(env) if env in ("0", "32", "64") else 64
-    return w > 0 and d % w == 0 and 2 <= d // w <= 64
+    """True when the Y-returning arms copy X in 64-column blocks (csrc/pipeline_host.cu, schedule)"""
+    return d % 64 == 0 and 2 <= d // 64 <= 64
 
 
 def main():
@@ -145,7 +142,7 @@ def main():
     line = {"tool": "tools/e2e_bf16_bench.py", "nodes": n, "headline_graph": n == HEADLINE_NODES,
             "stored_entries": nnz, "dim": d, "classes": C, "norm": "sym D^-1/2 (A+I) D^-1/2 on the fly",
             "reps": args.reps, "warmup": args.warmup, "timer": "host clock around the synchronous call",
-            "host_memory": "pinned", "e2e_colw_env": os.environ.get("WDGH_E2E_COLW"), "arms": res,
+            "host_memory": "pinned", "arms": res,
             "speedup_e2e_bf16_f32y": res["e2e_f32"]["ms"] / res["e2e_bf16_f32y"]["ms"],
             "speedup_e2e_bf16_bf16y": res["e2e_f32"]["ms"] / res["e2e_bf16_bf16y"]["ms"],
             "speedup_counters_bf16": res["counters_f32"]["ms"] / res["counters_bf16"]["ms"],

@@ -3,30 +3,33 @@
 // normaliser, A_hat X, label statistics and the D2H result copies are all inside the caller's
 // timed region (bench.py "e2e").
 //
-// The pass is PCIe-bound (the feature matrix is 85% of the bytes), so the entry is a two-stream
-// pipeline: the CSR and the labels go first; the feature matrix follows in 16 row blocks on
-// a copy stream while the compute stream builds the plan, runs the label pass and then aggregates,
-// per arriving block, the entries whose source node lies in that block (wdgh_spmm_csr_ranged:
-// column ranges of every row, y +=, self loop + scale with the last block).  Only the last
-// block's phase is exposed after the copies end.
+// The pass is PCIe-bound (the feature matrix is 85% of the bytes), so the entry is a pipeline on three streams.  The CSR
+// and the labels go first on a copy stream, and the feature matrix follows on the same stream as KC = d / W column
+// blocks of width W, each in R row chunks.  Meanwhile the compute stream builds the plan and runs the label pass, then
+// aggregates every chunk as it arrives: with R > 1 one phase per chunk (wdgh_spmm_csr_ranged: the entries whose source
+// node lies in the chunk, y +=, self loop + scale with the last chunk), with R = 1 one full launch.  When Y comes back,
+// each Y block leaves on the third stream as soon as its last phase is done.  So only the last chunk's phase is exposed
+// after the H2D copies end.  schedule() picks (W, KC, R):
 //
-// When Y = A_hat X has to come back to the host as well (y_host != NULL) the D2H copy of Y would follow the whole
-// H2D stream -- Y depends on every feature ROW block -- and the step would cost H2D + D2H back to back (1070 ms for
-// 30.1 + 25.6 GB).  PCIe is full duplex, and a COLUMN block of Y needs only the same column block of X, so this form
-// splits the feature matrix by columns instead: pitched copies (cudaMemcpy2DAsync, 256-byte rows out of the 512-byte
-// pitch keep the full link rate: 55.6 / 53.5 GB/s alone, 48 + 50 GB/s both directions at once, tools/pcie_probe.cu),
-// aggregation of a column block on strided views (ldx = ldy = d; bit-identical to the one-launch result,
-// tools/colblock_probe.py) phased by arriving row chunk exactly like the counters-only form, so that only the last
-// chunk's phase separates the end of a block's H2D copy from the start of its D2H copy, and the D2H copy of block k
-// runs under the H2D copy of block k + 1.
+//   case                                                  W    KC       R
+//   Y wanted, d % 64 == 0 and 2 <= d / 64 <= 64           64   d / 64   4, halved while KC * R > 64
+//   otherwise, d % 4 == 0 and d in {32, 64} or d >= 128   d    1        16   (row blocks)
+//   otherwise (widths the ranged entries do not take)     d    1        1    (one copy, one launch)
+//
+// Why column blocks when Y comes back: with row blocks the D2H copy of Y would follow the whole H2D stream -- Y depends
+// on every feature ROW block -- and the step would cost H2D + D2H back to back (1070 ms for 30.1 + 25.6 GB).  PCIe is
+// full duplex, and a COLUMN block of Y needs only the same column block of X, so the feature matrix is split by columns
+// instead: pitched copies (cudaMemcpy2DAsync), aggregation of a column block on strided views (ldx = ldy = d;
+// bit-identical to the one-launch result, tools/colblock_probe.py) phased by arriving row chunk, so that only the last
+// chunk's phase separates the end of a block's H2D copy from the start of its D2H copy, and the D2H copy of block k runs
+// under the H2D copy of block k + 1.
 //
 // bfloat16 features (wdgh_pipeline_host_bf16) take the same body with the bf16 aggregation entries: half the bytes of
 // X on the link, fp32 phases (a phase is bit-identical to the fp32 phase on the upcast matrix).  Y is always
 // aggregated in fp32 into the device Y buffer; for a bf16 Y the last phase of a block is followed by a rounding pass
 // into a bf16 staging buffer, which the D2H copy reads -- so a bf16 Y is exactly the rounding of the fp32 Y of the
 // same schedule, and the schedule does not depend on the type of Y.
-#include <stdlib.h>
-
+#include <algorithm>
 #include <mutex>
 #include <type_traits>
 
@@ -34,12 +37,53 @@
 
 namespace wdgh {
 
+// Block chunks (KC * R) of one call: each has its own H2D event, and each column block its own Y event.
+constexpr int kMaxChunks = 64;
+
+// Row chunks when the feature matrix travels whole-width (1 = copy everything, then compute).  Measured (30.1 GB per
+// pass): 1 -> 635 ms, 4 -> 587, 8 -> 579, 16 -> 574 ms; the copies alone take ~548 ms.
+constexpr int kRowChunks = 16;
+
+// Width (elements) of the column blocks when Y comes back.  64 floats = 256-byte rows: the narrowest pitched copy that
+// still runs at the full PCIe rate in both directions (55.6 / 53.5 GB/s alone, 48 + 50 GB/s both directions at once;
+// 128-byte rows: 34 + 40 GB/s, tools/pcie_probe.cu), and a width the row-group aggregation kernel runs natively.
+// bf16 features take the same 64 columns, i.e. 128-byte rows (the slower pitched copy): measured on the 50M-node /
+// 976M-entry graph at d = 128 (tools/e2e_bf16_bench.py, NVIDIA B200, 1000 W power limit, each form in its own process),
+// column blocks 735.7 ms with fp32 Y back and 536.8 ms with bf16 Y back, against 795.1 / 578.3 ms for row blocks (full-rate
+// contiguous H2D, Y copied after the last phase).
+constexpr int64_t kColWidth = 64;
+
+// Row chunks per column block: the block's aggregation is phased by arriving row chunk, so that only the last chunk's
+// phase -- not a whole-graph launch -- stands between the end of a block's H2D copy and the start of its D2H copy.  A
+// phase over 50M rows costs 20-23 ms at 64 columns whatever the range length (tools/phase_probe.py; 52.8 ms for the
+// whole block in one launch), so the phases of a block must fit under its 230 ms H2D copy.  Measured per step: 858.9 ms
+// (1 chunk), 831.7 ms (4), 828.9 ms (8); 4 keeps the larger margin.
+constexpr int kColRows = 4;
+
+// The feature matrix travels as KC = d / W column blocks of width W, each in R row chunks.
+struct Schedule {
+  int64_t W;
+  int KC, R;
+};
+
+static Schedule schedule(int64_t d, bool y_wanted) {
+  if (y_wanted && d % kColWidth == 0 && d / kColWidth >= 2 && d / kColWidth <= kMaxChunks) {
+    const int KC = (int)(d / kColWidth);
+    int R = kColRows;
+    while (R > 1 && KC * R > kMaxChunks) R /= 2;
+    return {kColWidth, KC, R};
+  }
+  // the widths the ranged aggregation entries take (16-byte fp32 / 8-byte bf16 rows, row-group kernel widths)
+  if (d % 4 == 0 && (d == 32 || d == 64 || d >= 128)) return {d, 1, kRowChunks};
+  return {d, 1, 1};
+}
+
 struct HostPipelineCache {
-  int64_t n = -1, nnz = -1, d = -1, cap = -1, partial_elems = 0;
+  int64_t n = -1, nnz = -1, d = -1, cap = -1;
   int C = -1, device = -1;
   // The feature buffer is sized in bytes and grows when a call needs more (an fp32 call after a bf16 one); a bf16 call
   // after an fp32 one reuses it, so a caller alternating feature types does not reallocate the largest buffer.
-  size_t x_bytes = 0, ystage_bytes = 0;
+  size_t x_bytes = 0, ystage_bytes = 0, partial_bytes = 0;
   int64_t *rowptr = nullptr;
   int32_t *col = nullptr;
   void *x = nullptr;
@@ -49,10 +93,10 @@ struct HostPipelineCache {
   uint8_t *labels8 = nullptr, *deg_code = nullptr;
   int64_t *plan = nullptr, *counters = nullptr;
   double *node_sum = nullptr;
-  int64_t *seg = nullptr, *bounds = nullptr;  // column segments of the feature row blocks
+  int64_t *seg = nullptr, *bounds = nullptr;  // column segments of the feature row chunks
   uint8_t *skip = nullptr;
   cudaStream_t st = nullptr, st_copy = nullptr, st_back = nullptr;
-  cudaEvent_t ev_csr = nullptr, ev_x[64] = {nullptr}, ev_y[64] = {nullptr};
+  cudaEvent_t ev_csr = nullptr, ev_x[kMaxChunks] = {nullptr}, ev_y[kMaxChunks] = {nullptr};
   void release() {
     cudaFree(seg); cudaFree(bounds); cudaFree(skip);
     if (st_copy) cudaStreamDestroy(st_copy);
@@ -70,48 +114,17 @@ static HostPipelineCache g_cache;  // one cached pipeline per process, guarded b
 static std::mutex g_cache_mu;
 constexpr int64_t kHostPipelineThreshold = 512;
 
-// feature row blocks of the pipelined copy (1 = copy everything, then compute); WDGH_E2E_CHUNKS overrides
-static int e2e_chunks() {
-  static int cached = 0;
-  if (cached == 0) {
-    int v = 16;  // measured (30.1 GB per pass): 1 -> 635 ms, 4 -> 587, 8 -> 579, 16 -> 574 ms; the copies alone take ~548 ms
-    if (const char *e = getenv("WDGH_E2E_CHUNKS")) v = atoi(e);
-    cached = (v >= 1 && v <= 64) ? v : 16;
-  }
-  return cached;
-}
-
-// Width (elements) of the column blocks of the Y-returning form, 0 = row-block form.  64 floats = 256-byte rows: the
-// narrowest pitched copy that still runs at the full PCIe rate in both directions (128-byte rows: 34 + 40 GB/s), and a
-// width the row-group aggregation kernel runs natively.  WDGH_E2E_COLW overrides (0, 32 or 64).
-// bf16 features take the same 64 columns, i.e. 128-byte rows (the slower pitched copy): measured on the 50M-node /
-// 976M-entry graph at d = 128 (tools/e2e_bf16_bench.py, NVIDIA B200, 1000 W power limit, each form in its own process),
-// column blocks 735.7 ms with fp32 Y back and 536.8 ms with bf16 Y back, against 795.1 / 578.3 ms for row blocks (full-rate
-// contiguous H2D, Y copied after the last phase).
-static int64_t e2e_col_width(int64_t d) {
-  static int cached = -1;
-  if (cached < 0) {
-    int v = 64;
-    if (const char *e = getenv("WDGH_E2E_COLW")) v = atoi(e);
-    cached = (v == 0 || v == 32 || v == 64) ? v : 64;
-  }
-  return (cached > 0 && d % cached == 0 && d / cached >= 2 && d / cached <= 64) ? cached : 0;
-}
-
-// Row chunks per column block of the Y-returning form: the block's aggregation is phased by arriving row chunk (as in
-// the counters-only form), so that only the last chunk's phase -- not a whole-graph launch -- stands between the end of
-// a block's H2D copy and the start of its D2H copy.  A phase over 50M rows costs 20-23 ms at 64 columns whatever the
-// range length (tools/phase_probe.py; 52.8 ms for the whole block in one launch), so the phases of a block must fit under
-// its 230 ms H2D copy.  Measured per step: 858.9 ms (1 chunk), 831.7 ms (4), 828.9 ms (8); 4 keeps the larger margin.
-// WDGH_E2E_COLROWS overrides (1 = one launch per column block).
-static int e2e_col_rows() {
-  static int cached = 0;
-  if (cached == 0) {
-    int v = 4;
-    if (const char *e = getenv("WDGH_E2E_COLROWS")) v = atoi(e);
-    cached = (v >= 1 && v <= 32) ? v : 4;
-  }
-  return cached;
+// The buffers of the cache that only grow (features, bf16 Y staging, split-row partial sums): reallocates p when it
+// holds fewer than `bytes`.
+template <typename T>
+static cudaError_t grow(T *&p, size_t &cap, size_t bytes) {
+  if (cap >= bytes) return cudaSuccess;
+  cudaFree(p);
+  p = nullptr;
+  cap = 0;
+  const cudaError_t e = cudaMalloc(&p, bytes);
+  if (e == cudaSuccess) cap = bytes;
+  return e;
 }
 
 #define WDGH_REQUIRE_AT(cond, what)                                      \
@@ -156,76 +169,56 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
     WDGH_CUDA(cudaStreamCreateWithFlags(&c.st_copy, cudaStreamNonBlocking));
     WDGH_CUDA(cudaStreamCreateWithFlags(&c.st_back, cudaStreamNonBlocking));
     WDGH_CUDA(cudaEventCreateWithFlags(&c.ev_csr, cudaEventDisableTiming));
-    for (int k = 0; k < 64; ++k) WDGH_CUDA(cudaEventCreateWithFlags(&c.ev_x[k], cudaEventDisableTiming));
-    for (int k = 0; k < 64; ++k) WDGH_CUDA(cudaEventCreateWithFlags(&c.ev_y[k], cudaEventDisableTiming));
-    WDGH_CUDA(cudaMalloc(&c.seg, (size_t)(e2e_chunks() + 1) * (size_t)n * sizeof(int64_t)));
-    WDGH_CUDA(cudaMalloc(&c.bounds, 65 * sizeof(int64_t)));
+    for (auto &e : c.ev_x) WDGH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    for (auto &e : c.ev_y) WDGH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    WDGH_CUDA(cudaMalloc(&c.seg, (size_t)(kRowChunks + 1) * (size_t)n * sizeof(int64_t)));
+    WDGH_CUDA(cudaMalloc(&c.bounds, (kRowChunks + 1) * sizeof(int64_t)));
     WDGH_CUDA(cudaMalloc(&c.skip, (size_t)n));
     c.n = n; c.nnz = nnz; c.d = d; c.C = C; c.cap = cap; c.device = device;
   }
-  if (c.x_bytes < (size_t)(n * d) * sizeof(Tin)) {
-    cudaFree(c.x);
-    c.x = nullptr;
-    c.x_bytes = 0;
-    WDGH_CUDA(cudaMalloc(&c.x, (size_t)(n * d) * sizeof(Tin)));
-    c.x_bytes = (size_t)(n * d) * sizeof(Tin);
-  }
+  WDGH_CUDA(grow(c.x, c.x_bytes, (size_t)(n * d) * sizeof(Tin)));
   const bool y16 = y_host && y_dtype == WDGH_DTYPE_BF16;
-  if (y16 && c.ystage_bytes < (size_t)(n * d) * 2) {
-    cudaFree(c.ystage);
-    c.ystage = nullptr;
-    c.ystage_bytes = 0;
-    WDGH_CUDA(cudaMalloc(&c.ystage, (size_t)(n * d) * 2));
-    c.ystage_bytes = (size_t)(n * d) * 2;
-  }
+  if (y16) WDGH_CUDA(grow(c.ystage, c.ystage_bytes, (size_t)(n * d) * 2));
   const size_t ysz = y16 ? 2 : sizeof(float);  // bytes of one element of Y on the host
   Tin *x = static_cast<Tin *>(c.x);
   cudaStream_t st = c.st, sc = c.st_copy, sb = c.st_back;
-  const bool ranged_ok = (d % 4 == 0) && (d >= 128 || d == 64 || d == 32);
-  const int64_t colw = y_host ? e2e_col_width(d) : 0;   // > 0: column-block form (Y travels back under the X copies)
-  const int KC = colw ? (int)(d / colw) : 0;
-  int R = colw ? e2e_col_rows() : 1;                    // row chunks per column block
-  while (R > 1 && (KC * R > 64 || R > e2e_chunks())) R /= 2;
-  const int K = colw ? R : (ranged_ok ? e2e_chunks() : 1);   // row blocks whose column segments are needed
+  const Schedule sched = schedule(d, y_host != nullptr);
+  const int64_t W = sched.W;
+  const int KC = sched.KC, R = sched.R;
+  // rows [r0, r0 + rows) of column block kc between two row-major n x d matrices: contiguous when the block is the
+  // whole width, pitched otherwise
+  auto copy_block = [&](void *dst, const void *src, size_t esz, int kc, int64_t r0, int64_t rows, cudaMemcpyKind kind,
+                        cudaStream_t stream) -> cudaError_t {
+    const size_t off = (size_t)(r0 * d + kc * W) * esz;
+    char *to = static_cast<char *>(dst) + off;
+    const char *from = static_cast<const char *>(src) + off;
+    if (W == d) return cudaMemcpyAsync(to, from, (size_t)(rows * d) * esz, kind, stream);
+    return cudaMemcpy2DAsync(to, d * esz, from, d * esz, W * esz, rows, kind, stream);
+  };
   // 1. graph + labels first (the compute stream needs them at once) ...
   WDGH_CUDA(cudaMemcpyAsync(c.rowptr, rowptr_host, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, sc));
   if (nnz) WDGH_CUDA(cudaMemcpyAsync(c.col, col_host, nnz * sizeof(int32_t), cudaMemcpyHostToDevice, sc));
   WDGH_CUDA(cudaMemcpyAsync(c.labels, labels_host, n * sizeof(int32_t), cudaMemcpyHostToDevice, sc));
   WDGH_CUDA(cudaEventRecord(c.ev_csr, sc));
-  // 2. ... then the feature matrix on the copy stream: column blocks (pitched, each in R row chunks) when Y goes back
-  //    to the host, row blocks otherwise
-  const int64_t blk = (n + K - 1) / K;
-  int64_t bounds_h[65];
-  for (int k = 0; k < K; ++k) bounds_h[k] = (int64_t)k * blk < n ? (int64_t)k * blk : n;
+  // 2. ... then the feature matrix on the copy stream, block by block and chunk by chunk (rows [bounds_h[r],
+  //    bounds_h[r + 1]) form row chunk r)
+  const int64_t blk = (n + R - 1) / R;
+  int64_t bounds_h[kRowChunks + 1];
+  for (int r = 0; r <= R; ++r) bounds_h[r] = std::min((int64_t)r * blk, n);
   for (int kc = 0; kc < KC; ++kc) {
     for (int r = 0; r < R; ++r) {
-      const int64_t r0 = bounds_h[r], r1 = (r0 + blk < n) ? r0 + blk : n;
-      if (r1 > r0)
-        WDGH_CUDA(cudaMemcpy2DAsync(x + r0 * d + kc * colw, d * sizeof(Tin), x_host + r0 * d + kc * colw,
-                                    d * sizeof(Tin), colw * sizeof(Tin), r1 - r0, cudaMemcpyHostToDevice, sc));
+      if (bounds_h[r + 1] > bounds_h[r])
+        WDGH_CUDA(copy_block(x, x_host, sizeof(Tin), kc, bounds_h[r], bounds_h[r + 1] - bounds_h[r],
+                             cudaMemcpyHostToDevice, sc));
       WDGH_CUDA(cudaEventRecord(c.ev_x[kc * R + r], sc));
     }
   }
-  for (int k = 0; k < K && !colw; ++k) {
-    const int64_t r0 = bounds_h[k], r1 = (r0 + blk < n) ? r0 + blk : n;
-    if (r1 > r0)
-      WDGH_CUDA(cudaMemcpyAsync(x + r0 * d, x_host + r0 * d, (size_t)(r1 - r0) * d * sizeof(Tin),
-                                cudaMemcpyHostToDevice, sc));
-    WDGH_CUDA(cudaEventRecord(c.ev_x[k], sc));
-  }
-  bounds_h[K] = n;
   WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_csr, 0));
   int64_t plan_host[8];
   int rc = wdgh_plan_build(c.rowptr, n, nnz, kHostPipelineThreshold, c.plan, cap, plan_host, st);
   if (rc) return rc;
   const int64_t ldp = (d + 3) & ~int64_t(3);
-  const int64_t n_part = plan_host[1];
-  if (n_part * ldp > c.partial_elems) {
-    cudaFree(c.partial);
-    c.partial = nullptr;
-    c.partial_elems = n_part * ldp;
-    WDGH_CUDA(cudaMalloc(&c.partial, c.partial_elems * sizeof(float)));
-  }
+  WDGH_CUDA(grow(c.partial, c.partial_bytes, (size_t)(plan_host[1] * ldp) * sizeof(float)));
   if (norm != WDGH_NORM_NONE) {
     rc = wdgh_degree_scale(c.rowptr, nullptr, n, norm, add_self_loop, c.dinv, nullptr, c.deg_code, st);
     if (rc) return rc;
@@ -241,7 +234,7 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
       return wdgh_spmm_csr_bf16(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, WDGH_DTYPE_F32, norm, add_self_loop, dinv,
                                 code, c.plan, plan_host, c.partial, 0, st);
   };
-  // the phase of row block k: y (+)= the entries whose column lies in block k; the last phase finalizes
+  // the phase of row chunk k: y (+)= the entries whose column lies in chunk k; the last phase finalizes
   auto phase = [&](int k, const Tin *xb, int64_t w, float *yb, int accumulate, int last) -> int {
     const int64_t *b = c.seg + (size_t)k * n, *e = c.seg + (size_t)(k + 1) * n;
     if constexpr (F32)
@@ -256,62 +249,31 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
   rc = wdgh_structure_counts(c.rowptr, c.col, n, nnz, c.labels, C, c.plan, plan_host, c.counters, c.node_sum, c.deg,
                              c.match, c.labels8, n, 0, st);
   if (rc) return rc;
-  if (colw) {
-    // 4'. per column block: one aggregation phase per arriving row chunk (R = 1: one full-graph launch); the Y block
-    //     leaves on the third stream as soon as its last phase (and, for a bf16 Y, its rounding) is done
-    if (R > 1) {
-      WDGH_CUDA(cudaMemcpyAsync(c.bounds, bounds_h, (R + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-      rc = wdgh_column_segments(c.rowptr, c.col, n, c.bounds, R + 1, c.seg, st);
-      if (rc) return rc;
-      rc = wdgh_plan_heavy_flags(c.plan, plan_host, n, c.skip, st);
-      if (rc) return rc;
-    }
-    for (int kc = 0; kc < KC; ++kc) {
-      const Tin *xb = x + kc * colw;
-      float *yb = c.y + kc * colw;
-      for (int r = 0; r < R; ++r) {
-        WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[kc * R + r], 0));
-        rc = (R == 1) ? full(xb, colw, yb) : phase(r, xb, colw, yb, r > 0, r == R - 1);
-        if (rc) return rc;
-      }
-      uint16_t *yb16 = y16 ? static_cast<uint16_t *>(c.ystage) + kc * colw : nullptr;
-      if (y16) {
-        rc = round_to_bf16(yb, n, colw, d, yb16, d, st);
-        if (rc) return rc;
-      }
-      const void *src = y16 ? static_cast<const void *>(yb16) : yb;
-      WDGH_CUDA(cudaEventRecord(c.ev_y[kc], st));
-      WDGH_CUDA(cudaStreamWaitEvent(sb, c.ev_y[kc], 0));
-      WDGH_CUDA(cudaMemcpy2DAsync(static_cast<char *>(y_host) + kc * colw * ysz, d * ysz, src, d * ysz, colw * ysz, n,
-                                  cudaMemcpyDeviceToHost, sb));
-    }
-  } else if (K == 1) {
-    WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[0], 0));
-    rc = full(x, d, c.y);
-    if (rc) return rc;
-  } else {
-    // 4. one aggregation phase per arriving feature block
-    WDGH_CUDA(cudaMemcpyAsync(c.bounds, bounds_h, (K + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    rc = wdgh_column_segments(c.rowptr, c.col, n, c.bounds, K + 1, c.seg, st);
+  // 4. per column block: one aggregation phase per arriving row chunk (R = 1: one full launch); the Y block leaves on
+  //    the third stream as soon as its last phase (and, for a bf16 Y, its rounding) is done
+  if (R > 1) {
+    WDGH_CUDA(cudaMemcpyAsync(c.bounds, bounds_h, (R + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    rc = wdgh_column_segments(c.rowptr, c.col, n, c.bounds, R + 1, c.seg, st);
     if (rc) return rc;
     rc = wdgh_plan_heavy_flags(c.plan, plan_host, n, c.skip, st);
     if (rc) return rc;
-    for (int k = 0; k < K; ++k) {
-      WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[k], 0));
-      rc = phase(k, x, d, c.y, k > 0, k == K - 1);
-      if (rc) return rc;
-    }
   }
-  // Y leaves on the copy stream as soon as the last phase is done; the counters follow on the compute stream
-  if (y_host && !colw) {
-    if (y16) {
-      rc = round_to_bf16(c.y, n, d, d, c.ystage, d, st);
+  for (int kc = 0; kc < KC; ++kc) {
+    const Tin *xb = x + kc * W;
+    float *yb = c.y + kc * W;
+    for (int r = 0; r < R; ++r) {
+      WDGH_CUDA(cudaStreamWaitEvent(st, c.ev_x[kc * R + r], 0));
+      rc = (R == 1) ? full(xb, W, yb) : phase(r, xb, W, yb, r > 0, r == R - 1);
       if (rc) return rc;
     }
-    WDGH_CUDA(cudaEventRecord(c.ev_csr, st));
-    WDGH_CUDA(cudaStreamWaitEvent(sc, c.ev_csr, 0));
-    WDGH_CUDA(cudaMemcpyAsync(y_host, y16 ? c.ystage : static_cast<void *>(c.y), n * d * ysz, cudaMemcpyDeviceToHost,
-                              sc));
+    if (!y_host) continue;
+    if (y16) {
+      rc = round_to_bf16(yb, n, W, d, static_cast<uint16_t *>(c.ystage) + kc * W, d, st);
+      if (rc) return rc;
+    }
+    WDGH_CUDA(cudaEventRecord(c.ev_y[kc], st));
+    WDGH_CUDA(cudaStreamWaitEvent(sb, c.ev_y[kc], 0));
+    WDGH_CUDA(copy_block(y_host, y16 ? c.ystage : static_cast<void *>(c.y), ysz, kc, 0, n, cudaMemcpyDeviceToHost, sb));
   }
   WDGH_CUDA(cudaMemcpyAsync(counters_host, c.counters, n_counters * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
   WDGH_CUDA(cudaMemcpyAsync(node_sum_host, c.node_sum, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -326,7 +288,7 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
     WDGH_CUDA(cudaMemcpyAsync(node_sum_host, c.node_sum, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
     WDGH_CUDA(cudaStreamSynchronize(st));
   }
-  if (y_host) WDGH_CUDA(cudaStreamSynchronize(colw ? sb : sc));
+  if (y_host) WDGH_CUDA(cudaStreamSynchronize(sb));
   return 0;
 }
 #undef WDGH_REQUIRE_AT
