@@ -205,6 +205,9 @@ int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *range_begin,
  *                       [1] the same with the stored diagonal counted as a matching entry
  *                           (utils/homophily_plot.py:92-100, which does not strip self-loops)
  *   deg_nsl / match_nsl int32[n]: per-row off-diagonal entry count / label matches (scratch AND output)
+ * A label counts as labelled when 0 <= l < num_classes.  Any other value -- negative, or >= num_classes -- is
+ * unlabelled: it indexes no class table and no pair bin, but the match counts (MATCH_ALL, match_nsl) still compare
+ * raw labels, so two such values match only when equal (hm.py:51).
  */
 #define WDGH_SC_MATCH_ALL   0
 #define WDGH_SC_MATCH_LAB   1
@@ -213,7 +216,8 @@ int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *range_begin,
 #define WDGH_SC_N_EMPTY     4
 #define WDGH_SC_NBINS       5
 #define WDGH_SC_N_NODES_NSL 6
-#define WDGH_SC_N_MULTI_NEG 7 /* labels < -1 seen while packing to 1 byte: re-run without labels_u8_scratch */
+#define WDGH_SC_N_MULTI_NEG 7 /* labels the 1-byte copy cannot represent exactly (< -1 or >= num_classes) seen
+                                 while packing: re-run without labels_u8_scratch */
 #define WDGH_SC_HEADER      8
 #define WDGH_SC_WORDS(C)    (WDGH_SC_HEADER + 3 * (C) + (C) * (C))
 int wdgh_structure_counts(const int64_t *rowptr, const int32_t *col, int64_t n, int64_t nnz,

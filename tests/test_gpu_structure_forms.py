@@ -1,14 +1,16 @@
 """Every form of the label-statistics pass (csrc/structure.cu) against an exact reference, at its dispatch boundaries.
 
-`wdgh_structure_counts` picks its kernels from the class count C, the label copy and the row lengths:
-  * C <= 63 with the 1-byte label copy: `structure_stream_kernel` ((C+1)^2 <= 4096 pair bins in shared memory) with
-    the per-node reductions in its epilogue and `structure_heavy_nodes_kernel` for the split rows;
+`wdgh_structure_counts` picks its edge kernel from the class count C and the label copy:
+  * C <= 63 with the 1-byte label copy: `structure_stream_kernel` ((C+1)^2 <= 4096 pair bins in shared memory);
   * otherwise `structure_rowgroup_kernel<uint8_t>` (C <= 254) or `<int32_t>` (C > 254, no 1-byte scratch, or the
-    re-run after several distinct negative labels), pair table in shared memory while C*C <= 4096, followed by
-    `structure_nodes_kernel` (class accumulators in shared memory while C <= 2048);
-  * rows longer than the plan threshold T: `structure_chunks_kernel<uint8_t | int32_t>`.
+    re-run after labels the 1-byte copy cannot represent: below -1 or >= C), pair table in shared memory while
+    C*C <= 4096, class accumulators in shared memory while C <= 2048.
+Both reduce the nodes of the rows up to the plan threshold T in their group epilogue; longer rows go through
+`structure_chunks_kernel<uint8_t | int32_t>` and then `structure_heavy_nodes_kernel`.  The edge-list form is
+`structure_coo_kernel` + `structure_nodes_kernel`.
 The reference is `oracle.structure_counts` plus the outputs it does not return, restated here in numpy.  Integers must be
-equal; the two float64 node sums may differ by the order of the atomic additions only (rtol 1e-12).
+equal; the two float64 node sums may differ by the order of the atomic additions only (rtol 1e-12).  A label >= C is
+unlabelled but compared raw (include/wdgh_b200.h): the reference sees it as a distinct negative value, -1000 - v.
 """
 import numpy as np
 import pytest
@@ -34,6 +36,7 @@ def reference(row, col, labels, n, C, coo=False, hist_self=False):
     (row, col), repeats counted with multiplicity."""
     row, col = np.asarray(row, np.int64), np.asarray(col, np.int64)
     lab = np.asarray(labels, np.int64)
+    lab = np.where(lab >= C, -1000 - lab, lab)
     o = O.structure_counts(row, col, lab, n, num_classes=C)
     d_all, d_nsl, m_nsl = o["deg_all"], o["deg_nsl"], o["match_nsl"]
     labelled = lab >= 0
@@ -112,6 +115,16 @@ def labels_with(rng, n, C, neg_frac=0.1):
     lab[rng.random(n) < neg_frac] = -1
     top = min(n - 1, 5)
     lab[top] = C - 1            # the largest class id is always present
+    return lab
+
+
+def with_out_of_range(rng, labels, C, frac=0.05):
+    """labels >= C, which only the C ABI can pass, on about `frac` of the nodes"""
+    vals = np.array([C, C + 1, 254, 255, 1000, 2 ** 31 - 1], np.int64)
+    vals = np.unique(vals[vals >= C])
+    lab = np.asarray(labels, np.int64).copy()
+    pick = rng.random(lab.shape[0]) < frac
+    lab[pick] = rng.choice(vals, int(pick.sum()))
     return lab
 
 
@@ -235,7 +248,8 @@ def test_row_group_shapes(W, n, T):
 
 
 # ---------------------------------------------------------------------------
-# 3. several distinct negative labels: the 1-byte copy folds them together, the host re-runs on int32 labels
+# 3. several distinct unlabelled values (-1, -2, labels >= C): the 1-byte copy folds them together, the host re-runs
+#    on int32 labels
 # ---------------------------------------------------------------------------
 @pytest.mark.parametrize("C", [3, 64, 200])
 def test_distinct_negative_labels(W, C):
@@ -244,12 +258,13 @@ def test_distinct_negative_labels(W, C):
     rng = np.random.default_rng(C)
     labels = labels_with(rng, n, C, neg_frac=0.15)
     labels[rng.random(n) < 0.1] = -2
-    n_below = int((labels < -1).sum())
+    labels = with_out_of_range(rng, labels, C)
+    n_below = int(((labels < -1) | (labels >= C)).sum())
     g = csr(W, row, col, n, T)
     lab32 = to_lab32(labels)
     ref = reference(row, col, labels, n, C)
-    folded = reference(row, col, np.maximum(labels, -1), n, C)
-    assert ref["match_all"] != folded["match_all"]   # raw equality must tell -1 and -2 apart
+    folded = reference(row, col, np.where((labels >= 0) & (labels < C), labels, -1), n, C)
+    assert ref["match_all"] != folded["match_all"]   # raw equality must tell -1, -2 and labels >= C apart
     s_u8, neg = run(W, g, lab32, C, "u8")
     assert neg == n_below
     assert s_u8.match_all == folded["match_all"]     # what the 1-byte copy sees, before the re-run
@@ -310,7 +325,7 @@ def test_edge_list_form(W, C, hist_self):
     dst = np.concatenate([col, col[rep], [7, 7, 7]])
     perm = rng.permutation(src.shape[0])
     src, dst = src[perm], dst[perm]
-    labels = labels_with(rng, n, C)
+    labels = with_out_of_range(rng, labels_with(rng, n, C), C)
     labels[7] = 0
     ei = torch.from_numpy(np.vstack([src, dst]).astype(np.int64))
     s = W.graph.structure_counts_coo(ei, n, to_lab32(labels), C, hist_includes_self_loops=hist_self)

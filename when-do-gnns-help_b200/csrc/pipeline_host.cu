@@ -279,7 +279,7 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
   WDGH_CUDA(cudaMemcpyAsync(node_sum_host, c.node_sum, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
   WDGH_CUDA(cudaStreamSynchronize(st));
   if (counters_host[WDGH_SC_N_MULTI_NEG] != 0) {
-    // several distinct negative labels: the 1-byte label copy folds them together, but the reference compares raw
+    // labels below -1 or >= C: the 1-byte label copy folds them together with -1, but the reference compares raw
     // labels (hm.py:51) -- redo the label pass on the int32 labels
     rc = wdgh_structure_counts(c.rowptr, c.col, n, nnz, c.labels, C, c.plan, plan_host, c.counters, c.node_sum, c.deg,
                                c.match, nullptr, n, 0, st);

@@ -6,8 +6,9 @@
 //                single shared-memory atomic per distinct key (C*C <= 4096 bins in shared memory,
 //                global 64-bit atomics beyond that); the scalar counters travel as per-lane
 //                registers and are combined by warp shuffles -- all counts are exact integers.
-//   node pass  : per node: f32(match)/f32(deg) for node homophily (hm.py:77-78), class sizes,
-//                class degree mass (hm.py:141), empty rows, bincount length.
+//   node part  : per node: f32(match)/f32(deg) for node homophily (hm.py:77-78), class sizes,
+//                class degree mass (hm.py:141), empty rows, bincount length -- in the group epilogue of
+//                the edge kernel; split rows after their chunks (structure_heavy_nodes_kernel).
 // HBM traffic per entry: 4 B of `col` plus one label gather that is served by L2 whenever the
 // label array (4 B/node) fits its 126 MB.
 #include <limits.h>
@@ -17,38 +18,119 @@
 
 namespace wdgh {
 
+constexpr int kClassSmemClasses = 2048;  // 2*C 64-bit class accumulators kept in shared memory per CTA
+
+// A label indexes the class tables only when 0 <= l < C.  Any other value -- negative, or >= C through the C ABI --
+// is unlabelled; match counts compare raw labels all the same (hm.py:51).
+__device__ __forceinline__ bool labelled(int l, int C) { return (unsigned)l < (unsigned)C; }
+
 struct EdgeAcc {
   unsigned match_all = 0, match_lab = 0, n_lab = 0, n_self = 0;
+
+  // one stored entry with endpoint labels li, lj; returns its class-pair key (both endpoints labelled, off the
+  // diagonal unless hist_self), -1 for none
+  __device__ __forceinline__ int add(int li, int lj, bool self, int C, bool hist_self = false) {
+    const bool same = (li == lj);
+    const bool both = labelled(li, C) && labelled(lj, C);
+    match_all += same;
+    match_lab += (same && both);
+    n_lab += both;
+    n_self += self;
+    return (both && (!self || hist_self)) ? li * C + lj : -1;
+  }
+  __device__ __forceinline__ void flush(unsigned long long *counters) {
+    long long v0 = warp_sum((long long)match_all), v1 = warp_sum((long long)match_lab);
+    long long v2 = warp_sum((long long)n_lab), v3 = warp_sum((long long)n_self);
+    if ((threadIdx.x & 31) == 0) {
+      if (v0) atomicAdd(&counters[WDGH_SC_MATCH_ALL], (unsigned long long)v0);
+      if (v1) atomicAdd(&counters[WDGH_SC_MATCH_LAB], (unsigned long long)v1);
+      if (v2) atomicAdd(&counters[WDGH_SC_N_LAB], (unsigned long long)v2);
+      if (v3) atomicAdd(&counters[WDGH_SC_N_SELF], (unsigned long long)v3);
+    }
+  }
 };
 
-__device__ __forceinline__ void visit(int64_t row, int li, int j, int lj, int C, EdgeAcc &a, int &m_nsl, int &d_nsl,
-                                      int &key, bool hist_self = false) {
-  const bool self = (j == row);
-  const bool same = (li == lj);
-  const bool both = (li >= 0) && (lj >= 0);
-  a.match_all += same;
-  a.match_lab += (same && both);
-  a.n_lab += both;
-  a.n_self += self;
-  if (!self) {
-    d_nsl += 1;
-    m_nsl += same;
-    if (both) key = li * C + lj;
-  } else if (hist_self && both) {
-    key = li * C + lj;
-  }
-}
+// Per-node reductions of the rows a thread owns: node-homophily sums, rows with an off-diagonal entry, empty rows and
+// the bincount length.  flush() combines them per warp (every lane of the warp calls it).
+struct NodeAcc {
+  double sum = 0.0, sum_self = 0.0;
+  unsigned n_nsl = 0, n_empty = 0;
+  long long nbins = 0;
 
-__device__ __forceinline__ void flush(EdgeAcc &a, unsigned long long *counters) {
-  long long v0 = warp_sum((long long)a.match_all), v1 = warp_sum((long long)a.match_lab);
-  long long v2 = warp_sum((long long)a.n_lab), v3 = warp_sum((long long)a.n_self);
-  if ((threadIdx.x & 31) == 0) {
-    if (v0) atomicAdd(&counters[WDGH_SC_MATCH_ALL], (unsigned long long)v0);
-    if (v1) atomicAdd(&counters[WDGH_SC_MATCH_LAB], (unsigned long long)v1);
-    if (v2) atomicAdd(&counters[WDGH_SC_N_LAB], (unsigned long long)v2);
-    if (v3) atomicAdd(&counters[WDGH_SC_N_SELF], (unsigned long long)v3);
+  // a row with d_nsl off-diagonal entries, m_nsl of them label matches (edge-list input: row lengths unknown)
+  __device__ __forceinline__ void add_nsl(int d_nsl, int m_nsl, int64_t global_row) {
+    if (d_nsl > 0) {
+      sum += (double)((float)m_nsl / (float)d_nsl);  // float32 division as torch does (hm.py:77)
+      n_nsl += 1;
+      nbins = max(nbins, (long long)(global_row + 1));  // rows do not come in order
+    }
   }
+  // the same with the stored row length deg_all known: empty rows, and the variant that counts the stored diagonal
+  // entries as matches (homophily_plot.py:92-100, which does not strip self loops)
+  __device__ __forceinline__ void add(int d_nsl, int m_nsl, int deg_all, int64_t global_row) {
+    add_nsl(d_nsl, m_nsl, global_row);
+    if (deg_all == 0) n_empty += 1;
+    else sum_self += (double)((float)(m_nsl + (deg_all - d_nsl)) / (float)deg_all);
+  }
+  // class size, class degree mass and (rare: no off-diagonal entry) isolated count of a node with label l
+  template <typename T>
+  static __device__ __forceinline__ void add_class(int l, int C, int d_nsl, T deg_all, T *cls_count, T *cls_deg,
+                                                   unsigned long long *counters) {
+    if (!labelled(l, C)) return;
+    atomicAdd(&cls_count[l], (T)1);
+    atomicAdd(&cls_deg[l], deg_all);
+    if (d_nsl == 0) atomicAdd(&counters[WDGH_SC_HEADER + 2 * C + (size_t)C * C + l], 1ull);
+  }
+  __device__ __forceinline__ void flush(unsigned long long *counters, double *node_sum) {
+    const double s0 = warp_sum(sum), s1 = warp_sum(sum_self);
+    const long long a0 = warp_sum((long long)n_nsl), a1 = warp_sum((long long)n_empty);
+    long long nbm = nbins;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) nbm = max(nbm, __shfl_xor_sync(0xffffffffu, nbm, o));
+    if ((threadIdx.x & 31) == 0) {
+      if (s0 != 0.0) atomicAdd(node_sum, s0);
+      if (s1 != 0.0) atomicAdd(node_sum + 1, s1);
+      if (a0) atomicAdd(&counters[WDGH_SC_N_NODES_NSL], (unsigned long long)a0);
+      if (a1) atomicAdd(&counters[WDGH_SC_N_EMPTY], (unsigned long long)a1);
+      if (nbm) atomicMax(&counters[WDGH_SC_NBINS], (unsigned long long)nbm);
+    }
+  }
+};
+
+// Counts of one CTA bound for global 64-bit counters: shared-memory words T while the table fits, otherwise the global
+// counters themselves.  Every thread of the CTA constructs it; the constructor ends with __syncthreads().
+template <typename T>
+struct CtaTable {
+  T *s;
+  unsigned long long *g;
+  int words;
+  bool smem;
+  __device__ __forceinline__ CtaTable(T *s_words, unsigned long long *g_words, int n_words, bool fits)
+      : s(s_words), g(g_words), words(n_words), smem(fits) {
+    if (smem)
+      for (int b = threadIdx.x; b < words; b += blockDim.x) s[b] = 0;
+    __syncthreads();
+  }
+  __device__ __forceinline__ T *ptr() const { return smem ? s : g; }         // T = unsigned long long
+  __device__ __forceinline__ void fold(int key) { fold_keys(key, s, g, smem); }  // T = unsigned
+  __device__ __forceinline__ void flush() {
+    if (!smem) return;
+    __syncthreads();
+    for (int b = threadIdx.x; b < words; b += blockDim.x)
+      if (s[b]) atomicAdd(&g[b], (unsigned long long)s[b]);
+  }
+};
+// the C x C class-pair histogram: 32-bit shared bins while C*C <= kHistSmemBins
+__device__ __forceinline__ CtaTable<unsigned> pair_table(unsigned *s, unsigned long long *counters, int C) {
+  return CtaTable<unsigned>(s, counters + WDGH_SC_HEADER + 2 * C, C * C, C * C <= kHistSmemBins);
 }
+// [C] class sizes, [C] class degree mass: 64-bit shared words while C <= kClassSmemClasses
+__device__ __forceinline__ CtaTable<unsigned long long> class_table(unsigned long long *s, unsigned long long *counters,
+                                                                    int C) {
+  return CtaTable<unsigned long long>(s, counters + WDGH_SC_HEADER, 2 * C, C <= kClassSmemClasses);
+}
+static size_t pair_smem(int C) { return ((size_t)C * C <= (size_t)kHistSmemBins) ? (size_t)C * C * sizeof(unsigned) : 0; }
+static size_t class_smem(int C) { return (C <= kClassSmemClasses) ? 2 * (size_t)C * sizeof(unsigned long long) : 0; }
 
 // label fetch: int32 labels as given, or the uint8 copy (0xFF = unlabelled) that keeps the gathered
 // array L2-resident for graphs up to ~100M nodes
@@ -68,30 +150,29 @@ __device__ __forceinline__ int load_label<uint8_t>(const uint8_t *p, int64_t i) 
 // lanes on a power-law graph).  The row slot of a stream position comes from a 5-step search in the scanned
 // row lengths; per-row counts are popcounts over the runs of equal row slots inside a 32-entry slice,
 // accumulated in shared memory and written coalesced at the end of the group.  Column ids are requested one
-// iteration ahead (and across the group boundary), label gathers right before they are consumed.
+// iteration ahead (and across the group boundary), label gathers right before they are consumed.  The per-node
+// reductions of the group's non-split rows ride in the group epilogue, as in the stream form below.
+// 4 CTAs / SM: the grid never holds more (launch in wdgh_structure_counts).
 template <typename L>
-__global__ void __launch_bounds__(256, 5)
+__global__ void __launch_bounds__(256, 4)
 structure_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__restrict__ col, int64_t n,
                           const L *__restrict__ labels, int C, int64_t threshold,
-                          unsigned long long *__restrict__ counters, int32_t *__restrict__ deg_nsl,
-                          int32_t *__restrict__ match_nsl, int64_t row_offset,
+                          unsigned long long *__restrict__ counters, double *__restrict__ node_sum,
+                          int32_t *__restrict__ deg_nsl, int32_t *__restrict__ match_nsl, int64_t row_offset,
                           unsigned long long *__restrict__ sched) {
-  extern __shared__ unsigned s_hist[];
+  extern __shared__ unsigned long long s_dyn64[];  // class_smem(C) bytes of class table, then the pair table
   __shared__ int s_off[8][2][33];
   __shared__ int64_t s_beg[8][2][32];
   __shared__ int s_match[8][2][32], s_self[8][2][32];
   constexpr unsigned kFull = 0xffffffffu;
   constexpr int EPL = 4;
-  const bool use_smem = (C * C <= kHistSmemBins);
-  unsigned long long *g_hist = counters + WDGH_SC_HEADER + 2 * C;
-  if (use_smem) {
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) s_hist[b] = 0;
-    __syncthreads();
-  }
+  CtaTable<unsigned long long> cls = class_table(s_dyn64, counters, C);
+  CtaTable<unsigned> pairs = pair_table(reinterpret_cast<unsigned *>(s_dyn64 + (cls.smem ? 2 * C : 0)), counters, C);
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int64_t W = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const int64_t n_groups = (n + 31) >> 5;
   EdgeAcc acc;
+  NodeAcc nodes;
 
   auto take = [&]() -> int64_t {
     unsigned long long t = 0;
@@ -147,10 +228,11 @@ structure_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__r
   int64_t g = (int64_t)blockIdx.x * 8 + wid;
   if (g < n_groups) {
     int64_t b, e;
-    int li_cur, li_next = -1, li_load;
+    int li_cur, li_next = -1, li_load, dall, n_dall = 0;  // dall: full row length (split rows included)
     load_bounds(g, b, e, li_cur);
     int buf = 0, total, len, n_total = 0, n_len = 0;
     publish(0, b, e, total, len);
+    dall = (int)(e - b);
     int64_t gn = take(), gnn = 0;
     load_bounds(gn, b, e, li_load);
     int j[EPL], rho[EPL], nj[EPL], nrho[EPL];
@@ -162,6 +244,7 @@ structure_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__r
           load_cols(buf, t0 + 32 * EPL, total, nj, nrho);
         } else {
           publish(buf ^ 1, b, e, n_total, n_len);
+          n_dall = (int)(e - b);
           li_next = li_load;
           load_cols(buf ^ 1, 0, n_total, nj, nrho);
           gnn = take();
@@ -181,15 +264,9 @@ structure_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__r
           const int lie = __shfl_sync(kFull, li_cur, rho[k]);
           const int64_t grow = (g << 5) + rho[k] + row_offset;
           const bool self = valid && ((int64_t)j[k] == grow);
-          const bool same = valid && (lie == lj[k]);
-          const bool both = valid && (lie >= 0) && (lj[k] >= 0);
-          acc.match_all += same;
-          acc.match_lab += (same && both);
-          acc.n_lab += both;
-          acc.n_self += self;
-          fold_keys((both && !self) ? lie * C + lj[k] : -1, s_hist, g_hist, use_smem);
+          pairs.fold(valid ? acc.add(lie, lj[k], self, C) : -1);
           // per-row counts: one popcount per run of equal row slots
-          const unsigned m = __ballot_sync(kFull, same && !self), sf = __ballot_sync(kFull, self);
+          const unsigned m = __ballot_sync(kFull, valid && !self && lie == lj[k]), sf = __ballot_sync(kFull, self);
           const int prev = __shfl_up_sync(kFull, rho[k], 1);
           const bool head = valid && (lane == 0 || prev != rho[k]);
           const unsigned heads = __ballot_sync(kFull, head);
@@ -218,28 +295,32 @@ structure_rowgroup_kernel(const int64_t *__restrict__ rowptr, const int32_t *__r
         }
       }
       __syncwarp();
+      // group epilogue: per-row outputs (split rows: zero here, the chunk kernel adds atomically) and the per-node
+      // reductions of the non-split rows this warp owns (split rows: structure_heavy_nodes_kernel)
       const int64_t r = (g << 5) + lane;
-      if (r < n) {  // split rows: zero here, the chunk kernel adds atomically
-        deg_nsl[r] = len - s_self[wid][buf][lane];
-        match_nsl[r] = s_match[wid][buf][lane];
+      if (r < n) {
+        const int dn = len - s_self[wid][buf][lane], mn = s_match[wid][buf][lane];
+        deg_nsl[r] = dn;
+        match_nsl[r] = mn;
+        if (dall <= threshold) {
+          nodes.add(dn, mn, len, r + row_offset);
+          NodeAcc::add_class(li_cur, C, dn, (unsigned long long)len, cls.ptr(), cls.ptr() + C, counters);
+        }
       }
       g = gn;
       gn = gnn;
       buf ^= 1;
       total = n_total;
       len = n_len;
+      dall = n_dall;
       li_cur = li_next;
       if (g >= n_groups) break;
     }
   }
-  flush(acc, counters);
-  if (use_smem) {
-    __syncthreads();
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) {
-      const unsigned v = s_hist[b];
-      if (v) atomicAdd(&g_hist[b], (unsigned long long)v);
-    }
-  }
+  acc.flush(counters);
+  nodes.flush(counters, node_sum);
+  cls.flush();
+  pairs.flush();
   sched_retire(sched, gridDim.x);
 }
 
@@ -280,9 +361,7 @@ structure_stream_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
   const int64_t W = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const int64_t n_groups = (n + 31) >> 5;
   unsigned n_self = 0, n_self_lab = 0;                  // warp-uniform
-  double sum = 0.0, sum_self = 0.0;                     // per lane (row owner)
-  unsigned n_nsl = 0, n_empty = 0;
-  long long nbins = 0;
+  NodeAcc nodes;                                        // per lane (row owner)
 
   auto take = [&]() -> int64_t {
     unsigned long long t = 0;
@@ -411,24 +490,13 @@ structure_stream_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
       // group epilogue: per-row outputs and the per-node reductions of the rows this warp owns
       const int64_t r = (g << 5) + lane;
       if (r < n) {
-        const int deg_all = dall;
-        const bool heavy = deg_all > threshold;
+        const bool heavy = dall > threshold;
         const int dn = len - my_self;
         deg_nsl[r] = heavy ? 0 : dn;       // split rows: zero here, the chunk kernel adds atomically
         match_nsl[r] = heavy ? 0 : my_match;
-        if (!heavy) {
-          if (dn > 0) {
-            sum += (double)((float)my_match / (float)dn);  // float32 division as torch does (hm.py:77)
-            n_nsl += 1;
-            nbins = max(nbins, (long long)(r + row_offset + 1));  // ticket order: groups do not come in row order
-          }
-          if (deg_all == 0) n_empty += 1;
-          else sum_self += (double)((float)(my_match + my_self) / (float)deg_all);  // homophily_plot.py:92-100
-          if (li_cur < C) {
-            atomicAdd(&s_cnt[li_cur], 1u);
-            atomicAdd(&s_deg[li_cur], (unsigned)deg_all);
-            if (dn == 0) atomicAdd(&counters[WDGH_SC_HEADER + 2 * C + (size_t)C * C + li_cur], 1ull);  // isolated: rare
-          }
+        if (!heavy) {                      // len == dall
+          nodes.add(dn, my_match, dall, r + row_offset);
+          NodeAcc::add_class(li_cur, C, dn, (unsigned)len, s_cnt, s_deg, counters);
         }
       }
       g = gn;
@@ -440,26 +508,15 @@ structure_stream_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
     }
   }
   // ---- per-warp scalars ----
-  {
-    const double s0 = warp_sum(sum), s1 = warp_sum(sum_self);
-    const long long a0 = warp_sum((long long)n_nsl), a1 = warp_sum((long long)n_empty);
-    long long nbm = nbins;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) nbm = max(nbm, __shfl_xor_sync(kFull, nbm, o));
-    if (lane == 0) {
-      if (s0 != 0.0) atomicAdd(node_sum, s0);
-      if (s1 != 0.0) atomicAdd(node_sum + 1, s1);
-      if (a0) atomicAdd(&counters[WDGH_SC_N_NODES_NSL], (unsigned long long)a0);
-      if (a1) atomicAdd(&counters[WDGH_SC_N_EMPTY], (unsigned long long)a1);
-      if (nbm) atomicMax(&counters[WDGH_SC_NBINS], (unsigned long long)nbm);
-      if (n_self) {
-        atomicAdd(&counters[WDGH_SC_N_SELF], (unsigned long long)n_self);
-        atomicAdd(&counters[WDGH_SC_MATCH_ALL], (unsigned long long)n_self);
-      }
-      if (n_self_lab) {
-        atomicAdd(&counters[WDGH_SC_MATCH_LAB], (unsigned long long)n_self_lab);
-        atomicAdd(&counters[WDGH_SC_N_LAB], (unsigned long long)n_self_lab);
-      }
+  nodes.flush(counters, node_sum);
+  if (lane == 0) {
+    if (n_self) {
+      atomicAdd(&counters[WDGH_SC_N_SELF], (unsigned long long)n_self);
+      atomicAdd(&counters[WDGH_SC_MATCH_ALL], (unsigned long long)n_self);
+    }
+    if (n_self_lab) {
+      atomicAdd(&counters[WDGH_SC_MATCH_LAB], (unsigned long long)n_self_lab);
+      atomicAdd(&counters[WDGH_SC_N_LAB], (unsigned long long)n_self_lab);
     }
   }
   // ---- per-CTA tables: the pair table also yields the scalar counters ----
@@ -501,36 +558,31 @@ __global__ void structure_heavy_nodes_kernel(const int64_t *__restrict__ rowptr,
                                              int64_t row_offset) {
   const int64_t n_heavy = plan[kPlanNHeavy];
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  unsigned long long *g_cls = counters + WDGH_SC_HEADER;
+  NodeAcc nodes;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_heavy; k += stride) {
     const int64_t i = plan_heavy_row(plan)[k];
     const int d = deg_nsl[i], m = match_nsl[i];
-    const int64_t deg_all = rowptr[i + 1] - rowptr[i];
-    if (d > 0) {
-      atomicAdd(node_sum, (double)((float)m / (float)d));
-      atomicAdd(&counters[WDGH_SC_N_NODES_NSL], 1ull);
-      atomicMax(&counters[WDGH_SC_NBINS], (unsigned long long)(i + row_offset + 1));
-    }
-    atomicAdd(node_sum + 1, (double)((float)(m + (deg_all - d)) / (float)deg_all));
-    const int l = labels[i + row_offset];
-    if (l >= 0 && l < C) {
-      atomicAdd(&counters[WDGH_SC_HEADER + l], 1ull);
-      atomicAdd(&counters[WDGH_SC_HEADER + C + l], (unsigned long long)deg_all);
-      if (d == 0) atomicAdd(&counters[WDGH_SC_HEADER + 2 * C + (size_t)C * C + l], 1ull);
-    }
+    const int deg_all = (int)(rowptr[i + 1] - rowptr[i]);
+    nodes.add(d, m, deg_all, i + row_offset);
+    NodeAcc::add_class(labels[i + row_offset], C, d, (unsigned long long)deg_all, g_cls, g_cls + C, counters);
   }
+  nodes.flush(counters, node_sum);
 }
 
-// int32 labels -> uint8 (0xFF = negative / unlabelled); requires C <= 254
-// counters[WDGH_SC_N_MULTI_NEG] counts labels < -1: distinct negative labels all map to 0xFF, so their
-// mutual (in)equality (hm.py:51 compares raw labels) is only exact on the int32 path -- the host re-runs it.
-__global__ void labels_to_u8_kernel(const int32_t *__restrict__ in, int64_t n, uint8_t *__restrict__ out,
+// int32 labels -> uint8 (0xFF = unlabelled); requires C <= 254.
+// counters[WDGH_SC_N_MULTI_NEG] counts the labels the 1-byte copy cannot represent exactly, those below -1 or >= C:
+// they all map to 0xFF like -1, so their mutual (in)equality (hm.py:51 compares raw labels) is only exact on the
+// int32 path -- the host re-runs it.
+__global__ void labels_to_u8_kernel(const int32_t *__restrict__ in, int64_t n, int C, uint8_t *__restrict__ out,
                                     unsigned long long *__restrict__ counters) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   long long odd = 0;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     const int v = in[i];
-    out[i] = (v < 0 || v > 254) ? (uint8_t)255 : (uint8_t)v;
-    odd += (v < -1);
+    const bool lab = labelled(v, C);
+    out[i] = lab ? (uint8_t)v : (uint8_t)255;
+    odd += (!lab && v != -1);
   }
   odd = warp_sum(odd);
   if ((threadIdx.x & 31) == 0 && odd) atomicAdd(&counters[WDGH_SC_N_MULTI_NEG], (unsigned long long)odd);
@@ -544,12 +596,7 @@ structure_chunks_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
                         int64_t n_chunks, unsigned long long *__restrict__ counters,
                         int32_t *__restrict__ deg_nsl, int32_t *__restrict__ match_nsl, int64_t row_offset) {
   extern __shared__ unsigned s_hist[];
-  const bool use_smem = (C * C <= kHistSmemBins);
-  unsigned long long *g_hist = counters + WDGH_SC_HEADER + 2 * C;
-  if (use_smem) {
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) s_hist[b] = 0;
-    __syncthreads();
-  }
+  CtaTable<unsigned> pairs = pair_table(s_hist, counters, C);
   const int lane = threadIdx.x & 31;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const int64_t cap = plan[kPlanCapacity], T = plan[kPlanThreshold];
@@ -568,9 +615,12 @@ structure_chunks_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
       if (idx < e) {
         const int j = __ldg(col + idx);
         const int lj = load_label<L>(labels, j);
-        visit(row + row_offset, li, j, lj, C, acc, m_nsl, d_nsl, key);
+        const bool self = (j == row + row_offset);
+        key = acc.add(li, lj, self, C);
+        d_nsl += !self;
+        m_nsl += (!self && li == lj);
       }
-      fold_keys(key, s_hist, g_hist, use_smem);
+      pairs.fold(key);
     }
     m_nsl = (int)warp_sum((long long)m_nsl);
     d_nsl = (int)warp_sum((long long)d_nsl);
@@ -579,30 +629,19 @@ structure_chunks_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
       atomicAdd(&match_nsl[row], m_nsl);
     }
   }
-  flush(acc, counters);
-  if (use_smem) {
-    __syncthreads();
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) {
-      const unsigned v = s_hist[b];
-      if (v) atomicAdd(&g_hist[b], (unsigned long long)v);
-    }
-  }
+  acc.flush(counters);
+  pairs.flush();
 }
 
 // Edge-list input (an arbitrary, possibly unsorted / repeated `edge_index` as handed to
 // node_homophily_edge_idx / compact_matrix_edge_idx, hm.py:71,81): one lane per listed edge,
 // per-node counts through 32-bit global atomics.  deg / match must be zeroed by the caller.
 __global__ void __launch_bounds__(256)
-structure_coo_kernel(const int64_t *__restrict__ edge_index, int64_t E, int64_t n,
-                     const int32_t *__restrict__ labels, int C, unsigned long long *__restrict__ counters,
-                     int32_t *__restrict__ deg_nsl, int32_t *__restrict__ match_nsl, bool hist_self) {
+structure_coo_kernel(const int64_t *__restrict__ edge_index, int64_t E, const int32_t *__restrict__ labels, int C,
+                     unsigned long long *__restrict__ counters, int32_t *__restrict__ deg_nsl,
+                     int32_t *__restrict__ match_nsl, bool hist_self) {
   extern __shared__ unsigned s_hist[];
-  const bool use_smem = (C * C <= kHistSmemBins);
-  unsigned long long *g_hist = counters + WDGH_SC_HEADER + 2 * C;
-  if (use_smem) {
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) s_hist[b] = 0;
-    __syncthreads();
-  }
+  CtaTable<unsigned> pairs = pair_table(s_hist, counters, C);
   EdgeAcc acc;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   const int64_t rounds = (E + stride - 1) / stride;  // uniform trip count for the warp-wide fold
@@ -612,81 +651,36 @@ structure_coo_kernel(const int64_t *__restrict__ edge_index, int64_t E, int64_t 
     if (t < E) {
       const int64_t src = edge_index[t], dst = edge_index[E + t];
       const int li = __ldg(labels + src), lj = __ldg(labels + dst);
-      int m = 0, d = 0;
-      visit(src, li, (int)dst, lj, C, acc, m, d, key, hist_self);
-      if (d) atomicAdd(&deg_nsl[src], 1);
-      if (m) atomicAdd(&match_nsl[src], 1);
+      const bool self = (dst == src);
+      key = acc.add(li, lj, self, C, hist_self);
+      if (!self) {
+        atomicAdd(&deg_nsl[src], 1);
+        if (li == lj) atomicAdd(&match_nsl[src], 1);
+      }
     }
-    fold_keys(key, s_hist, g_hist, use_smem);
+    pairs.fold(key);
   }
-  flush(acc, counters);
-  if (use_smem) {
-    __syncthreads();
-    for (int b = threadIdx.x; b < C * C; b += blockDim.x) {
-      const unsigned v = s_hist[b];
-      if (v) atomicAdd(&g_hist[b], (unsigned long long)v);
-    }
-  }
+  acc.flush(counters);
+  pairs.flush();
 }
 
-// Per-node reductions.  Shared memory: 2*C 64-bit class accumulators when C <= 2048.
+// Per-node reductions of the edge-list form.  Row lengths are unknown there: no empty rows, no diagonal variant of
+// the node sum, no class degree mass.
 __global__ void __launch_bounds__(256)
-structure_nodes_kernel(const int64_t *__restrict__ rowptr, int64_t n, const int32_t *__restrict__ labels, int C,
-                       const int32_t *__restrict__ deg_nsl, const int32_t *__restrict__ match_nsl,
-                       unsigned long long *__restrict__ counters, double *__restrict__ node_sum,
-                       int64_t row_offset) {
-  extern __shared__ unsigned long long s_cls[];  // [C] class_count, [C] class_deg
-  const bool use_smem = (C <= 2048);
-  unsigned long long *g_cls = counters + WDGH_SC_HEADER;
-  if (use_smem) {
-    for (int b = threadIdx.x; b < 2 * C; b += blockDim.x) s_cls[b] = 0ull;
-    __syncthreads();
-  }
-  unsigned long long *cls = use_smem ? s_cls : g_cls;
-  double sum = 0.0, sum_self = 0.0;
-  long long n_nsl = 0, n_empty = 0, nbins = 0;
-  unsigned long long *g_iso = counters + WDGH_SC_HEADER + 2 * C + (size_t)C * C;
+structure_nodes_kernel(int64_t n, const int32_t *__restrict__ labels, int C, const int32_t *__restrict__ deg_nsl,
+                       const int32_t *__restrict__ match_nsl, unsigned long long *__restrict__ counters,
+                       double *__restrict__ node_sum) {
+  extern __shared__ unsigned long long s_cls[];
+  CtaTable<unsigned long long> cls = class_table(s_cls, counters, C);
+  NodeAcc nodes;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
     const int d = deg_nsl[i], m = match_nsl[i];
-    const int64_t deg_all = rowptr ? rowptr[i + 1] - rowptr[i] : 1;  // edge-list input: row lengths unknown
-    if (d > 0) {
-      sum += (double)((float)m / (float)d);  // float32 division as torch does (hm.py:77)
-      n_nsl += 1;
-      nbins = i + row_offset + 1;  // i is increasing per thread
-    }
-    if (deg_all == 0) n_empty += 1;
-    if (rowptr && deg_all > 0) {  // diagonal entries kept and counted as matches (homophily_plot.py:92-100)
-      const int64_t self = deg_all - d;
-      sum_self += (double)((float)(m + self) / (float)deg_all);
-    }
-    const int l = labels[i + row_offset];
-    if (l >= 0 && l < C && d == 0) atomicAdd(&g_iso[l], 1ull);  // rare: isolated nodes only
-    if (l >= 0 && l < C) {
-      atomicAdd(&cls[l], 1ull);
-      if (rowptr) atomicAdd(&cls[C + l], (unsigned long long)deg_all);
-    }
+    nodes.add_nsl(d, m, i);
+    NodeAcc::add_class(labels[i], C, d, 0ull, cls.ptr(), cls.ptr() + C, counters);
   }
-  sum = warp_sum(sum);
-  sum_self = warp_sum(sum_self);
-  n_nsl = warp_sum(n_nsl);
-  n_empty = warp_sum(n_empty);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) nbins = max(nbins, __shfl_xor_sync(0xffffffffu, nbins, o));
-  if ((threadIdx.x & 31) == 0) {
-    if (sum != 0.0) atomicAdd(node_sum, sum);
-    if (sum_self != 0.0) atomicAdd(node_sum + 1, sum_self);
-    if (n_nsl) atomicAdd(&counters[WDGH_SC_N_NODES_NSL], (unsigned long long)n_nsl);
-    if (n_empty) atomicAdd(&counters[WDGH_SC_N_EMPTY], (unsigned long long)n_empty);
-    if (nbins) atomicMax(&counters[WDGH_SC_NBINS], (unsigned long long)nbins);
-  }
-  if (use_smem) {
-    __syncthreads();
-    for (int b = threadIdx.x; b < 2 * C; b += blockDim.x) {
-      const unsigned long long v = s_cls[b];
-      if (v) atomicAdd(&g_cls[b], v);
-    }
-  }
+  nodes.flush(counters, node_sum);
+  cls.flush();
 }
 
 // edge_homophily with a 2-D label matrix: elementwise equality of the two label rows (hm.py:51)
@@ -708,18 +702,6 @@ label_rows_equal_kernel(const int64_t *__restrict__ rowptr, const int32_t *__res
   if (lane == 0 && cnt) atomicAdd(out, (unsigned long long)cnt);
 }
 
-// generic edge pass (int32 labels, or more classes than the shared-memory pair table of the stream kernel holds)
-template <typename L>
-static int launch_edge_rows(const int64_t *rowptr, const int32_t *col, int64_t n, const L *labels, int C,
-                            int64_t threshold, unsigned long long *cnt, int32_t *deg_nsl, int32_t *match_nsl,
-                            size_t hist_smem, cudaStream_t st, int64_t row_offset, unsigned long long *sched) {
-  const int64_t n_groups = ceil_div(n, 32);
-  structure_rowgroup_kernel<L><<<persistent_grid(ceil_div(n_groups, 8), 4), 256, hist_smem, st>>>(
-      rowptr, col, n, labels, C, threshold, cnt, deg_nsl, match_nsl, row_offset, sched);
-  WDGH_LAUNCHED("structure_rowgroup_kernel");
-  return 0;
-}
-
 }  // namespace wdgh
 
 using namespace wdgh;
@@ -734,7 +716,7 @@ static int structure_prepare(const int32_t *labels, int64_t n_labels, int C, uin
   *labels8_out = nullptr;
   if (labels_u8_scratch != nullptr && C <= 254 && n_labels > 0) {
     labels_to_u8_kernel<<<persistent_grid(ceil_div(n_labels, 256), 8), 256, 0, st>>>(
-        labels, n_labels, labels_u8_scratch, reinterpret_cast<unsigned long long *>(counters));
+        labels, n_labels, C, labels_u8_scratch, reinterpret_cast<unsigned long long *>(counters));
     WDGH_LAUNCHED("labels_to_u8_kernel");
     *labels8_out = labels_u8_scratch;
   }
@@ -758,27 +740,29 @@ extern "C" int wdgh_structure_counts(const int64_t *rowptr, const int32_t *col, 
   if (rc || n == 0) return rc;
   unsigned long long *cnt = reinterpret_cast<unsigned long long *>(counters);
   unsigned long long *sched = plan_sched(plan_i64, kPlanLabelTicket);
-  const size_t hist_smem = ((size_t)C * C <= (size_t)kHistSmemBins) ? (size_t)C * C * sizeof(unsigned) : 0;
+  const size_t hist_smem = pair_smem(C);
   const int64_t threshold = plan_host[2], n_heavy = plan_host[0], n_chunks = plan_host[1];
-  const int64_t n_groups = ceil_div(n, 32);
-  // default: stream kernel with the per-node reductions folded in
+  const unsigned edge_grid = persistent_grid(ceil_div(ceil_div(n, 32), 8), 4);
+  // every form: edge pass with the per-node reductions of the non-split rows -> split-row chunks -> split-row nodes
   const bool stream_form = labels8 != nullptr && (size_t)(C + 1) * (C + 1) <= (size_t)kHistSmemBins &&
                            n + row_offset < (int64_t)INT32_MAX;
   if (stream_form) {
     const size_t smem = ((size_t)(C + 1) * (C + 1) + 2 * (size_t)(C + 1)) * sizeof(unsigned);
     // 4 CTAs / SM (64 registers, 76 B of spills): 5.89 ms on the 976M-entry graph against 6.16 ms at 3 CTAs / SM
     // (76 registers, no spills) and 6.71 ms at 5 (48 registers)
-    structure_stream_kernel<<<persistent_grid(ceil_div(n_groups, 8), 4), 256, smem, st>>>(
-        rowptr, col, n, labels8, C, threshold, cnt, node_sum, deg_nsl, match_nsl, row_offset, sched);
+    structure_stream_kernel<<<edge_grid, 256, smem, st>>>(rowptr, col, n, labels8, C, threshold, cnt, node_sum,
+                                                          deg_nsl, match_nsl, row_offset, sched);
     WDGH_LAUNCHED("structure_stream_kernel");
-  } else if (labels8) {
-    rc = launch_edge_rows<uint8_t>(rowptr, col, n, labels8, C, threshold, cnt, deg_nsl, match_nsl, hist_smem, st,
-                                   row_offset, sched);
   } else {
-    rc = launch_edge_rows<int32_t>(rowptr, col, n, labels, C, threshold, cnt, deg_nsl, match_nsl, hist_smem, st,
-                                   row_offset, sched);
+    const size_t smem = class_smem(C) + hist_smem;
+    if (labels8)
+      structure_rowgroup_kernel<uint8_t><<<edge_grid, 256, smem, st>>>(rowptr, col, n, labels8, C, threshold, cnt,
+                                                                       node_sum, deg_nsl, match_nsl, row_offset, sched);
+    else
+      structure_rowgroup_kernel<int32_t><<<edge_grid, 256, smem, st>>>(rowptr, col, n, labels, C, threshold, cnt,
+                                                                       node_sum, deg_nsl, match_nsl, row_offset, sched);
+    WDGH_LAUNCHED("structure_rowgroup_kernel");
   }
-  if (rc) return rc;
   if (n_chunks > 0) {  // split rows: one warp per chunk
     const unsigned grid = persistent_grid(ceil_div(n_chunks, 8), 8);
     if (labels8)
@@ -789,18 +773,11 @@ extern "C" int wdgh_structure_counts(const int64_t *rowptr, const int32_t *col, 
                                                                     deg_nsl, match_nsl, row_offset);
     WDGH_LAUNCHED("structure_chunks_kernel");
   }
-  if (stream_form) {
-    if (n_heavy > 0) {
-      structure_heavy_nodes_kernel<<<persistent_grid(ceil_div(n_heavy, 256), 4), 256, 0, st>>>(
-          rowptr, labels, C, plan_i64, deg_nsl, match_nsl, cnt, node_sum, row_offset);
-      WDGH_LAUNCHED("structure_heavy_nodes_kernel");
-    }
-    return 0;
+  if (n_heavy > 0) {
+    structure_heavy_nodes_kernel<<<persistent_grid(ceil_div(n_heavy, 256), 4), 256, 0, st>>>(
+        rowptr, labels, C, plan_i64, deg_nsl, match_nsl, cnt, node_sum, row_offset);
+    WDGH_LAUNCHED("structure_heavy_nodes_kernel");
   }
-  const size_t cls_smem = (C <= 2048) ? 2 * (size_t)C * sizeof(unsigned long long) : 0;
-  structure_nodes_kernel<<<persistent_grid(ceil_div(n, 256), 8), 256, cls_smem, st>>>(rowptr, n, labels, C, deg_nsl,
-                                                                                     match_nsl, cnt, node_sum, row_offset);
-  WDGH_LAUNCHED("structure_nodes_kernel");
   return 0;
 }
 
@@ -814,22 +791,19 @@ extern "C" int wdgh_structure_counts_coo(const int64_t *edge_index, int64_t num_
                "wdgh_structure_counts_coo: bad shape");
   cudaStream_t st = as_stream(stream);
   const int C = num_classes;
-  const size_t n_counters = WDGH_SC_WORDS((size_t)C);
-  WDGH_CUDA(cudaMemsetAsync(counters, 0, n_counters * sizeof(int64_t), st));
-  WDGH_CUDA(cudaMemsetAsync(node_sum, 0, 2 * sizeof(double), st));
-  if (n == 0) return 0;
+  const uint8_t *labels8 = nullptr;
+  int rc = structure_prepare(labels, 0, C, nullptr, counters, node_sum, &labels8, st);
+  if (rc || n == 0) return rc;
   WDGH_CUDA(cudaMemsetAsync(deg_nsl, 0, n * sizeof(int32_t), st));
   WDGH_CUDA(cudaMemsetAsync(match_nsl, 0, n * sizeof(int32_t), st));
   unsigned long long *cnt = reinterpret_cast<unsigned long long *>(counters);
-  const size_t hist_smem = ((size_t)C * C <= (size_t)kHistSmemBins) ? (size_t)C * C * sizeof(unsigned) : 0;
   if (num_edges > 0) {
-    structure_coo_kernel<<<persistent_grid(ceil_div(num_edges, 256), 8), 256, hist_smem, st>>>(
-        edge_index, num_edges, n, labels, C, cnt, deg_nsl, match_nsl, hist_includes_self_loops != 0);
+    structure_coo_kernel<<<persistent_grid(ceil_div(num_edges, 256), 8), 256, pair_smem(C), st>>>(
+        edge_index, num_edges, labels, C, cnt, deg_nsl, match_nsl, hist_includes_self_loops != 0);
     WDGH_LAUNCHED("structure_coo_kernel");
   }
-  const size_t cls_smem = (C <= 2048) ? 2 * (size_t)C * sizeof(unsigned long long) : 0;
-  structure_nodes_kernel<<<persistent_grid(ceil_div(n, 256), 8), 256, cls_smem, st>>>(nullptr, n, labels, C, deg_nsl,
-                                                                                     match_nsl, cnt, node_sum, 0);
+  structure_nodes_kernel<<<persistent_grid(ceil_div(n, 256), 8), 256, class_smem(C), st>>>(n, labels, C, deg_nsl,
+                                                                                          match_nsl, cnt, node_sum);
   WDGH_LAUNCHED("structure_nodes_kernel");
   return 0;
 }

@@ -393,7 +393,7 @@ def structure_counts_raw(g: CSRGraph, labels32, num_classes, scratch=None):
 def structure_counts(g: CSRGraph, labels32, num_classes) -> StructureCounts:
     counters, node_sum, deg, match, _ = structure_counts_raw(g, labels32, num_classes)
     if int(counters[_lib.SC_N_MULTI_NEG].item()):
-        # several distinct negative labels: the 1-byte label copy folds them together, redo on int32 labels
+        # labels below -1 or >= num_classes: the 1-byte label copy folds them together with -1, redo on int32 labels
         c = int(num_classes)
         scratch = (counters, node_sum, deg, match, None)
         counters, node_sum, deg, match, _ = structure_counts_raw(g, labels32, c, scratch)
