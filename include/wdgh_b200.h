@@ -288,6 +288,22 @@ int wdgh_gather_rows(const float *x, int64_t d, int64_t ldx, const int64_t *ids,
 /* w[m][C]: w[i][c] = sum (is_mean=0) or mean (is_mean=1) over j with labels[j]==c of g[i][j] (hm.py:201-206) */
 int wdgh_class_colsum(const float *g, int64_t m, int64_t ldg, const int32_t *labels, int32_t num_classes,
                       int is_mean, float *w, void *stream);
+/* The same w without the m x m matrix g = z z^T: w[i][c] = sum (is_mean = 0) / mean (is_mean = 1) over j with
+ * labels[j] == c of <z_i, z_j>, computed as <z_i, s_c> with the class sums s_c = sum_{j: labels[j] == c} z_j
+ * (hm.py:192,199-206; homophily_plot.py similarity, non-NTK branch :196-206).  z float32[m][d] with row stride ldz >= d,
+ * any d >= 1, any C >= 1; m = 0 does nothing.  w float32[m][C] row-major, as wdgh_las_score takes it.
+ *   Summation order: s and the class counts are accumulated in fp64.  The rows are cut into contiguous segments
+ *   (their number and bounds depend on m, d and C only); each segment is summed in row order into its own partial
+ *   table, and the partials are added in segment order (8 contiguous runs, then the run sums).  w[i][c] =
+ *   f32(sum_k z[i][k] * s[c][k]) with products and sum in fp64 in k order, or f32(that sum / count) -- one rounding
+ *   to float32 for the sum, fp64 division then one rounding for the mean.  No atomics: the result is a function of
+ *   the inputs alone, independent of the device's SM count and of scheduling.
+ *   A label outside [0, C) joins no class (as in wdgh_class_colsum).  An empty class gives 0 (sum) and NaN (mean).
+ *   workspace: double[wdgh_class_inner_workspace_doubles(m, d, C)], at most C (d + 1) + max(C (d + 1), 2^22)
+ *   doubles (32 MiB plus two [C][d + 1] tables); the size function returns -1 for invalid sizes. */
+int64_t wdgh_class_inner_workspace_doubles(int64_t m, int64_t d, int32_t num_classes);
+int wdgh_class_inner_sums(const float *z, int64_t m, int64_t d, int64_t ldz, const int32_t *labels,
+                          int32_t num_classes, int is_mean, double *workspace, float *w, void *stream);
 /* aggregation-similarity score from w (hm.py:207-229).  label_rows: float32[m][C] (the `label` argument).
  * *count (device uint64) = number of nodes whose indicator is true; the score is count / m.
  * scratch_c: float32[C]. */

@@ -67,6 +67,8 @@ SIGNATURES = {
     "wdgh_gram": [_p, _i64, _i64, _i64, _p, _i64, _int, _p, _p],
     "wdgh_gather_rows": [_p, _i64, _i64, _p, _i64, _p, _i64, _p],
     "wdgh_class_colsum": [_p, _i64, _i64, _p, _i32, _int, _p, _p],
+    "wdgh_class_inner_workspace_doubles": [_i64, _i64, _i32],
+    "wdgh_class_inner_sums": [_p, _i64, _i64, _i64, _p, _i32, _int, _p, _p, _p],
     "wdgh_las_score": [_p, _p, _p, _i64, _i32, _int, _int, _int, _p, _p, _p],
     "wdgh_ntk_clamp_transform": [_p, _i64, _i64, _p],
     "wdgh_gntk_transform": [_p, _i64, _i64, _int, _p, _p],
@@ -74,7 +76,8 @@ SIGNATURES = {
     "wdgh_pipeline_host_bf16": [_p, _p, _i64, _i64, _p, _i64, _p, _i32, _int, _int, _p, _int, _p, _p],
     "wdgh_pipeline_host_release": [],
 }
-_RESTYPE = {"wdgh_last_error": C.c_char_p, "wdgh_launch_count": C.c_uint64, "wdgh_gram_workspace_floats": C.c_int64}
+_RESTYPE = {"wdgh_last_error": C.c_char_p, "wdgh_launch_count": C.c_uint64, "wdgh_gram_workspace_floats": C.c_int64,
+            "wdgh_class_inner_workspace_doubles": C.c_int64}
 
 for _name, _args in SIGNATURES.items():
     _fn = getattr(lib, _name)  # AttributeError here = header / library mismatch

@@ -567,6 +567,39 @@ def class_colsum(gm, labels32, num_classes, is_mean=False):
     return w
 
 
+def class_inner_sums(z, labels32, num_classes, is_mean=False):
+    """w[m, C]: sum (or mean) over the rows j of class c of <z_i, z_j>, computed as <z_i, s_c> with fp64 class sums
+    s_c (two passes over z, no m x m Gram; include/wdgh_b200.h wdgh_class_inner_sums).  A float32 view with unit
+    column stride (a row gather or a column slab of a wider matrix) is read in place."""
+    if not (isinstance(z, torch.Tensor) and z.device.type == "cuda" and z.dtype == torch.float32 and z.dim() == 2
+            and z.stride(1) == 1 and z.stride(0) >= z.shape[1]):
+        z = _cuda(z, torch.float32)
+    m, d, c = int(z.shape[0]), int(z.shape[1]), int(num_classes)
+    if labels32.shape[0] < m:
+        raise ValueError(f"labels must cover the {m} rows of z, got {labels32.shape[0]}")
+    w = torch.empty((m, c), dtype=torch.float32, device=z.device)
+    words = int(lib.wdgh_class_inner_workspace_doubles(m, d, c))
+    if words < 0:
+        raise ValueError(f"bad class-sum shape m={m} d={d} C={c}")
+    ws = torch.empty(max(1, words), dtype=torch.float64, device=z.device)
+    check(lib.wdgh_class_inner_sums(ptr(z), m, d, max(1, z.stride(0)), ptr(labels32), c, int(bool(is_mean)), ptr(ws),
+                                    ptr(w), stream_ptr()), "wdgh_class_inner_sums")
+    return w
+
+
+# Above this many rows las_weights takes the Gram-free class sums: the Gram is 4 m^2 bytes (17 GB at 65,536 rows).
+# Up to it the Gram path is kept, so every result of earlier releases at those sizes stays bit-identical.
+GRAM_SIMILARITY_MAX_ROWS = 65536
+
+
+def las_weights(z, labels32, num_classes, is_mean):
+    """The class table w[m, C] of the aggregation similarity (hm.py:199-206): class sums (or means) of the rows of
+    z z^T.  Up to GRAM_SIMILARITY_MAX_ROWS rows from the Gram (class_colsum(gram(z))), above from class_inner_sums."""
+    if int(z.shape[0]) <= GRAM_SIMILARITY_MAX_ROWS:
+        return class_colsum(gram(z), labels32, num_classes, is_mean=is_mean)
+    return class_inner_sums(z, labels32, num_classes, is_mean=is_mean)
+
+
 def las_count(w, labels32, label_rows, hard, lp, is_sum) -> int:
     m, c = int(w.shape[0]), int(w.shape[1])
     label_rows = _cuda(label_rows, torch.float32)

@@ -222,7 +222,8 @@ def _ids(mask_or_ids, device):
 
 
 def similarity(features, adj, label, hard=None, LP=1, ifsum=1, idx_train=None):
-    """hm.py:190-229: aggregation similarity score (soft / hard LAS) from (A X)(A X)^T."""
+    """hm.py:190-229: aggregation similarity score (soft / hard LAS) from (A X)(A X)^T -- for more than
+    graph.GRAM_SIMILARITY_MAX_ROWS rows without forming it (class sums of A X), so whole graphs of any size work."""
     z = _propagate(adj, features)
     label = G._cuda(label, torch.float32)
     labels = G.argmax_rows(label)                                   # hm.py:193
@@ -233,8 +234,7 @@ def similarity(features, adj, label, hard=None, LP=1, ifsum=1, idx_train=None):
         label = label[ids].contiguous()                             # hm.py:197
     m = int(z.shape[0])
     c = int(labels.max().item()) + 1
-    gm = G.gram(z)                                                  # hm.py:192 / 199-200
-    w = G.class_colsum(gm, labels, c, is_mean=(ifsum != 1))         # hm.py:201-206
+    w = G.las_weights(z, labels, c, is_mean=(ifsum != 1))           # hm.py:192 / 199-206
     if label.shape[1] != c:
         if LP != 1:
             raise RuntimeError(f"The size of tensor a ({c}) must match the size of tensor b ({label.shape[1]})")

@@ -158,13 +158,15 @@ def similarity(features, adj, label, NTK=None, hard=None, LP=1, ifsum=1, idx_tra
         z = G.spmm(g, features)
         if ids is not None:
             z = G.gather_rows(z, ids)
-        gm = G.gram(z)                                                          # hp.py:196
     if ids is not None:
         labels = labels[ids].contiguous()
         label = label[ids].contiguous()
-    m = int(gm.shape[0])
+    m = int((gm if NTK else z).shape[0])
     c = int(labels.max().item()) + 1
-    w = G.class_colsum(gm, labels, c, is_mean=(ifsum != 1))
+    if NTK:
+        w = G.class_colsum(gm, labels, c, is_mean=(ifsum != 1))
+    else:
+        w = G.las_weights(z, labels, c, is_mean=(ifsum != 1))                  # hp.py:196-206
     if label.shape[1] != c:
         if LP != 1:
             raise RuntimeError(f"The size of tensor a ({c}) must match the size of tensor b ({label.shape[1]})")
