@@ -127,9 +127,11 @@ int wdgh_spmm_csr(const int64_t *rowptr, const int32_t *col, const float *val, i
                   int64_t *plan_i64, const int64_t *plan_host, float *partial,
                   int64_t row_offset, void *stream);
 
-/* Element types of wdgh_spmm_csr_bf16's and wdgh_pipeline_host_bf16's output */
+/* Element types of the output of wdgh_spmm_csr_bf16 / _f16 and wdgh_pipeline_host_bf16 / _f16: float32, or the half
+ * type of the features (a bf16 entry rejects WDGH_DTYPE_F16, an f16 entry WDGH_DTYPE_BF16) */
 #define WDGH_DTYPE_F32  0
 #define WDGH_DTYPE_BF16 1
+#define WDGH_DTYPE_F16  2
 /* wdgh_spmm_csr with a bfloat16 feature matrix (raw bf16 bits), fp32 accumulation, y float32 or bf16 (y_dtype).
  * ldx / ldy in elements; plan, dinv, deg_code, partial (float32) exactly as for wdgh_spmm_csr.
  * Every row is summed in the order of wdgh_spmm_csr, and bf16 -> fp32 is exact: fp32 output is bit-identical to
@@ -140,6 +142,16 @@ int wdgh_spmm_csr_bf16(const int64_t *rowptr, const int32_t *col, const float *v
                        int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
                        int64_t *plan_i64, const int64_t *plan_host, float *partial,
                        int64_t row_offset, void *stream);
+/* wdgh_spmm_csr with a float16 feature matrix (raw IEEE binary16 bits), fp32 accumulation, y float32 or float16
+ * (y_dtype WDGH_DTYPE_F32 / WDGH_DTYPE_F16).  Every row is summed in the order of wdgh_spmm_csr, and fp16 -> fp32 is
+ * exact for every value (subnormals, +-0, +-inf, NaN): fp32 output is bit-identical to wdgh_spmm_csr on the upcast
+ * matrix, fp16 output is that result rounded to nearest even (overflow to +-inf).  Alignment rules as for
+ * wdgh_spmm_csr_bf16. */
+int wdgh_spmm_csr_f16(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                      const uint16_t *x, int64_t d, int64_t ldx, void *y, int64_t ldy, int y_dtype,
+                      int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                      int64_t *plan_i64, const int64_t *plan_host, float *partial,
+                      int64_t row_offset, void *stream);
 
 /* ---- phased aggregation (overlap of the feature all-gather with compute, N > 1) ---- */
 /* seg[b][r] (int64[num_bounds][n]) = first stored entry of row r whose column id is >= bounds_dev[b]; with
@@ -185,6 +197,16 @@ int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *range_begin,
                               const uint8_t *skip_rows, int accumulate, int finalize, int run_split_rows,
                               int64_t *plan_i64, const int64_t *plan_host, float *partial,
                               int64_t row_offset, void *stream);
+/* wdgh_spmm_csr_ranged with a float16 feature matrix (raw binary16 bits, ldx in elements) and float32 y: fp32 partial
+ * sums, so each call is bit-identical to wdgh_spmm_csr_ranged on the upcast matrix with the same arguments.  No extra
+ * partial sums and no ctas_per_sm; alignment and widths as for wdgh_spmm_csr_ranged_bf16. */
+int wdgh_spmm_csr_ranged_f16(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                             const int32_t *col, const float *val, int64_t n,
+                             const uint16_t *x, int64_t d, int64_t ldx, float *y, int64_t ldy,
+                             int norm, int add_self_loop, const float *dinv, const uint8_t *deg_code,
+                             const uint8_t *skip_rows, int accumulate, int finalize, int run_split_rows,
+                             int64_t *plan_i64, const int64_t *plan_host, float *partial,
+                             int64_t row_offset, void *stream);
 
 /* ---- label metrics: one pass over the edges ------------------------------ */
 /* Integer statistics every label metric of homophily_metrics.py is a ratio of
@@ -334,7 +356,15 @@ int wdgh_pipeline_host_bf16(const int64_t *rowptr_host, const int32_t *col_host,
                             const uint16_t *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
                             int norm, int add_self_loop,
                             void *y_host, int y_dtype, int64_t *counters_host, double *node_sum_host);
-/* free the buffers cached by wdgh_pipeline_host / wdgh_pipeline_host_bf16 */
+/* wdgh_pipeline_host with a float16 feature matrix (raw binary16 bits, [n][d] contiguous): half the bytes of X on the
+ * link.  y_host (NULL = counters only) is [n][d] of y_dtype: WDGH_DTYPE_F32, or WDGH_DTYPE_F16 (the fp32 Y of the same
+ * call rounded to nearest even, overflow to +-inf).  Same schedule, cache and ordering as wdgh_pipeline_host_bf16: an
+ * fp32 Y is bit-identical to wdgh_pipeline_host on the upcast matrix.  SYNCHRONOUS. */
+int wdgh_pipeline_host_f16(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                           const uint16_t *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
+                           int norm, int add_self_loop,
+                           void *y_host, int y_dtype, int64_t *counters_host, double *node_sum_host);
+/* free the buffers cached by wdgh_pipeline_host / _bf16 / _f16 */
 int wdgh_pipeline_host_release(void);
 
 #ifdef __cplusplus

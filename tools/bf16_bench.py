@@ -1,20 +1,23 @@
 #!/usr/bin/env python
-"""bf16 features against fp32 features on the headline graph (BASELINE.json configs[4], bench.gen_rows):
+"""bf16 and fp16 features against fp32 features on the headline graph (BASELINE.json configs[4], bench.gen_rows):
 50M nodes, ~976M stored entries, d = 128, 10 classes, Y = D^-1/2 (A+I) D^-1/2 X with the degree scale on the fly.
 
-    python tools/bf16_bench.py [--reps 10] [--warmup 3] [--out profiles/bf16_r03.json]
+    python tools/bf16_bench.py [--reps 10] [--warmup 3] [--out profiles/f16_r06.json]
 
-X is drawn in fp32 by the generator and cast to bf16 once; the fp32 arm reads Xb.float(), so every arm aggregates the
-same values.  Timed in one process with CUDA events, the arms alternating within every repetition:
+X is drawn in fp32 by the generator and cast to bf16 and to fp16 once; the fp32 arm reads Xb.float().  Timed in one
+process with CUDA events, the arms alternating within every repetition:
     spmm_f32         fp32 X -> fp32 Y                          (wdgh_spmm_csr)
     spmm_bf16_f32    bf16 X -> fp32 Y                          (wdgh_spmm_csr_bf16)
     spmm_bf16_bf16   bf16 X -> bf16 Y
+    spmm_f16_f32     fp16 X -> fp32 Y                          (wdgh_spmm_csr_f16)
+    spmm_f16_f16     fp16 X -> fp16 Y
     step_bf16        degree scale + bf16 -> fp32 SpMM + label pass (the step bench.py times, with bf16 features)
     step_f32         the same step with fp32 features: bench.py's step (its spmm_structure_fused is wdgh_spmm_csr followed
                      by wdgh_structure_counts on one stream, the two launches made here; it has no bf16 form)
 Per arm: median ms, GEdges/s (stored entries / time) and the algorithmic-bytes roofline fraction (bytes below, peak as
-bench.py takes it).  On the full graph, Y of the bf16 arms must be torch.equal to the fp32 arm's Y (fp32 output) and
-to its rounding to bf16 (bf16 output).  Prints one JSON line and writes it to --out.
+bench.py takes it).  After the timing, on the full graph: Y of the bf16 arms must be torch.equal to the fp32 call on
+Xb.float() (fp32 output) and to its rounding to bf16 (bf16 output), Y of the fp16 arms likewise to the fp32 call on
+Xh.float() and its rounding to fp16.  Prints one JSON line and writes it to --out.
 """
 import argparse
 import json
@@ -83,7 +86,7 @@ def main():
     ap.add_argument("--homophily", type=float, default=0.3)
     ap.add_argument("--reps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "bf16_r03.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "f16_r06.json"))
     args = ap.parse_args()
 
     import wdgh_b200 as W
@@ -94,6 +97,7 @@ def main():
     n, d, C = args.nodes, args.dim, args.classes
     rowptr, col, x, labels = bench.gen_rows(0, n, n, args.avg_degree, C, args.homophily, d, device)
     xb = x.to(torch.bfloat16)
+    xh = x.to(torch.float16)
     del x
     x32 = xb.float()
     torch.cuda.empty_cache()
@@ -101,10 +105,13 @@ def main():
     g = G.CSRGraph(rowptr, col, None, n)
     _ = g.plan
     dinv, _, code = g.degree_scale(W.NORM_SYM, True)
+    # one fp32 and one 2-byte output buffer serve every half arm (the checks re-run each arm after the timing), so that
+    # the five matrices of the full graph fit next to the three feature matrices
     y32 = torch.empty((n, d), dtype=torch.float32, device=device)
-    yb32 = torch.empty((n, d), dtype=torch.float32, device=device)
+    yh32 = torch.empty((n, d), dtype=torch.float32, device=device)
     ybb = torch.empty((n, d), dtype=torch.bfloat16, device=device)
-    ystep = torch.empty((n, d), dtype=torch.float32, device=device)
+    yhh = ybb.view(torch.float16)
+    ystep = yh32
     scratch = [None]
 
     def step(xx):
@@ -115,8 +122,10 @@ def main():
 
     arms = {
         "spmm_f32": lambda: G.spmm(g, x32, W.NORM_SYM, True, out=y32, dinv=dinv, deg_code=code),
-        "spmm_bf16_f32": lambda: G.spmm(g, xb, W.NORM_SYM, True, out=yb32, dinv=dinv, deg_code=code),
+        "spmm_bf16_f32": lambda: G.spmm(g, xb, W.NORM_SYM, True, out=yh32, dinv=dinv, deg_code=code),
         "spmm_bf16_bf16": lambda: G.spmm(g, xb, W.NORM_SYM, True, out=ybb, dinv=dinv, deg_code=code),
+        "spmm_f16_f32": lambda: G.spmm(g, xh, W.NORM_SYM, True, out=yh32, dinv=dinv, deg_code=code),
+        "spmm_f16_f16": lambda: G.spmm(g, xh, W.NORM_SYM, True, out=yhh, dinv=dinv, deg_code=code),
         "step_bf16": lambda: step(xb),
         "step_f32": lambda: step(x32),
     }
@@ -133,13 +142,24 @@ def main():
             ev[k][r][1].record()
     torch.cuda.synchronize()
 
-    # the last timed launch of every SpMM arm left its Y behind
-    eq_f32 = equal_rows(yb32, y32)
-    eq_bf16 = equal_rows(ybb, y32, to=torch.bfloat16)
+    # every half arm once more against the fp32 call on the same values: bf16 first, then fp16 (x32 <- Xh.float())
+    def check(arm16_f32, arm16_16, y16, dtype):
+        arms["spmm_f32"]()
+        arms[arm16_f32]()
+        eq32 = equal_rows(yh32, y32)
+        arms[arm16_16]()
+        torch.cuda.synchronize()
+        return eq32, equal_rows(y16, y32, to=dtype)
+
+    eq_f32, eq_bf16 = check("spmm_bf16_f32", "spmm_bf16_bf16", ybb, torch.bfloat16)
+    for r in range(0, n, 1 << 22):
+        x32[r:r + (1 << 22)].copy_(xh[r:r + (1 << 22)])
+    eq_f16_f32, eq_f16 = check("spmm_f16_f32", "spmm_f16_f16", yhh, torch.float16)
 
     peak, peak_src = hbm_peak()
     alg = {"spmm_f32": spmm_bytes(nnz, n, d, 4, 4), "spmm_bf16_f32": spmm_bytes(nnz, n, d, 2, 4),
-           "spmm_bf16_bf16": spmm_bytes(nnz, n, d, 2, 2)}
+           "spmm_bf16_bf16": spmm_bytes(nnz, n, d, 2, 2), "spmm_f16_f32": spmm_bytes(nnz, n, d, 2, 4),
+           "spmm_f16_f16": spmm_bytes(nnz, n, d, 2, 2)}
     alg["step_bf16"] = alg["spmm_bf16_f32"] + label_bytes(nnz, n)
     alg["step_f32"] = alg["spmm_f32"] + label_bytes(nnz, n)
     res = {}
@@ -153,8 +173,12 @@ def main():
             "norm": "sym D^-1/2 (A+I) D^-1/2 on the fly", "reps": args.reps, "warmup": args.warmup,
             "arms": res, "speedup_spmm_bf16_f32": res["spmm_f32"]["ms"] / res["spmm_bf16_f32"]["ms"],
             "speedup_spmm_bf16_bf16": res["spmm_f32"]["ms"] / res["spmm_bf16_bf16"]["ms"],
+            "speedup_spmm_f16_f32": res["spmm_f32"]["ms"] / res["spmm_f16_f32"]["ms"],
+            "speedup_spmm_f16_f16": res["spmm_f32"]["ms"] / res["spmm_f16_f16"]["ms"],
+            "f16_f32_over_bf16_f32": res["spmm_f16_f32"]["ms"] / res["spmm_bf16_f32"]["ms"],
             "speedup_step": res["step_f32"]["ms"] / res["step_bf16"]["ms"],
             "equal_bf16_f32_vs_f32": eq_f32, "equal_bf16_bf16_vs_f32_rounded": eq_bf16,
+            "equal_f16_f32_vs_f32": eq_f16_f32, "equal_f16_f16_vs_f32_rounded": eq_f16,
             "peak_gbs": peak, "peak_source": peak_src, "card": card(device)}
     text = json.dumps(line)
     print(text, flush=True)
@@ -162,7 +186,7 @@ def main():
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
             f.write(text + "\n")
-    if not (eq_f32 and eq_bf16):
+    if not (eq_f32 and eq_bf16 and eq_f16_f32 and eq_f16):
         sys.exit(3)
 
 

@@ -1,22 +1,26 @@
 #!/usr/bin/env python
-"""Host-buffer pipeline (the e2e path) with bf16 features against fp32 features on the headline graph (BASELINE.json
-configs[4], bench.gen_rows): 50M nodes, ~976M stored entries, d = 128, 10 classes, Y = D^-1/2 (A+I) D^-1/2 X.
+"""Host-buffer pipeline (the e2e path) with bf16 and fp16 features against fp32 features on the headline graph
+(BASELINE.json configs[4], bench.gen_rows): 50M nodes, ~976M stored entries, d = 128, 10 classes,
+Y = D^-1/2 (A+I) D^-1/2 X.
 
-    python tools/e2e_bf16_bench.py [--reps 5] [--warmup 1] [--out profiles/e2e_bf16_r04.json]
+    python tools/e2e_bf16_bench.py [--reps 5] [--warmup 1] [--out profiles/e2e_f16_r06.json]
 
-X is drawn in fp32 by the generator and cast to bf16 once; the fp32 arms read Xb.float(), so every arm moves the same
-values.  All inputs and outputs live in pinned host memory (about 80 GB at full size).  Timed in one process with a host
-clock around the synchronous call, the arms alternating within every repetition:
+X is drawn in fp32 by the generator and cast to bf16 and to fp16 once; the fp32 arms read Xb.float().  All inputs and
+outputs live in pinned host memory (about 95 GB at full size; the bf16 and fp16 Y share one buffer).  Timed in one
+process with a host clock around the synchronous call, the arms alternating within every repetition:
     e2e_f32          wdgh_pipeline_host, fp32 X, fp32 Y back          (what bench.py's e2e times)
     e2e_bf16_f32y    wdgh_pipeline_host_bf16, bf16 X, fp32 Y back
     e2e_bf16_bf16y   wdgh_pipeline_host_bf16, bf16 X, bf16 Y back
+    e2e_f16_f32y     wdgh_pipeline_host_f16, fp16 X, fp32 Y back
+    e2e_f16_f16y     wdgh_pipeline_host_f16, fp16 X, fp16 Y back
     counters_f32     wdgh_pipeline_host, fp32 X, counters only (y_host = NULL)
     counters_bf16    wdgh_pipeline_host_bf16, bf16 X, counters only
+    counters_f16     wdgh_pipeline_host_f16, fp16 X, counters only
 Per arm: median ms and spread, GEdges/s, H2D / D2H bytes and the effective link rate ((H2D + D2H) / time).
-Checks in the same run: the counters of every arm are identical; on a seeded sample of rows, the fp32 Y of the bf16
-features equals the fp32 Y of e2e_f32 exactly (both feature types take the same copy / compute form, whose phases are
-bit-identical), and the bf16 Y equals the fp32 Y of the bf16 features rounded to nearest even.  Prints one JSON line,
-writes it to --out and exits non-zero when a check fails.
+Checks in the same run: the counters of every arm are identical; on a seeded sample of rows, the fp32 Y of the half
+features equals the fp32 Y of e2e_f32 on the same values (Xb.float(), then Xh.float()) exactly (every feature type
+takes the same copy / compute form, whose phases are bit-identical), and the half Y equals the fp32 Y of the same
+features rounded to nearest even.  Prints one JSON line, writes it to --out and exits non-zero when a check fails.
 """
 import argparse
 import json
@@ -53,7 +57,7 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--sample-rows", type=int, default=1 << 20)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "e2e_bf16_r04.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "e2e_f16_r06.json"))
     args = ap.parse_args()
 
     import wdgh_b200 as W
@@ -65,6 +69,7 @@ def main():
     rowptr, col, x, labels = bench.gen_rows(0, n, n, args.avg_degree, C, args.homophily, d, device)
     nnz = int(col.shape[0])
     xb = x.to(torch.bfloat16)
+    xh = x.to(torch.float16)
     del x
 
     def pinned(t, dtype=None):
@@ -76,15 +81,16 @@ def main():
     try:
         rowptr_h, col_h = pinned(rowptr), pinned(col)
         lab_h = pinned(labels, torch.int32)
-        xb_h, x32_h = pinned(xb), pinned(xb, torch.float32)
+        xb_h, xh_h, x32_h = pinned(xb), pinned(xh), pinned(xb, torch.float32)
         y32_h = torch.empty((n, d), dtype=torch.float32, pin_memory=True)
         ybf_h = torch.empty((n, d), dtype=torch.bfloat16, pin_memory=True)
+        yh_h = ybf_h.view(torch.float16)
     except RuntimeError as e:
         print(json.dumps({"tool": "tools/e2e_bf16_bench.py", "nodes": n,
                           "error": f"pinning the host buffers failed ({str(e)[:120]}); run again with a smaller --nodes"}),
               flush=True)
         sys.exit(2)
-    del rowptr, col, labels, xb
+    del rowptr, col, labels, xb, xh
     torch.cuda.empty_cache()
 
     n_cnt = W._lib.sc_words(C)
@@ -99,8 +105,11 @@ def main():
         "e2e_f32": (x32_h, y32_h),
         "e2e_bf16_f32y": (xb_h, y32_h),
         "e2e_bf16_bf16y": (xb_h, ybf_h),
+        "e2e_f16_f32y": (xh_h, y32_h),
+        "e2e_f16_f16y": (xh_h, yh_h),
         "counters_f32": (x32_h, None),
         "counters_bf16": (xb_h, None),
+        "counters_f16": (xh_h, None),
     }
     for _ in range(args.warmup):
         for k, (xh, yh) in arms.items():
@@ -117,20 +126,29 @@ def main():
     counters_equal = all((c == ref_c).all() and (s == ref_s).all() for c, s in counters.values())
     gen = torch.Generator().manual_seed(7)
     rows = torch.randint(0, n, (min(args.sample_rows, n),), generator=gen)
-    run("e2e_f32", x32_h, y32_h)
-    y_f32 = y32_h[rows].clone()
-    run("e2e_bf16_f32y", xb_h, y32_h)
-    y_bf = y32_h[rows].clone()
-    run("e2e_bf16_bf16y", xb_h, ybf_h)
-    y_bfbf = ybf_h[rows].clone()
-    scale = y_f32.abs().max().item()
-    err = (y_bf - y_f32).abs().max().item()
-    y_ok = torch.equal(y_bf, y_f32)
-    bf16_ok = torch.equal(y_bfbf, y_bf.to(torch.bfloat16))
+
+    def check(arm_f32y, arm_halfy, x_h, y_half_h):
+        """(max abs error and equality of the half features' fp32 Y against e2e_f32 on x32_h, the half Y is its
+        rounding, max |Y|) on the sample rows"""
+        run("e2e_f32", x32_h, y32_h)
+        y_f32 = y32_h[rows].clone()
+        run(arm_f32y, x_h, y32_h)
+        y_h32 = y32_h[rows].clone()
+        run(arm_halfy, x_h, y_half_h)
+        y_hh = y_half_h[rows].clone()
+        return ((y_h32 - y_f32).abs().max().item(), torch.equal(y_h32, y_f32),
+                torch.equal(y_hh, y_h32.to(y_half_h.dtype)), y_f32.abs().max().item())
+
+    err, y_ok, bf16_ok, scale = check("e2e_bf16_f32y", "e2e_bf16_bf16y", xb_h, ybf_h)
+    for r in range(0, n, 1 << 22):               # the fp32 arm on the fp16 values
+        x32_h[r:r + (1 << 22)].copy_(xh_h[r:r + (1 << 22)])
+    err16, y16_ok, f16_ok, _ = check("e2e_f16_f32y", "e2e_f16_f16y", xh_h, yh_h)
     W._lib.lib.wdgh_pipeline_host_release()
 
-    x_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 2, "e2e_bf16_bf16y": 2, "counters_f32": 4, "counters_bf16": 2}
-    y_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 4, "e2e_bf16_bf16y": 2, "counters_f32": 0, "counters_bf16": 0}
+    x_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 2, "e2e_bf16_bf16y": 2, "e2e_f16_f32y": 2, "e2e_f16_f16y": 2,
+               "counters_f32": 4, "counters_bf16": 2, "counters_f16": 2}
+    y_bytes = {"e2e_f32": 4, "e2e_bf16_f32y": 4, "e2e_bf16_bf16y": 2, "e2e_f16_f32y": 4, "e2e_f16_f16y": 2,
+               "counters_f32": 0, "counters_bf16": 0, "counters_f16": 0}
     res = {}
     for k, ts in times.items():
         ms = statistics.median(ts) * 1e3
@@ -146,16 +164,21 @@ def main():
             "speedup_e2e_bf16_f32y": res["e2e_f32"]["ms"] / res["e2e_bf16_f32y"]["ms"],
             "speedup_e2e_bf16_bf16y": res["e2e_f32"]["ms"] / res["e2e_bf16_bf16y"]["ms"],
             "speedup_counters_bf16": res["counters_f32"]["ms"] / res["counters_bf16"]["ms"],
+            "speedup_e2e_f16_f32y": res["e2e_f32"]["ms"] / res["e2e_f16_f32y"]["ms"],
+            "speedup_e2e_f16_f16y": res["e2e_f32"]["ms"] / res["e2e_f16_f16y"]["ms"],
+            "speedup_counters_f16": res["counters_f32"]["ms"] / res["counters_f16"]["ms"],
             "check_counters_identical": bool(counters_equal), "check_sample_rows": int(rows.shape[0]),
             "check_y_f32_max_abs_err": err, "check_y_max_abs": scale,
-            "check_y_f32": bool(y_ok), "check_y_bf16_is_rounded_f32": bool(bf16_ok), "card": card(device)}
+            "check_y_f32": bool(y_ok), "check_y_bf16_is_rounded_f32": bool(bf16_ok),
+            "check_y_f16_f32_max_abs_err": err16, "check_y_f16_f32": bool(y16_ok),
+            "check_y_f16_is_rounded_f32": bool(f16_ok), "card": card(device)}
     text = json.dumps(line)
     print(text, flush=True)
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
             f.write(text + "\n")
-    if not (counters_equal and y_ok and bf16_ok):
+    if not (counters_equal and y_ok and bf16_ok and y16_ok and f16_ok):
         sys.exit(3)
 
 

@@ -1,13 +1,30 @@
 // Internal (non-ABI) entry points shared between translation units.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 
 namespace wdgh {
 
 constexpr int kHistSmemBins = 4096;  // C*C bins kept in shared memory per CTA
 
-// y[r][c] = bf16(x[r][c]) rounded to nearest even, r < rows, c < cols (spmm.cu); y holds raw bf16 bits
-int round_to_bf16(const float *x, int64_t rows, int64_t cols, int64_t ldx, void *y, int64_t ldy, cudaStream_t st);
+using bf16 = __nv_bfloat16;
+using f16 = __half;
+
+// The WDGH_DTYPE of the half Y an aggregation with features of type T may write besides fp32: the type of the features
+// itself (fp32 features: fp32 Y only)
+template <typename T>
+constexpr int kHalfY = WDGH_DTYPE_F32;
+template <>
+constexpr int kHalfY<bf16> = WDGH_DTYPE_BF16;
+template <>
+constexpr int kHalfY<f16> = WDGH_DTYPE_F16;
+
+// y[r][c] = x[r][c] rounded to nearest even to H (bf16 or f16; fp16 overflow -> +-inf), r < rows, c < cols (spmm.cu);
+// y holds raw H bits
+template <typename H>
+int round_to_half(const float *x, int64_t rows, int64_t cols, int64_t ldx, void *y, int64_t ldy, cudaStream_t st);
 
 // Folds one warp-wide batch of class-pair keys (key < 0: nothing to count) into the histogram:
 // one atomic per distinct key, multiplicity from __match_any_sync + popc.

@@ -24,14 +24,13 @@
 // chunk's phase separates the end of a block's H2D copy from the start of its D2H copy, and the D2H copy of block k runs
 // under the H2D copy of block k + 1.
 //
-// bfloat16 features (wdgh_pipeline_host_bf16) take the same body with the bf16 aggregation entries: half the bytes of
-// X on the link, fp32 phases (a phase is bit-identical to the fp32 phase on the upcast matrix).  Y is always
-// aggregated in fp32 into the device Y buffer; for a bf16 Y the last phase of a block is followed by a rounding pass
-// into a bf16 staging buffer, which the D2H copy reads -- so a bf16 Y is exactly the rounding of the fp32 Y of the
-// same schedule, and the schedule does not depend on the type of Y.
+// bfloat16 and float16 features (wdgh_pipeline_host_bf16 / _f16) take the same body with their aggregation entries
+// (Elem below): half the bytes of X on the link, fp32 phases (a phase is bit-identical to the fp32 phase on the upcast
+// matrix).  Y is always aggregated in fp32 into the device Y buffer; for a half Y (the type of X) the last phase of a
+// block is followed by a rounding pass into a 2-byte staging buffer, which the D2H copy reads -- so a half Y is exactly
+// the rounding of the fp32 Y of the same schedule, and the schedule depends neither on the type of X nor on that of Y.
 #include <algorithm>
 #include <mutex>
-#include <type_traits>
 
 #include "internal.cuh"
 
@@ -47,7 +46,7 @@ constexpr int kRowChunks = 16;
 // Width (elements) of the column blocks when Y comes back.  64 floats = 256-byte rows: the narrowest pitched copy that
 // still runs at the full PCIe rate in both directions (55.6 / 53.5 GB/s alone, 48 + 50 GB/s both directions at once;
 // 128-byte rows: 34 + 40 GB/s, tools/pcie_probe.cu), and a width the row-group aggregation kernel runs natively.
-// bf16 features take the same 64 columns, i.e. 128-byte rows (the slower pitched copy): measured on the 50M-node /
+// bf16 and fp16 features take the same 64 columns, i.e. 128-byte rows (the slower pitched copy): measured on the 50M-node /
 // 976M-entry graph at d = 128 (tools/e2e_bf16_bench.py, NVIDIA B200, 1000 W power limit, each form in its own process),
 // column blocks 735.7 ms with fp32 Y back and 536.8 ms with bf16 Y back, against 795.1 / 578.3 ms for row blocks (full-rate
 // contiguous H2D, Y copied after the last phase).
@@ -73,7 +72,7 @@ static Schedule schedule(int64_t d, bool y_wanted) {
     while (R > 1 && KC * R > kMaxChunks) R /= 2;
     return {kColWidth, KC, R};
   }
-  // the widths the ranged aggregation entries take (16-byte fp32 / 8-byte bf16 rows, row-group kernel widths)
+  // the widths the ranged aggregation entries take (16-byte fp32 / 8-byte bf16 and fp16 rows, row-group kernel widths)
   if (d % 4 == 0 && (d == 32 || d == 64 || d >= 128)) return {d, 1, kRowChunks};
   return {d, 1, 1};
 }
@@ -81,14 +80,14 @@ static Schedule schedule(int64_t d, bool y_wanted) {
 struct HostPipelineCache {
   int64_t n = -1, nnz = -1, d = -1, cap = -1;
   int C = -1, device = -1;
-  // The feature buffer is sized in bytes and grows when a call needs more (an fp32 call after a bf16 one); a bf16 call
+  // The feature buffer is sized in bytes and grows when a call needs more (an fp32 call after a half one); a half call
   // after an fp32 one reuses it, so a caller alternating feature types does not reallocate the largest buffer.
   size_t x_bytes = 0, ystage_bytes = 0, partial_bytes = 0;
   int64_t *rowptr = nullptr;
   int32_t *col = nullptr;
   void *x = nullptr;
   float *y = nullptr, *dinv = nullptr, *partial = nullptr;
-  void *ystage = nullptr;  // bf16 Y rounded for the D2H copy (allocated by the first bf16-Y call)
+  void *ystage = nullptr;  // half Y (bf16 or fp16) rounded for the D2H copy (allocated by the first half-Y call)
   int32_t *labels = nullptr, *deg = nullptr, *match = nullptr;
   uint8_t *labels8 = nullptr, *deg_code = nullptr;
   int64_t *plan = nullptr, *counters = nullptr;
@@ -114,7 +113,7 @@ static HostPipelineCache g_cache;  // one cached pipeline per process, guarded b
 static std::mutex g_cache_mu;
 constexpr int64_t kHostPipelineThreshold = 512;
 
-// The buffers of the cache that only grow (features, bf16 Y staging, split-row partial sums): reallocates p when it
+// The buffers of the cache that only grow (features, half Y staging, split-row partial sums): reallocates p when it
 // holds fewer than `bytes`.
 template <typename T>
 static cudaError_t grow(T *&p, size_t &cap, size_t bytes) {
@@ -135,15 +134,55 @@ static cudaError_t grow(T *&p, size_t &cap, size_t bytes) {
     }                                                                    \
   } while (0)
 
-// The body of wdgh_pipeline_host (Tin = float) and wdgh_pipeline_host_bf16 (Tin = uint16_t, raw bf16 bits).
-template <typename Tin>
+// What the body needs of a feature type T: the element type of its C-ABI pointers (Bits), and its full aggregation
+// launch and phase entry, both with fp32 Y, in the argument order of the half-type entries.  The half Y it may return
+// is kHalfY<T>, rounded by round_to_half<T>.
+template <typename T>
+struct Elem;
+template <>
+struct Elem<float> {
+  using Bits = float;
+  static int full(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n, const float *x, int64_t d,
+                  int64_t ldx, void *y, int64_t ldy, int /* y_dtype: always WDGH_DTYPE_F32 */, int norm,
+                  int add_self_loop, const float *dinv, const uint8_t *deg_code, int64_t *plan_i64,
+                  const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+    return wdgh_spmm_csr(rowptr, col, val, n, x, d, ldx, static_cast<float *>(y), ldy, norm, add_self_loop, dinv,
+                         deg_code, plan_i64, plan_host, partial, row_offset, stream);
+  }
+  static int phase(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end, const int32_t *col,
+                   const float *val, int64_t n, const float *x, int64_t d, int64_t ldx, float *y, int64_t ldy, int norm,
+                   int add_self_loop, const float *dinv, const uint8_t *deg_code, const uint8_t *skip_rows,
+                   int accumulate, int finalize, int run_split_rows, int64_t *plan_i64, const int64_t *plan_host,
+                   float *partial, int64_t row_offset, void *stream) {
+    return wdgh_spmm_csr_ranged(rowptr, range_begin, range_end, col, val, n, x, d, ldx, y, ldy, norm, add_self_loop,
+                                dinv, deg_code, skip_rows, accumulate, finalize, run_split_rows, nullptr, 0, 0, 0, 0, 0,
+                                plan_i64, plan_host, partial, row_offset, stream);
+  }
+};
+template <>
+struct Elem<bf16> {
+  using Bits = uint16_t;
+  static constexpr auto full = wdgh_spmm_csr_bf16;
+  static constexpr auto phase = wdgh_spmm_csr_ranged_bf16;
+};
+template <>
+struct Elem<f16> {
+  using Bits = uint16_t;
+  static constexpr auto full = wdgh_spmm_csr_f16;
+  static constexpr auto phase = wdgh_spmm_csr_ranged_f16;
+};
+
+// The body of wdgh_pipeline_host (T = float), wdgh_pipeline_host_bf16 and wdgh_pipeline_host_f16.
+template <typename T>
 static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
-                         const Tin *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes, int norm,
-                         int add_self_loop, void *y_host, int y_dtype, int64_t *counters_host, double *node_sum_host) {
-  constexpr bool F32 = std::is_same<Tin, float>::value;
+                         const typename Elem<T>::Bits *x_host, int64_t d, const int32_t *labels_host,
+                         int32_t num_classes, int norm, int add_self_loop, void *y_host, int y_dtype,
+                         int64_t *counters_host, double *node_sum_host) {
+  using E = Elem<T>;
+  using Tin = typename E::Bits;
   WDGH_REQUIRE_AT(rowptr_host && x_host && labels_host && counters_host && node_sum_host, "null pointer");
   WDGH_REQUIRE_AT(n > 0 && nnz >= 0 && d > 0 && num_classes >= 1 && (col_host || nnz == 0), "bad shape");
-  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == WDGH_DTYPE_BF16, "bad y_dtype");
+  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == kHalfY<T>, "bad y_dtype (float32, or the type of x)");
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached buffers and streams serve one call at a time
   HostPipelineCache &c = g_cache;
   const int C = num_classes;
@@ -177,7 +216,7 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
     c.n = n; c.nnz = nnz; c.d = d; c.C = C; c.cap = cap; c.device = device;
   }
   WDGH_CUDA(grow(c.x, c.x_bytes, (size_t)(n * d) * sizeof(Tin)));
-  const bool y16 = y_host && y_dtype == WDGH_DTYPE_BF16;
+  const bool y16 = y_host && y_dtype != WDGH_DTYPE_F32;
   if (y16) WDGH_CUDA(grow(c.ystage, c.ystage_bytes, (size_t)(n * d) * 2));
   const size_t ysz = y16 ? 2 : sizeof(float);  // bytes of one element of Y on the host
   Tin *x = static_cast<Tin *>(c.x);
@@ -227,30 +266,21 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
   const uint8_t *code = norm != WDGH_NORM_NONE ? c.deg_code : nullptr;
   // one launch over every row of a column slab of width w (fp32 Y)
   auto full = [&](const Tin *xb, int64_t w, float *yb) -> int {
-    if constexpr (F32)
-      return wdgh_spmm_csr(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv, code, c.plan,
-                           plan_host, c.partial, 0, st);
-    else
-      return wdgh_spmm_csr_bf16(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, WDGH_DTYPE_F32, norm, add_self_loop, dinv,
-                                code, c.plan, plan_host, c.partial, 0, st);
+    return E::full(c.rowptr, c.col, nullptr, n, xb, w, d, yb, d, WDGH_DTYPE_F32, norm, add_self_loop, dinv, code, c.plan,
+                   plan_host, c.partial, 0, st);
   };
   // the phase of row chunk k: y (+)= the entries whose column lies in chunk k; the last phase finalizes
   auto phase = [&](int k, const Tin *xb, int64_t w, float *yb, int accumulate, int last) -> int {
     const int64_t *b = c.seg + (size_t)k * n, *e = c.seg + (size_t)(k + 1) * n;
-    if constexpr (F32)
-      return wdgh_spmm_csr_ranged(c.rowptr, b, e, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv, code,
-                                  c.skip, accumulate, last, last, nullptr, 0, 0, 0, 0, 0, c.plan, plan_host, c.partial,
-                                  0, st);
-    else
-      return wdgh_spmm_csr_ranged_bf16(c.rowptr, b, e, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv,
-                                       code, c.skip, accumulate, last, last, c.plan, plan_host, c.partial, 0, st);
+    return E::phase(c.rowptr, b, e, c.col, nullptr, n, xb, w, d, yb, d, norm, add_self_loop, dinv, code, c.skip,
+                    accumulate, last, last, c.plan, plan_host, c.partial, 0, st);
   };
   // 3. label pass: needs only the graph and the labels, runs under the feature copy
   rc = wdgh_structure_counts(c.rowptr, c.col, n, nnz, c.labels, C, c.plan, plan_host, c.counters, c.node_sum, c.deg,
                              c.match, c.labels8, n, 0, st);
   if (rc) return rc;
   // 4. per column block: one aggregation phase per arriving row chunk (R = 1: one full launch); the Y block leaves on
-  //    the third stream as soon as its last phase (and, for a bf16 Y, its rounding) is done
+  //    the third stream as soon as its last phase (and, for a half Y, its rounding) is done
   if (R > 1) {
     WDGH_CUDA(cudaMemcpyAsync(c.bounds, bounds_h, (R + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     rc = wdgh_column_segments(c.rowptr, c.col, n, c.bounds, R + 1, c.seg, st);
@@ -267,9 +297,11 @@ static int pipeline_host(const char *fn, const int64_t *rowptr_host, const int32
       if (rc) return rc;
     }
     if (!y_host) continue;
-    if (y16) {
-      rc = round_to_bf16(yb, n, W, d, static_cast<uint16_t *>(c.ystage) + kc * W, d, st);
-      if (rc) return rc;
+    if constexpr (kHalfY<T> != WDGH_DTYPE_F32) {
+      if (y16) {
+        rc = round_to_half<T>(yb, n, W, d, static_cast<uint16_t *>(c.ystage) + kc * W, d, st);
+        if (rc) return rc;
+      }
     }
     WDGH_CUDA(cudaEventRecord(c.ev_y[kc], st));
     WDGH_CUDA(cudaStreamWaitEvent(sb, c.ev_y[kc], 0));
@@ -307,7 +339,7 @@ extern "C" int wdgh_pipeline_host(const int64_t *rowptr_host, const int32_t *col
                                   const float *x_host, int64_t d, const int32_t *labels_host, int32_t num_classes,
                                   int norm, int add_self_loop, float *y_host, int64_t *counters_host,
                                   double *node_sum_host) {
-  return pipeline_host("wdgh_pipeline_host", rowptr_host, col_host, n, nnz, x_host, d, labels_host, num_classes, norm,
+  return pipeline_host<float>("wdgh_pipeline_host", rowptr_host, col_host, n, nnz, x_host, d, labels_host, num_classes, norm,
                        add_self_loop, y_host, WDGH_DTYPE_F32, counters_host, node_sum_host);
 }
 
@@ -315,6 +347,14 @@ extern "C" int wdgh_pipeline_host_bf16(const int64_t *rowptr_host, const int32_t
                                        const uint16_t *x_host, int64_t d, const int32_t *labels_host,
                                        int32_t num_classes, int norm, int add_self_loop, void *y_host, int y_dtype,
                                        int64_t *counters_host, double *node_sum_host) {
-  return pipeline_host("wdgh_pipeline_host_bf16", rowptr_host, col_host, n, nnz, x_host, d, labels_host, num_classes,
-                       norm, add_self_loop, y_host, y_dtype, counters_host, node_sum_host);
+  return pipeline_host<bf16>("wdgh_pipeline_host_bf16", rowptr_host, col_host, n, nnz, x_host, d, labels_host,
+                             num_classes, norm, add_self_loop, y_host, y_dtype, counters_host, node_sum_host);
+}
+
+extern "C" int wdgh_pipeline_host_f16(const int64_t *rowptr_host, const int32_t *col_host, int64_t n, int64_t nnz,
+                                      const uint16_t *x_host, int64_t d, const int32_t *labels_host,
+                                      int32_t num_classes, int norm, int add_self_loop, void *y_host, int y_dtype,
+                                      int64_t *counters_host, double *node_sum_host) {
+  return pipeline_host<f16>("wdgh_pipeline_host_f16", rowptr_host, col_host, n, nnz, x_host, d, labels_host,
+                            num_classes, norm, add_self_loop, y_host, y_dtype, counters_host, node_sum_host);
 }

@@ -26,7 +26,13 @@
 // with fp32 output is bit-identical to the fp32 launch on x.float(), and with bf16 output (round to nearest even) to
 // that result .to(bfloat16).  The fp32 instances are unchanged.  The phased form (wdgh_spmm_csr_ranged_bf16) takes bf16
 // features with fp32 output only: its partial sums stay fp32, so a phase is bit-identical to the fp32 phase on x.float().
+//
+// float16 features (wdgh_spmm_csr_f16, wdgh_spmm_csr_ranged_f16): the same instances with Tin = __half.  fp16 -> fp32 is
+// exact for every value (subnormals, +-0, +-inf and NaN included; one HADD2.F32 per element), the order is the one
+// above, so fp32 output is bit-identical to the fp32 launch on x.float() and fp16 output (round to nearest even,
+// overflow to +-inf) to that result .to(float16).  A half Y has the type of X: no fp16 -> bf16 or bf16 -> fp16 launch.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <limits.h>
 #include <stdlib.h>
 
@@ -36,8 +42,6 @@
 
 namespace wdgh {
 
-using bf16 = __nv_bfloat16;
-
 // bf16 -> fp32 is exact: the bf16 bits are the upper half of the float
 __device__ __forceinline__ float bf16_lo(unsigned u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16_hi(unsigned u) { return __uint_as_float(u & 0xffff0000u); }
@@ -45,11 +49,36 @@ __device__ __forceinline__ unsigned bf16x2_rn(float a, float b) {  // round to n
   const __nv_bfloat162 h = __float22bfloat162_rn(make_float2(a, b));
   return *reinterpret_cast<const unsigned *>(&h);
 }
+
+// The 16-bit feature types: a packed pair (low half first) or one value widened to fp32 exactly, a pair or one value
+// rounded to nearest even
+template <typename H>
+struct Half;
+template <>
+struct Half<bf16> {
+  static __device__ __forceinline__ float2 widen2(unsigned u) { return make_float2(bf16_lo(u), bf16_hi(u)); }
+  static __device__ __forceinline__ float widen1(unsigned short u) { return bf16_lo(u); }
+  static __device__ __forceinline__ unsigned round2(float a, float b) { return bf16x2_rn(a, b); }
+  static __device__ __forceinline__ bf16 round1(float v) { return __float2bfloat16_rn(v); }
+};
+template <>
+struct Half<f16> {  // overflow rounds to +-inf, as Tensor.to(torch.float16) does
+  static __device__ __forceinline__ float2 widen2(unsigned u) { return __half22float2(*reinterpret_cast<const __half2 *>(&u)); }
+  static __device__ __forceinline__ float widen1(unsigned short u) { return __half2float(__ushort_as_half(u)); }
+  static __device__ __forceinline__ unsigned round2(float a, float b) {
+    const __half2 h = __float22half2_rn(make_float2(a, b));
+    return *reinterpret_cast<const unsigned *>(&h);
+  }
+  static __device__ __forceinline__ f16 round1(float v) { return __float2half_rn(v); }
+};
+
 // scalar element access of the split-row finish
 __device__ __forceinline__ float load1(const float *p) { return __ldg(p); }
 __device__ __forceinline__ float load1(const bf16 *p) { return __bfloat162float(__ldg(p)); }
+__device__ __forceinline__ float load1(const f16 *p) { return __half2float(__ldg(p)); }
 __device__ __forceinline__ void store1(float *p, float v) { *p = v; }
-__device__ __forceinline__ void store1(bf16 *p, float v) { *p = __float2bfloat16_rn(v); }
+template <typename H>
+__device__ __forceinline__ void store1(H *p, float v) { *p = Half<H>::round1(v); }
 
 template <int VEC>
 struct Vec;
@@ -71,13 +100,17 @@ struct Vec<4> {
   __device__ __forceinline__ void scale(float s) { v.x *= s; v.y *= s; v.z *= s; v.w *= s; }
   __device__ __forceinline__ void store_stream(float *p) const { st_cs(reinterpret_cast<float4 *>(p), v); }
   __device__ __forceinline__ void store(float *p) const { *reinterpret_cast<float4 *>(p) = v; }
-  __device__ __forceinline__ void load(const bf16 *p) {  // 8 bytes
+  template <typename H>
+  __device__ __forceinline__ void load(const H *p) {  // 8 bytes
     unsigned a, b;
     asm("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];" : "=r"(a), "=r"(b) : "l"(p));
-    v = make_float4(bf16_lo(a), bf16_hi(a), bf16_lo(b), bf16_hi(b));
+    const float2 lo = Half<H>::widen2(a), hi = Half<H>::widen2(b);
+    v = make_float4(lo.x, lo.y, hi.x, hi.y);
   }
-  __device__ __forceinline__ void store_stream(bf16 *p) const {
-    asm volatile("st.global.cs.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(bf16x2_rn(v.x, v.y)), "r"(bf16x2_rn(v.z, v.w))
+  template <typename H>
+  __device__ __forceinline__ void store_stream(H *p) const {
+    asm volatile("st.global.cs.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(Half<H>::round2(v.x, v.y)),
+                 "r"(Half<H>::round2(v.z, v.w))
                  : "memory");
   }
 };
@@ -99,13 +132,15 @@ struct Vec<2> {
     asm volatile("st.global.cs.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(v.x), "f"(v.y) : "memory");
   }
   __device__ __forceinline__ void store(float *p) const { *reinterpret_cast<float2 *>(p) = v; }
-  __device__ __forceinline__ void load(const bf16 *p) {  // 4 bytes
+  template <typename H>
+  __device__ __forceinline__ void load(const H *p) {  // 4 bytes
     unsigned a;
     asm("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(a) : "l"(p));
-    v = make_float2(bf16_lo(a), bf16_hi(a));
+    v = Half<H>::widen2(a);
   }
-  __device__ __forceinline__ void store_stream(bf16 *p) const {
-    asm volatile("st.global.cs.u32 [%0], %1;" ::"l"(p), "r"(bf16x2_rn(v.x, v.y)) : "memory");
+  template <typename H>
+  __device__ __forceinline__ void store_stream(H *p) const {
+    asm volatile("st.global.cs.u32 [%0], %1;" ::"l"(p), "r"(Half<H>::round2(v.x, v.y)) : "memory");
   }
 };
 template <>
@@ -119,12 +154,14 @@ struct Vec<1> {
   __device__ __forceinline__ void scale(float s) { v *= s; }
   __device__ __forceinline__ void store_stream(float *p) const { __stcs(p, v); }
   __device__ __forceinline__ void store(float *p) const { *p = v; }
-  __device__ __forceinline__ void load(const bf16 *p) {  // 2 bytes
+  template <typename H>
+  __device__ __forceinline__ void load(const H *p) {  // 2 bytes
     unsigned short a;
     asm("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(a) : "l"(p));
-    v = bf16_lo(a);
+    v = Half<H>::widen1(a);
   }
-  __device__ __forceinline__ void store_stream(bf16 *p) const { __stcs(p, __float2bfloat16_rn(v)); }
+  template <typename H>
+  __device__ __forceinline__ void store_stream(H *p) const { __stcs(p, Half<H>::round1(v)); }
 };
 
 // Accumulate entries [s, e) of one row into acc[NCH].  All G lanes of the group call this together.
@@ -590,10 +627,10 @@ struct SpmmArgs {
   const int32_t *col;
   const float *val;
   int64_t n;
-  const void *x;  // float or bf16 (the Tin of the launch)
+  const void *x;  // float, bf16 or f16 (the Tin of the launch)
   int d;
   int64_t ldx;
-  void *y;        // float or bf16 (Tout)
+  void *y;        // float, or Tin when it is a half type (Tout)
   int64_t ldy;
   int norm, self_loop;
   const float *dinv;
@@ -715,7 +752,7 @@ static int dispatch(const SpmmArgs &a, bool vec4) {
   return launch_heavy<1, 4, HAS_VAL, Tin, Tout>(a, none);
 }
 
-// every row of x / y starts on a 4-element boundary (16 bytes for fp32, 8 for bf16)
+// every row of x / y starts on a 4-element boundary (16 bytes for fp32, 8 for bf16 / f16)
 template <typename Tin, typename Tout>
 static bool rows_vec4(const Tin *x, int64_t d, int64_t ldx, const Tout *y, int64_t ldy, const float *partial) {
   return (d % 4 == 0) && (ldx % 4 == 0) && (ldy % 4 == 0) && (reinterpret_cast<uintptr_t>(x) % (4 * sizeof(Tin)) == 0) &&
@@ -728,8 +765,8 @@ static bool rows_vec4(const Tin *x, int64_t d, int64_t ldx, const Tout *y, int64
 using namespace wdgh;
 
 namespace wdgh {
-// argument checks and dispatch shared by wdgh_spmm_csr (Tin = float) and wdgh_spmm_csr_bf16; `fn` names the entry in
-// the error messages
+// argument checks and dispatch shared by wdgh_spmm_csr (Tin = float), wdgh_spmm_csr_bf16 and wdgh_spmm_csr_f16; `fn`
+// names the entry in the error messages
 #define WDGH_REQUIRE_AT(cond, what)                                      \
   do {                                                                   \
     if (!(cond)) {                                                       \
@@ -748,7 +785,7 @@ static int spmm_csr(const char *fn, const int64_t *rowptr, const int32_t *col, c
   WDGH_REQUIRE_AT(norm == WDGH_NORM_NONE || dinv != nullptr, "norm requires dinv");
   WDGH_REQUIRE_AT(static_cast<const void *>(x) != y, "in-place aggregation is not supported");
   WDGH_REQUIRE_AT(row_offset >= 0, "negative row_offset");
-  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == WDGH_DTYPE_BF16, "bad y_dtype");
+  WDGH_REQUIRE_AT(y_dtype == WDGH_DTYPE_F32 || y_dtype == kHalfY<Tin>, "bad y_dtype (float32, or the type of x)");
   if (n == 0) return 0;
   SpmmArgs a;
   a.rowptr = rowptr; a.col = col; a.val = val; a.n = n; a.x = x; a.d = (int)d; a.ldx = ldx; a.y = y; a.ldy = ldy;
@@ -759,9 +796,9 @@ static int spmm_csr(const char *fn, const int64_t *rowptr, const int32_t *col, c
   a.st = as_stream(stream);
   WDGH_REQUIRE_AT(a.n_chunks == 0 || partial != nullptr, "split rows need the partial buffer");
   if constexpr (!std::is_same<Tin, float>::value) {  // (fp32 features have fp32 output only)
-    if (y_dtype == WDGH_DTYPE_BF16) {
-      const bool vec4 = rows_vec4(x, d, ldx, static_cast<const bf16 *>(y), ldy, partial);
-      return val ? dispatch<true, Tin, bf16, false>(a, vec4) : dispatch<false, Tin, bf16, false>(a, vec4);
+    if (y_dtype == kHalfY<Tin>) {
+      const bool vec4 = rows_vec4(x, d, ldx, static_cast<const Tin *>(y), ldy, partial);
+      return val ? dispatch<true, Tin, Tin, false>(a, vec4) : dispatch<false, Tin, Tin, false>(a, vec4);
     }
   }
   const bool vec4 = rows_vec4(x, d, ldx, static_cast<const float *>(y), ldy, partial);
@@ -784,6 +821,14 @@ extern "C" int wdgh_spmm_csr_bf16(const int64_t *rowptr, const int32_t *col, con
                                   int64_t *plan_i64, const int64_t *plan_host, float *partial, int64_t row_offset,
                                   void *stream) {
   return spmm_csr("wdgh_spmm_csr_bf16", rowptr, col, val, n, reinterpret_cast<const bf16 *>(x), d, ldx, y, ldy, y_dtype,
+                  norm, add_self_loop, dinv, deg_code, plan_i64, plan_host, partial, row_offset, stream);
+}
+
+extern "C" int wdgh_spmm_csr_f16(const int64_t *rowptr, const int32_t *col, const float *val, int64_t n,
+                                 const uint16_t *x, int64_t d, int64_t ldx, void *y, int64_t ldy, int y_dtype, int norm,
+                                 int add_self_loop, const float *dinv, const uint8_t *deg_code, int64_t *plan_i64,
+                                 const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  return spmm_csr("wdgh_spmm_csr_f16", rowptr, col, val, n, reinterpret_cast<const f16 *>(x), d, ldx, y, ldy, y_dtype,
                   norm, add_self_loop, dinv, deg_code, plan_i64, plan_host, partial, row_offset, stream);
 }
 
@@ -864,37 +909,42 @@ extern "C" int wdgh_plan_heavy_flags(const int64_t *plan_i64, const int64_t *pla
 }
 
 namespace wdgh {
-// fp32 -> bf16 of a strided block, round to nearest even (the rounding of __float22bfloat162_rn): one warp per row
-__global__ void round_bf16_kernel(const float *__restrict__ x, int64_t rows, int64_t cols, int64_t ldx,
-                                  bf16 *__restrict__ y, int64_t ldy, int pairs) {
+// fp32 -> H (bf16 or f16) of a strided block, round to nearest even (the rounding of the streaming stores): one warp
+// per row
+template <typename H>
+__global__ void round_half_kernel(const float *__restrict__ x, int64_t rows, int64_t cols, int64_t ldx,
+                                  H *__restrict__ y, int64_t ldy, int pairs) {
   const int lane = threadIdx.x & 31;
   const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < rows; r += warps) {
     const float *xr = x + r * ldx;
-    bf16 *yr = y + r * ldy;
+    H *yr = y + r * ldy;
     if (pairs) {
       for (int64_t c = 2 * lane; c < cols; c += 64) {
         const float2 v = *reinterpret_cast<const float2 *>(xr + c);
-        *reinterpret_cast<unsigned *>(yr + c) = bf16x2_rn(v.x, v.y);
+        *reinterpret_cast<unsigned *>(yr + c) = Half<H>::round2(v.x, v.y);
       }
     } else {
-      for (int64_t c = lane; c < cols; c += 32) yr[c] = __float2bfloat16_rn(xr[c]);
+      for (int64_t c = lane; c < cols; c += 32) yr[c] = Half<H>::round1(xr[c]);
     }
   }
 }
 
-int round_to_bf16(const float *x, int64_t rows, int64_t cols, int64_t ldx, void *y, int64_t ldy, cudaStream_t st) {
+template <typename H>
+int round_to_half(const float *x, int64_t rows, int64_t cols, int64_t ldx, void *y, int64_t ldy, cudaStream_t st) {
   if (rows == 0) return 0;
   const int pairs = (cols % 2 == 0) && (ldx % 2 == 0) && (ldy % 2 == 0) && (reinterpret_cast<uintptr_t>(x) % 8 == 0) &&
                     (reinterpret_cast<uintptr_t>(y) % 4 == 0);
-  round_bf16_kernel<<<persistent_grid(ceil_div(rows, 8), 8), 256, 0, st>>>(x, rows, cols, ldx, static_cast<bf16 *>(y),
-                                                                          ldy, pairs);
-  WDGH_LAUNCHED("round_bf16_kernel");
+  round_half_kernel<H><<<persistent_grid(ceil_div(rows, 8), 8), 256, 0, st>>>(x, rows, cols, ldx, static_cast<H *>(y),
+                                                                             ldy, pairs);
+  WDGH_LAUNCHED("round_half_kernel");
   return 0;
 }
+template int round_to_half<bf16>(const float *, int64_t, int64_t, int64_t, void *, int64_t, cudaStream_t);
+template int round_to_half<f16>(const float *, int64_t, int64_t, int64_t, void *, int64_t, cudaStream_t);
 
-// argument checks and dispatch shared by wdgh_spmm_csr_ranged (Tin = float) and wdgh_spmm_csr_ranged_bf16 (no extra
-// partial sums, n_extra = 0)
+// argument checks and dispatch shared by wdgh_spmm_csr_ranged (Tin = float), wdgh_spmm_csr_ranged_bf16 and
+// wdgh_spmm_csr_ranged_f16 (no extra partial sums, n_extra = 0)
 template <typename Tin>
 static int spmm_ranged(const char *fn, const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
                        const int32_t *col, const float *val, int64_t n, const Tin *x, int64_t d, int64_t ldx, float *y,
@@ -972,6 +1022,18 @@ extern "C" int wdgh_spmm_csr_ranged_bf16(const int64_t *rowptr, const int64_t *r
                                          const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
   return spmm_ranged("wdgh_spmm_csr_ranged_bf16", rowptr, range_begin, range_end, col, val, n,
                      reinterpret_cast<const bf16 *>(x), d, ldx, y, ldy, norm, add_self_loop, dinv, deg_code, skip_rows,
+                     accumulate, finalize, run_split_rows, nullptr, 0, 0, 0, 0, 0, plan_i64, plan_host, partial,
+                     row_offset, stream);
+}
+
+extern "C" int wdgh_spmm_csr_ranged_f16(const int64_t *rowptr, const int64_t *range_begin, const int64_t *range_end,
+                                        const int32_t *col, const float *val, int64_t n, const uint16_t *x, int64_t d,
+                                        int64_t ldx, float *y, int64_t ldy, int norm, int add_self_loop,
+                                        const float *dinv, const uint8_t *deg_code, const uint8_t *skip_rows,
+                                        int accumulate, int finalize, int run_split_rows, int64_t *plan_i64,
+                                        const int64_t *plan_host, float *partial, int64_t row_offset, void *stream) {
+  return spmm_ranged("wdgh_spmm_csr_ranged_f16", rowptr, range_begin, range_end, col, val, n,
+                     reinterpret_cast<const f16 *>(x), d, ldx, y, ldy, norm, add_self_loop, dinv, deg_code, skip_rows,
                      accumulate, finalize, run_split_rows, nullptr, 0, 0, 0, 0, 0, plan_i64, plan_host, partial,
                      row_offset, stream);
 }

@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libwdgh_b200.so")
 
 NORM_NONE, NORM_RW, NORM_SYM = 0, 1, 2
 NORM_RW_SUM, NORM_SYM_RAW = 3, 4   # scale modes of wdgh_degree_scale / wdgh_scale_values only (include/wdgh_b200.h)
-DTYPE_F32, DTYPE_BF16 = 0, 1       # output element type of wdgh_spmm_csr_bf16 / wdgh_pipeline_host_bf16
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2   # output element type of wdgh_spmm_csr_{bf16,f16} / wdgh_pipeline_host_*
 PLAN_HEADER = 16
 SC_MATCH_ALL, SC_MATCH_LAB, SC_N_LAB, SC_N_SELF, SC_N_EMPTY, SC_NBINS, SC_N_NODES_NSL, SC_N_MULTI_NEG = range(8)
 SC_HEADER = 8
@@ -51,12 +51,16 @@ SIGNATURES = {
                       _p],
     "wdgh_spmm_csr_bf16": [_p, _p, _p, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _int, _p, _p, _p, C.POINTER(_i64),
                            _p, _i64, _p],
+    "wdgh_spmm_csr_f16": [_p, _p, _p, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _int, _p, _p, _p, C.POINTER(_i64),
+                          _p, _i64, _p],
     "wdgh_column_segments": [_p, _p, _i64, _p, _i32, _p, _p],
     "wdgh_plan_heavy_flags": [_p, C.POINTER(_i64), _i64, _p, _p],
     "wdgh_spmm_csr_ranged": [_p, _p, _p, _p, _p, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _int, _int,
                              _int, _p, _i32, _i32, _i64, _i64, _i32, _p, C.POINTER(_i64), _p, _i64, _p],
     "wdgh_spmm_csr_ranged_bf16": [_p, _p, _p, _p, _p, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _int,
                                   _int, _int, _p, C.POINTER(_i64), _p, _i64, _p],
+    "wdgh_spmm_csr_ranged_f16": [_p, _p, _p, _p, _p, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _int,
+                                 _int, _int, _p, C.POINTER(_i64), _p, _i64, _p],
     "wdgh_structure_counts": [_p, _p, _i64, _i64, _p, _i32, _p, C.POINTER(_i64), _p, _p, _p, _p, _p, _i64, _i64, _p],
     "wdgh_spmm_structure_fused": [_p, _p, _i64, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _i32, _p,
                                   C.POINTER(_i64), _p, _p, _p, _p, _p, _p, _i64, _i64, _p],
@@ -74,6 +78,7 @@ SIGNATURES = {
     "wdgh_gntk_transform": [_p, _i64, _i64, _int, _p, _p],
     "wdgh_pipeline_host": [_p, _p, _i64, _i64, _p, _i64, _p, _i32, _int, _int, _p, _p, _p],
     "wdgh_pipeline_host_bf16": [_p, _p, _i64, _i64, _p, _i64, _p, _i32, _int, _int, _p, _int, _p, _p],
+    "wdgh_pipeline_host_f16": [_p, _p, _i64, _i64, _p, _i64, _p, _i32, _int, _int, _p, _int, _p, _p],
     "wdgh_pipeline_host_release": [],
 }
 _RESTYPE = {"wdgh_last_error": C.c_char_p, "wdgh_launch_count": C.c_uint64, "wdgh_gram_workspace_floats": C.c_int64,

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -15,6 +16,22 @@ from . import _lib
 from ._lib import NORM_NONE, NORM_RW, NORM_RW_SUM, NORM_SYM, NORM_SYM_RAW, check, lib, ptr, stream_ptr
 
 HEAVY_THRESHOLD = 512  # entries; longer rows are split into chunks of this many (degree binning)
+
+
+class _HalfEntries(NamedTuple):
+    code: int        # WDGH_DTYPE of an output of this type
+    spmm: str        # the C-ABI entries that read features of this type as they are (fp32 accumulation)
+    ranged: str
+    pipeline: str
+
+
+# The 16-bit feature types the aggregation reads without an fp32 copy.  Each writes float32, or its own type.
+_HALF = {
+    torch.bfloat16: _HalfEntries(_lib.DTYPE_BF16, "wdgh_spmm_csr_bf16", "wdgh_spmm_csr_ranged_bf16",
+                                 "wdgh_pipeline_host_bf16"),
+    torch.float16: _HalfEntries(_lib.DTYPE_F16, "wdgh_spmm_csr_f16", "wdgh_spmm_csr_ranged_f16",
+                                "wdgh_pipeline_host_f16"),
+}
 
 
 def _dev():
@@ -197,20 +214,20 @@ class CSRGraph:
 def spmm(g: CSRGraph, x, norm=NORM_NONE, add_self_loop=False, out=None, dinv=None, deg_code=None, out_dtype=None):
     """y = norm(A [+I]) x on the GPU with fp32 accumulation (hm.py:192,199,234; util_funcs.py:383-390,418-426).
 
-    A bfloat16 `x` is read as it is (no fp32 copy); its result is bit-identical to the one of `x.float()`.  The result
-    has the dtype of `out` if given, else `out_dtype`, else float32; bfloat16 output (round to nearest even) needs
-    bfloat16 features.  Any other `x` dtype is converted to float32 first.
+    A bfloat16 or float16 `x` is read as it is (no fp32 copy); its result is bit-identical to the one of `x.float()`.
+    The result has the dtype of `out` if given, else `out_dtype`, else float32; a half output (round to nearest even;
+    float16 overflows to +-inf) must have the dtype of the features.  Any other `x` dtype is converted to float32 first.
     For a row shard `x` (and `dinv`, the all-gathered degree scale) are global, the result is local."""
-    bf16 = isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16
+    half = _HALF.get(x.dtype) if isinstance(x, torch.Tensor) else None
     if out is not None:
         if out_dtype is not None and out_dtype != out.dtype:
             raise ValueError(f"out has dtype {out.dtype}, out_dtype asks for {out_dtype}")
         out_dtype = out.dtype
     out_dtype = torch.float32 if out_dtype is None else out_dtype
-    if out_dtype not in ((torch.float32, torch.bfloat16) if bf16 else (torch.float32,)):
-        raise ValueError(f"cannot write a {out_dtype} result from {x.dtype if bf16 else 'float32'} features "
-                         "(float32 output; bfloat16 output needs bfloat16 features)")
-    if bf16:
+    if out_dtype not in ((torch.float32, x.dtype) if half else (torch.float32,)):
+        raise ValueError(f"cannot write a {out_dtype} result from {x.dtype if half else 'float32'} features "
+                         "(float32 output, or the half type of the features)")
+    if half:
         # views with a unit column stride and whole rows apart (a column slab of a wider matrix) are read in place;
         # any other layout (transposed, broadcast rows) is copied like the float32 path does
         x = x.to(_dev(), non_blocking=True) if x.device.type != "cuda" else x
@@ -230,12 +247,11 @@ def spmm(g: CSRGraph, x, norm=NORM_NONE, add_self_loop=False, out=None, dinv=Non
         if g.n_global != g.n:
             raise ValueError("a row shard needs the all-gathered degree scale (dinv=...)")
         dinv, _, deg_code = g.degree_scale(norm, add_self_loop)
-    if bf16:
-        y_dtype = _lib.DTYPE_BF16 if out_dtype == torch.bfloat16 else _lib.DTYPE_F32
-        check(lib.wdgh_spmm_csr_bf16(ptr(g.rowptr), ptr(g.col), ptr(g.val), g.n, ptr(x), d, x.stride(0), ptr(y),
-                                     y.stride(0), y_dtype, norm, int(bool(add_self_loop)), ptr(dinv), ptr(deg_code),
-                                     ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()),
-              "wdgh_spmm_csr_bf16")
+    if half:
+        y_dtype = half.code if out_dtype == x.dtype else _lib.DTYPE_F32
+        check(getattr(lib, half.spmm)(ptr(g.rowptr), ptr(g.col), ptr(g.val), g.n, ptr(x), d, x.stride(0), ptr(y),
+                                      y.stride(0), y_dtype, norm, int(bool(add_self_loop)), ptr(dinv), ptr(deg_code),
+                                      ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()), half.spmm)
         return y
     check(lib.wdgh_spmm_csr(ptr(g.rowptr), ptr(g.col), ptr(g.val), g.n, ptr(x), d, x.stride(0), ptr(y), y.stride(0),
                             norm, int(bool(add_self_loop)), ptr(dinv), ptr(deg_code), ptr(plan), plan_host,
@@ -280,23 +296,23 @@ def spmm_ranged(g: CSRGraph, range_begin, range_end, x, y, norm, add_self_loop, 
     extra: [parts, rows >= n, d] tensor of raw partial sums of the same rows (possibly peer-mapped), added to every row
     as it is aggregated; the split-row pass adds only the last `extra_split` parts.  y may be peer memory.
     ctas_per_sm: 0 = default grid, smaller = leave room for a kernel running concurrently on another stream.
-    A bfloat16 `x` (float32 `y`, no `extra`, no `ctas_per_sm`) is read as it is; every phase sums in fp32 and is
-    bit-identical to the same call on `x.float()`."""
+    A bfloat16 or float16 `x` (float32 `y`, no `extra`, no `ctas_per_sm`) is read as it is; every phase sums in fp32
+    and is bit-identical to the same call on `x.float()`."""
     d = int(x.shape[1])
     x_ptr = x.data_ptr() - int(x_row0) * x.stride(0) * x.element_size()
     plan, plan_host = g.plan
     partial = _partial_scratch(g, d)
-    if x.dtype == torch.bfloat16:
+    half = _HALF.get(x.dtype)
+    if half:
         if extra is not None or ctas_per_sm:
             raise ValueError("extra partial sums and ctas_per_sm need float32 features")
         if y.dtype != torch.float32:
             raise ValueError(f"a phase writes float32 partial sums, got a {y.dtype} y")
-        check(lib.wdgh_spmm_csr_ranged_bf16(ptr(g.rowptr), ptr(range_begin), ptr(range_end), ptr(g.col), ptr(g.val),
-                                            g.n, x_ptr, d, x.stride(0), ptr(y), y.stride(0), norm,
-                                            int(bool(add_self_loop)), ptr(dinv), ptr(deg_code), ptr(skip_rows),
-                                            int(bool(accumulate)), int(bool(finalize)), int(bool(run_split_rows)),
-                                            ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()),
-              "wdgh_spmm_csr_ranged_bf16")
+        check(getattr(lib, half.ranged)(ptr(g.rowptr), ptr(range_begin), ptr(range_end), ptr(g.col), ptr(g.val),
+                                        g.n, x_ptr, d, x.stride(0), ptr(y), y.stride(0), norm,
+                                        int(bool(add_self_loop)), ptr(dinv), ptr(deg_code), ptr(skip_rows),
+                                        int(bool(accumulate)), int(bool(finalize)), int(bool(run_split_rows)),
+                                        ptr(plan), plan_host, ptr(partial), g.row_offset, stream_ptr()), half.ranged)
         return y
     n_extra = part_rows = ld_extra = 0
     if extra is not None:
@@ -404,16 +420,16 @@ def spmm_structure_fused(g: CSRGraph, x, labels32, num_classes, norm=NORM_SYM, a
                          dinv=None, deg_code=None, scratch=None, out_dtype=None):
     """One call: y = norm(A [+I]) x and the label statistics (device tensors, no sync).
 
-    Returns (y, (counters, node_sum, deg, match, labels_u8)); binary adjacency only.  A bfloat16 `x` is read as it is
-    (the bf16 aggregation, then the label pass on the same stream); `out_dtype` / `out` as in `spmm`."""
+    Returns (y, (counters, node_sum, deg, match, labels_u8)); binary adjacency only.  A bfloat16 or float16 `x` is read
+    as it is (the half aggregation, then the label pass on the same stream); `out_dtype` / `out` as in `spmm`."""
     if g.val is not None:
         raise ValueError("the fused pass needs a binary adjacency (values = None)")
-    if isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16:
+    if isinstance(x, torch.Tensor) and x.dtype in _HALF:
         y = spmm(g, x, norm, add_self_loop, out=out, dinv=dinv, deg_code=deg_code, out_dtype=out_dtype)
         return y, structure_counts_raw(g, labels32, num_classes, scratch)
     if out_dtype not in (None, torch.float32):
-        raise ValueError(f"cannot write a {out_dtype} result from float32 features (bfloat16 output needs bfloat16 "
-                         "features)")
+        raise ValueError(f"cannot write a {out_dtype} result from float32 features (a half output needs features of "
+                         "that type)")
     x = _cuda(x, torch.float32)
     d = int(x.shape[1])
     c = int(num_classes)
@@ -440,18 +456,19 @@ def spmm_structure_fused(g: CSRGraph, x, labels32, num_classes, norm=NORM_SYM, a
 
 
 def pipeline_host(rowptr, col, x, labels, num_classes, norm=NORM_SYM, add_self_loop=True, y=None):
-    """The whole pass from HOST memory (wdgh_pipeline_host / wdgh_pipeline_host_bf16): copies in, plan, degree scale,
+    """The whole pass from HOST memory (wdgh_pipeline_host / _bf16 / _f16): copies in, plan, degree scale,
     y = norm(A [+I]) x, label statistics, copies back.  Synchronous; device buffers are cached between calls.
 
-    rowptr int64 [n+1], col int32 [nnz], labels int32 [n] and x [n, d] float32 or bfloat16 (bfloat16 halves the
-    feature bytes on the link) are contiguous CPU tensors -- pinned memory lets the copies run at the full link rate.
-    y: None (counters only) or a contiguous [n, d] CPU tensor, filled in place: float32, or bfloat16 with bfloat16
-    features (the float32 result rounded to nearest even).  Returns (counters int64[sc_words(C)], node_sum float64[2])
-    as numpy arrays."""
+    rowptr int64 [n+1], col int32 [nnz], labels int32 [n] and x [n, d] float32, bfloat16 or float16 (a half type
+    halves the feature bytes on the link) are contiguous CPU tensors -- pinned memory lets the copies run at the full
+    link rate.  y: None (counters only) or a contiguous [n, d] CPU tensor, filled in place: float32, or the half type of
+    the features (the float32 result rounded to nearest even).  Returns (counters int64[sc_words(C)], node_sum
+    float64[2]) as numpy arrays."""
+    feature_dtypes = (torch.float32,) + tuple(_HALF)
     named = [("rowptr", rowptr, (torch.int64,)), ("col", col, (torch.int32,)), ("labels", labels, (torch.int32,)),
-             ("x", x, (torch.float32, torch.bfloat16))]
+             ("x", x, feature_dtypes)]
     if y is not None:
-        named.append(("y", y, (torch.float32, torch.bfloat16)))
+        named.append(("y", y, feature_dtypes))
     for name, t, dtypes in named:
         if not isinstance(t, torch.Tensor) or t.device.type != "cpu":
             raise ValueError(f"{name} must be a CPU tensor")
@@ -465,21 +482,21 @@ def pipeline_host(rowptr, col, x, labels, num_classes, norm=NORM_SYM, add_self_l
     if rowptr.shape != (n + 1,) or col.dim() != 1 or labels.shape != (n,):
         raise ValueError(f"rowptr must be [{n + 1}], col 1-D and labels [{n}]; got {tuple(rowptr.shape)}, "
                          f"{tuple(col.shape)}, {tuple(labels.shape)}")
-    bf16 = x.dtype == torch.bfloat16
+    half = _HALF.get(x.dtype)
     if y is not None:
         if y.shape != (n, d):
             raise ValueError(f"y must be [{n}, {d}], got {tuple(y.shape)}")
-        if y.dtype == torch.bfloat16 and not bf16:
-            raise ValueError("a bfloat16 y needs bfloat16 features")
+        if y.dtype not in (torch.float32, x.dtype):
+            raise ValueError(f"a {y.dtype} y needs {y.dtype} features, got {x.dtype}")
     c = int(num_classes)
     counters = np.zeros(_lib.sc_words(c), np.int64)
     node_sum = np.zeros(2, np.float64)
     _lib.require_device()
     args = (ptr(rowptr), ptr(col), n, int(col.shape[0]), ptr(x), d, ptr(labels), c, norm, int(bool(add_self_loop)))
-    if bf16:
-        y_dtype = _lib.DTYPE_BF16 if y is not None and y.dtype == torch.bfloat16 else _lib.DTYPE_F32
-        check(lib.wdgh_pipeline_host_bf16(*args, ptr(y), y_dtype, counters.ctypes.data, node_sum.ctypes.data),
-              "wdgh_pipeline_host_bf16")
+    if half:
+        y_dtype = half.code if y is not None and y.dtype == x.dtype else _lib.DTYPE_F32
+        check(getattr(lib, half.pipeline)(*args, ptr(y), y_dtype, counters.ctypes.data, node_sum.ctypes.data),
+              half.pipeline)
     else:
         check(lib.wdgh_pipeline_host(*args, ptr(y), counters.ctypes.data, node_sum.ctypes.data), "wdgh_pipeline_host")
     return counters, node_sum

@@ -223,7 +223,8 @@ def _ids(mask_or_ids, device):
 
 def similarity(features, adj, label, hard=None, LP=1, ifsum=1, idx_train=None):
     """hm.py:190-229: aggregation similarity score (soft / hard LAS) from (A X)(A X)^T -- for more than
-    graph.GRAM_SIMILARITY_MAX_ROWS rows without forming it (class sums of A X), so whole graphs of any size work."""
+    graph.GRAM_SIMILARITY_MAX_ROWS rows without forming it (class sums of A X), so whole graphs of any size work.
+    bfloat16 / float16 features are aggregated as they are (no fp32 copy) and give the score of features.float()."""
     z = _propagate(adj, features)
     label = G._cuda(label, torch.float32)
     labels = G.argmax_rows(label)                                   # hm.py:193

@@ -110,7 +110,8 @@ def sparse_mx_to_torch_sparse_tensor(sparse_mx):
 def propagate(adj, features, symmetric=1, add_self_loop=True, out_dtype=None):
     """SGC-1 / GCN propagation A_hat X without materialising A_hat (on-the-fly D^-1/2 or D^-1).
 
-    bfloat16 features are read as they are (fp32 accumulation); out_dtype=torch.bfloat16 returns a bfloat16 result."""
+    bfloat16 and float16 features are read as they are (fp32 accumulation, the bits of the call on features.float());
+    out_dtype=torch.bfloat16 / torch.float16, the dtype of the features, returns the result rounded to that type."""
     g = _to_graph(adj, binary=True)
     return G.spmm(g, features, G.NORM_SYM if symmetric else G.NORM_RW, add_self_loop, out_dtype=out_dtype)
 
